@@ -1,6 +1,6 @@
 """bench.py -- read pairs/s of the read-generation hot path (generate-reads + Illumina corruption).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload chr1|wgs]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload chr1|wgs] [--dump-outputs DIR]
 
 Workload (config.workload)
   N = 1   BASELINE.json configs[2]: one chr1-shaped synthetic contig (249,250,621 bp, ~10 % N in long
@@ -59,7 +59,13 @@ def parse():
   ap.add_argument('--e2e-steps', type=int, default=None, help='timed e2e steps (default: --steps, capped so that the leg stays within minutes)')
   ap.add_argument('--mode', default='generate-reads', choices=['generate-reads', 'corrupt-reads'], help="'corrupt-reads': the standalone corrupt kernel over a resident FASTQ pair (second-figure roofline, 1480 B/pair)")
   ap.add_argument('--soft-masked', action='store_true', help='chr1 workload with half of the bases in lower-case stretches (not the headline configuration)')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='after the timed steps, write what the last one computed as DIR/<name>.npy (see OutputSample); with several ranks, DIR/rank<r>/')
   a = ap.parse_args()
+  if a.steps < 1 or a.warmup < 0:
+    ap.error('--steps must be at least 1 and --warmup at least 0')
+  if a.dump_outputs and a.impl != 'b200':
+    ap.error('--dump-outputs records the outputs of this project (--impl b200)')
   world = int(os.environ.get('WORLD_SIZE', '1'))
   if a.workload is None:
     a.workload = 'wgs' if max(world, a.gpus) > 1 else 'chr1'
@@ -347,6 +353,61 @@ def pick_sink(args, bytes_per_step):
           '{} (tmpfs files; the native writer threads copy every piece to its final offset through a shared mapping)'.format(want))
 
 
+DUMP_BYTES = 12 << 20    # FASTQ bytes sampled from one step for --dump-outputs, shared by the ranks: 48 MB as float32
+DUMP_WINDOWS = 8         # sampled windows per unit and FASTQ file
+DUMP_SEED = 20240        # fixes where in a unit the windows lie
+
+
+class OutputSample(object):
+  """--dump-outputs: what the timed path hands its caller in its last step, as .npy files on which two
+  builds can be compared.  A step writes GBs of FASTQ, so of each FASTQ file of each unit (a work unit
+  of generate-reads, an input chunk of corrupt-reads) DUMP_WINDOWS windows are copied, at fixed seeded
+  fractions of the file's length: equal outputs are sampled at equal offsets.  With several ranks each
+  rank writes its own units under DIR/rank<r>/ and the ranks split DUMP_BYTES.
+
+    unit<k>_fastq<m>.npy   float32 [DUMP_WINDOWS, width]  the byte values of the windows of file m (1, 2)
+    window_offsets.npy     float64 [units, 2, DUMP_WINDOWS]  where the windows start
+    unit_bytes.npy         float64 [units, 2]  bytes of each file
+    unit_<count>.npy       float64 [units]  the counts the path returns per unit (templates, ...)
+  """
+
+  def __init__(self, path, max_units, alloc):
+    world = int(os.environ.get('WORLD_SIZE', '1'))
+    self.path = path if world == 1 else os.path.join(path, 'rank{}'.format(int(os.environ.get('RANK', '0'))))
+    self.max_units = max_units
+    self.width = max(1, DUMP_BYTES // world // (2 * DUMP_WINDOWS * max(1, max_units)))
+    self.buf = alloc(2 * DUMP_WINDOWS * self.width * max(1, max_units))
+    self.frac = np.sort(np.random.RandomState(DUMP_SEED).random_sample(DUMP_WINDOWS))
+    self.units = []
+
+  def take(self, read, sizes, **counts):
+    """One unit: read(m, offset, nbytes, dst) copies bytes of its file m (0, 1), of sizes[m] bytes, into dst."""
+    k = len(self.units)
+    if k == self.max_units:
+      raise RuntimeError('--dump-outputs: more than the {} units planned for'.format(self.max_units))
+    windows = []
+    for m in (0, 1):
+      w = min(self.width, int(sizes[m]))
+      offs = (self.frac * (int(sizes[m]) - w)).astype(np.int64)
+      for j, o in enumerate(offs):
+        start = ((2 * k + m) * DUMP_WINDOWS + j) * self.width
+        read(m, int(o), w, self.buf[start:start + w])
+      windows.append((offs, w))
+    self.units.append((counts, sizes, windows))
+
+  def write(self):
+    os.makedirs(self.path, exist_ok=True)
+    for k, (_, _, windows) in enumerate(self.units):
+      for m, (_, w) in enumerate(windows):
+        start = (2 * k + m) * DUMP_WINDOWS * self.width
+        rows = self.buf[start:start + DUMP_WINDOWS * self.width].reshape(DUMP_WINDOWS, self.width)[:, :w]
+        np.save(os.path.join(self.path, 'unit{}_fastq{}.npy'.format(k, m + 1)), rows.astype(np.float32))
+    np.save(os.path.join(self.path, 'window_offsets.npy'), np.array([[offs for offs, _ in u[2]] for u in self.units], dtype=np.float64))
+    np.save(os.path.join(self.path, 'unit_bytes.npy'), np.array([u[1] for u in self.units], dtype=np.float64))
+    for name in (self.units[0][0] if self.units else {}):
+      np.save(os.path.join(self.path, 'unit_{}.npy'.format(name)), np.array([u[0][name] for u in self.units], dtype=np.float64))
+
+
 def main():
   if os.environ.get('MG_BENCH_LOG'):
     import logging
@@ -410,9 +471,9 @@ def main():
   else:
     mine = [0]
 
-  def value_step(seed, rids):
+  def value_step(seed, rids, sample=None):
     """The rank's contigs: copies built from the resident packed region, then copies x passes units,
-    outputs left in HBM.  -> (pairs, fastq bytes)"""
+    outputs left in HBM (with `sample`, windows of them are also copied to the host).  -> (pairs, fastq bytes)"""
     pairs = nbytes = 0
     k = 0
     for ci, rid in zip(mine, rids):
@@ -420,8 +481,10 @@ def main():
       copies = [eng.build_copy(rid, vl) for vl in r_['v']]
       for cpy in range(len(copies)):
         for ps in range(rm['passes']):
-          _, _, cnt, _, nb = rg.generate_unit(eng, il, rm, copies[cpy], region_[0], cpy, (seed * 7919 + k * 104729) & 0xFFFFFFFF,
-                                              wl['sample'], 0, k, mode='philox', corrupt=corrupt, corrupt_seed=seed, fetch=False)
+          _, _, cnt, nk, nb = rg.generate_unit(eng, il, rm, copies[cpy], region_[0], cpy, (seed * 7919 + k * 104729) & 0xFFFFFFFF,
+                                               wl['sample'], 0, k, mode='philox', corrupt=corrupt, corrupt_seed=seed, fetch=False)
+          if sample is not None:
+            sample.take(eng.unit_read, (nb, nb), templates=cnt, te_kept=nk)
           pairs += cnt; nbytes += 2 * nb; k += 1
       for cp in copies:
         eng.free_copy(cp)
@@ -435,6 +498,11 @@ def main():
 
   # ---- value: inputs resident in HBM, outputs stay in HBM
   rids = [eng.load_region(refs[wl['regions'][ci]], wl['regions'][ci][1]) for ci in mine]
+  sample = None
+  if args.dump_outputs:
+    # the last timed step copies windows of each unit's output to page-locked memory on the library's copy stream,
+    # next to the following unit's kernels: that step's outputs themselves are recorded, not a later rerun
+    sample = OutputSample(args.dump_outputs, sum(len(vcf_df[ci]['v']) for ci in mine) * rm['passes'], eng.pinned)
   clocks = ClockSampler(local); clocks.start()
   for w in range(args.warmup):
     value_step(1000 + w, rids)
@@ -446,11 +514,14 @@ def main():
   with torch.cuda.stream(stream):
     ev0.record(stream)
     for s in range(args.steps):
-      p_, b_ = value_step(2000 + s, rids)
+      p_, b_ = value_step(2000 + s, rids, sample if s == args.steps - 1 else None)
       pairs += p_; nbytes += b_
     ev1.record(stream)
   barrier()
   ms = ev0.elapsed_time(ev1)
+  if sample is not None:
+    eng.wait_copies()
+    sample.write()
   clk = clocks.stop()
   prof = eng.prof()
   for rid in rids:
@@ -624,23 +695,30 @@ def bench_corrupt_reads(args, eng, rm, model):
   p1, p2 = eng.pinned(chunk), eng.pinned(chunk)
   outs = (eng.pinned(chunk + (1 << 20)), eng.pinned(chunk + (1 << 20)))
 
-  def one_pass():
-    o1 = o2 = 0; done = 0
+  def one_pass(sample=None):
+    """-> (templates, chunks) of one pass over the resident pair."""
+    o1 = o2 = 0; done = 0; chunks = 0
     while o1 < f1.size:
       a1 = f1[o1:o1 + chunk]; a2 = f2[o2:o2 + chunk]
       p1[:a1.size] = a1; p2[:a2.size] = a2
-      _, _, k, c1, c2 = eng.corrupt_fastq(p1[:a1.size], p2[:a2.size], mode=MODE_PHILOX, seed=args.seed, first_template=done, out=outs, partial=True)
-      o1 += c1; o2 += c2; done += k
-    return done
+      q1, q2, k, c1, c2 = eng.corrupt_fastq(p1[:a1.size], p2[:a2.size], mode=MODE_PHILOX, seed=args.seed, first_template=done, out=outs, partial=True)
+      if sample is not None:
+        sample.take(lambda m, off, n, dst: np.copyto(dst, (q1, q2)[m][off:off + n]), (q1.size, q2.size), templates=k)  # noqa: B023
+      o1 += c1; o2 += c2; done += k; chunks += 1
+    return done, chunks
 
   for _ in range(max(1, min(args.warmup, 2))):
-    one_pass()
+    _, n_chunks = one_pass()
+  # every pass cuts the same input into the same chunks: the warm-up's count is the count of the last timed pass
+  sample = OutputSample(args.dump_outputs, n_chunks, eng.pinned) if args.dump_outputs else None
   eng.prof_reset()
   t0 = time.perf_counter()
   pairs = 0
-  for _ in range(args.steps):
-    pairs += one_pass()
+  for s in range(args.steps):
+    pairs += one_pass(sample if s == args.steps - 1 else None)[0]
   wall = time.perf_counter() - t0
+  if sample is not None:
+    sample.write()
   prof = eng.prof()
   peak, peak_src = measured_peak()
   alg = 2.0 * (f1.size + f2.size) * args.steps                          # read once + written once, both files
