@@ -248,6 +248,31 @@ int mg_check_add_copy(mg_checker *k, int64_t copy_id, const char *chrom, int32_t
 int mg_check_fastq(mg_checker *k, const uint8_t *in1, int64_t len1, const uint8_t *in2, int64_t len2, int64_t *n_records,
                    int64_t *n_bad, int64_t *bad_index, int32_t *bad_code, int32_t bad_cap, int64_t *consumed1, int64_t *consumed2);
 
+/* ---- god-aligner: replaces mitty/benchmarking/god_aligner.py (process_multi_threaded, god_aligner.py:43-121).
+ * Every read of a FASTQ (pair) becomes one BAM record at the POS / CIGAR its qname states, strand-1 reads
+ * reverse-complemented back; the records are encoded and sorted by (refID, pos, reverse bit) on the device
+ * in runs of at most run_bytes of device memory (<= 0: derived from free memory) and written as a BGZF BAM
+ * with a BAI index by `threads` host deflate threads at `level`.
+ * mg_bam_open: the FASTA's contigs in order, the SAM header text (@HD / @SQ / @RG lines), the RG value;
+ * bai_path NULL writes no index.  mg_bam_add encodes the COMPLETE templates present in both buffers
+ * (consumed1/2 as for mg_corrupt_fastq; fewer when the run is full: call again with the rest); a read the
+ * BAM cannot hold is MG_EVALUE with bad_index = template * files + file and bad_code = 1 not a 4-line
+ * record, 2 malformed qname, 3 chrom not in the FASTA, 4 name over 254 bytes, 5 length differs from rlen /
+ * CIGAR, 6 malformed CIGAR, 7 alignment outside the contig.  mg_bam_close sorts / merges the last run and
+ * writes BAM + BAI (n_runs: sorted runs used; times[3] ms: device work incl. ingest, device-to-host copies,
+ * writing); on error nothing is left behind.  mg_bam_abort drops everything, temporary files included.
+ * mg_bam_write_sorted: the BGZF writer + BAI builder alone, without a device, over records already encoded
+ * and in coordinate order.                                                                            */
+typedef struct mg_bam mg_bam;
+int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
+                const char *header_text, const char *sample, int32_t level, int32_t threads, int64_t run_bytes, mg_bam **out);
+int mg_bam_add(mg_bam *b, const uint8_t *in1, int64_t len1, const uint8_t *in2, int64_t len2, int64_t *n_templates, int64_t *consumed1,
+               int64_t *consumed2, int64_t *bad_index, int32_t *bad_code);
+int mg_bam_close(mg_bam *b, int64_t *n_records, int64_t *n_runs, double *times);
+void mg_bam_abort(mg_bam *b);
+int mg_bam_write_sorted(const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
+                        const char *header_text, const uint8_t *records, int64_t len, int32_t level, int32_t threads, int64_t *n_records);
+
 /* ---- profiling: device time (CUDA events on the launch stream) of the emit / corrupt kernel
  * (emit_ms over emit_launches launches, emit_bytes written) and of the planning kernel (plan_ms);
  * total_launches counts every kernel this context launched since the last reset.               */

@@ -1,5 +1,5 @@
 """Command line with the reference's ``generate-reads`` / ``corrupt-reads`` / ``qname`` commands
-(mitty/cli.py:106-157): same positional arguments and options, plus ``--deterministic`` (consume
+(mitty/cli.py:106-157) and ``god-aligner`` (mitty/cli.py:191-204): same positional arguments and options, plus ``--deterministic`` (consume
 the reference's numpy draws; byte-exact against ``mitty ... --threads 1``) and, for
 generate-reads, ``--corrupt`` (fuse the corruption model into the emit kernel)."""
 import logging
@@ -111,6 +111,22 @@ def check_reads(fasta, vcf, sample_name, bed, fastq1, fastq2, device, max_report
   click.echo('{} reads of {} templates checked in {:0.2f}s: {} failed'.format(res['reads'], res['templates'], res['seconds'], res['bad']))
   if res['bad']:
     raise SystemExit(1)
+
+
+@cli.command('god-aligner', short_help='Write the perfect alignments of simulated reads as a sorted, indexed BAM')
+@click.argument('fasta', type=click.Path(exists=True))
+@click.argument('fastq1', type=click.Path(exists=True))
+@click.argument('bam', type=click.Path())
+@click.option('--fastq2', type=click.Path(exists=True))
+@click.option('--threads', type=int, default=None, help='host deflate threads (default: the cores of the box)')
+@click.option('--device', default=0, help='CUDA device')
+@click.option('--level', type=click.IntRange(0, 9), default=6, help='BGZF deflate level (0: stored blocks)')
+def god_aligner(fasta, fastq1, bam, fastq2, threads, device, level):
+  """Place every read exactly where its qname says: a coordinate-sorted BAM (and BAM.bai) of the
+  perfect alignments, the truth set for an aligner or variant caller benchmark."""
+  import mitty_b200.benchmarking.god_aligner as ga
+  res = ga.process_multi_threaded(fasta, bam, fastq1, fastq2, threads=threads, device=device, level=level)
+  click.echo('{} records written to {} in {:0.2f}s'.format(res['records'], bam, res['seconds']))
 
 
 @cli.command('corrupt-reads', short_help='Apply corruption model to FASTQ file of reads')

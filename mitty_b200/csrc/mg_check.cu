@@ -20,6 +20,7 @@
 
 #include "../../include/mitty_b200.h"
 #include "mg_internal.h"
+#include "mg_qname.cuh"
 
 namespace {
 
@@ -72,16 +73,6 @@ struct ChkParams {
   unsigned long long *n_bad;
 };
 
-__device__ __forceinline__ bool parse_int(const uint8_t *p, int64_t a, int64_t b, int64_t &v) {
-  if (a >= b) return false;
-  bool neg = false;
-  if (p[a] == '-') { neg = true; a++; if (a >= b) return false; }
-  int64_t x = 0;
-  for (int64_t i = a; i < b; i++) { const uint8_t c = p[i]; if (c < '0' || c > '9') return false; x = x * 10 + (c - '0'); if (x > (1ll << 40)) return false; }
-  v = neg ? -x : x;
-  return true;
-}
-
 __global__ void __launch_bounds__(256) k_roundtrip_check(ChkParams P) {
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= P.n_rec * P.n_files) return;
@@ -94,15 +85,13 @@ __global__ void __launch_bounds__(256) k_roundtrip_check(ChkParams P) {
   do {
     if (h1 <= h0 || q[h0] != '@' || nl[4 * r + 2] != s1 + 2 || q[s1 + 1] != '+' || nl[4 * r + 3] - nl[4 * r + 2] != s1 - s0 + 1) { code = CHK_FRAME; break; }
     // fields: 0 serial, 1 chrom, 2 copy, then strand | pos | rlen | cigar | vlist per read in file order; this file's read is the f-th
-    int64_t fs[16], fe[16]; int nf = 0;
-    int64_t a = h0 + 1;
-    for (int64_t i = h0 + 1; i <= h1 && nf < 16; i++)
-      if (i == h1 || q[i] == '|') { fs[nf] = a; fe[nf] = i; nf++; a = i + 1; }
+    int64_t fs[MG_QN_FIELDS], fe[MG_QN_FIELDS];
+    const int nf = mg_qname_split(q, h0 + 1, h1, fs, fe);
     const int base = 3 + 5 * f;
     if (nf < base + 5) { code = CHK_QNAME; break; }
     int64_t cpy, strand, pos, rlen;
-    if (!parse_int(q, fs[2], fe[2], cpy) || !parse_int(q, fs[base], fe[base], strand) || !parse_int(q, fs[base + 1], fe[base + 1], pos) ||
-        !parse_int(q, fs[base + 2], fe[base + 2], rlen) || (strand != 0 && strand != 1)) { code = CHK_QNAME; break; }
+    if (!mg_parse_int(q, fs[2], fe[2], cpy) || !mg_parse_int(q, fs[base], fe[base], strand) || !mg_parse_int(q, fs[base + 1], fe[base + 1], pos) ||
+        !mg_parse_int(q, fs[base + 2], fe[base + 2], rlen) || (strand != 0 && strand != 1)) { code = CHK_QNAME; break; }
     const ChkCopy *C = nullptr;
     const int cl = (int)(fe[1] - fs[1]);
     for (int k = 0; k < P.n_copies && !C; k++) {
@@ -122,7 +111,7 @@ __global__ void __launch_bounds__(256) k_roundtrip_check(ChkParams P) {
       int64_t colon = ca + 1;
       while (colon < cb && q[colon] != ':') colon++;
       int64_t off, n;
-      if (colon >= cb || q[cb - 1] != 'I' || !parse_int(q, ca + 1, colon, off) || !parse_int(q, colon + 1, cb - 1, n) || n != L) { code = CHK_QNAME; break; }
+      if (colon >= cb || q[cb - 1] != 'I' || !mg_parse_int(q, ca + 1, colon, off) || !mg_parse_int(q, colon + 1, cb - 1, n) || n != L) { code = CHK_QNAME; break; }
       int k = last_node_pr_le(C->nodes, C->n_nodes, pos + 1);
       while (k >= 0 && C->nodes[k].pr == pos + 1 && C->nodes[k].op != 'I') k--;
       if (k < 0 || C->nodes[k].pr != pos + 1 || C->nodes[k].op != 'I') { code = CHK_NOINS; break; }
@@ -137,7 +126,7 @@ __global__ void __launch_bounds__(256) k_roundtrip_check(ChkParams P) {
       int64_t e = ca;
       while (e < cb && q[e] >= '0' && q[e] <= '9') e++;
       int64_t c;
-      if (e == ca || e >= cb || !parse_int(q, ca, e, c)) { code = CHK_QNAME; break; }
+      if (e == ca || e >= cb || !mg_parse_int(q, ca, e, c)) { code = CHK_QNAME; break; }
       const uint8_t op = q[e];
       ca = e + 1;
       if (op == '=') {

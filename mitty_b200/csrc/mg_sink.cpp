@@ -42,6 +42,18 @@
 #include <vector>
 
 #include "../../include/mitty_b200.h"
+#include "mg_deflate.h"
+
+void mg_deflate(const uint8_t *in, int64_t n, int level, int window_bits, std::vector<uint8_t> &out, size_t head) {
+  z_stream z; memset(&z, 0, sizeof z);
+  deflateInit2(&z, level, Z_DEFLATED, window_bits, 8, Z_DEFAULT_STRATEGY);
+  out.resize(head + deflateBound(&z, (uLong)n) + 64);
+  z.next_in = const_cast<Bytef *>(in); z.avail_in = (uInt)n;
+  z.next_out = out.data() + head; z.avail_out = (uInt)(out.size() - head);
+  deflate(&z, Z_FINISH);
+  out.resize(out.size() - z.avail_out);
+  deflateEnd(&z);
+}
 
 namespace {
 
@@ -207,16 +219,7 @@ Slot *alloc_slot(mg_sink *s, int p) {
   return sl;
 }
 
-void deflate_piece(Piece *p, int level) {
-  z_stream z; memset(&z, 0, sizeof z);
-  deflateInit2(&z, level, Z_DEFLATED, 15 + 16 /* gzip wrapper */, 8, Z_DEFAULT_STRATEGY);
-  p->z.resize(deflateBound(&z, (uLong)p->bytes) + 64);
-  z.next_in = const_cast<Bytef *>(p->data); z.avail_in = (uInt)p->bytes;
-  z.next_out = p->z.data(); z.avail_out = (uInt)p->z.size();
-  deflate(&z, Z_FINISH);
-  p->z.resize(p->z.size() - z.avail_out);
-  deflateEnd(&z);
-}
+void deflate_piece(Piece *p, int level) { mg_deflate(p->data, p->bytes, level, 15 + 16 /* gzip wrapper */, p->z, 0); }
 
 void worker(mg_sink *s) {
   std::unique_lock<std::mutex> lk(s->mu);

@@ -368,6 +368,66 @@ class Checker(object):
       self._h = None
 
 
+BAM_CODES = {1: "not a 4-line record with a bare '+' line", 2: 'malformed qname', 3: 'chrom is not a contig of the FASTA',
+             4: 'read name longer than the 254 bytes BAM can hold', 5: 'read length differs from rlen / the CIGAR', 6: 'malformed CIGAR',
+             7: 'alignment outside its contig'}
+
+
+class BamWriter(object):
+  """The god-aligner on the device (mg_bam_*): FASTQ chunks in, a coordinate-sorted BGZF BAM + BAI out.
+  ``add`` encodes the complete templates of a chunk pair into the current sorted run; ``close`` sorts /
+  merges and writes.  ``run_bytes``: device memory of one run (None: derived from free memory)."""
+
+  def __init__(self, engine, bam, bai, contigs, header_text, sample, level=6, threads=1, run_bytes=None):
+    self.engine, self._L = engine, engine._L
+    names = [str(n).encode() for n, _ in contigs]
+    self._names = (C.c_char_p * len(names))(*names)
+    self._lens = np.ascontiguousarray([int(l) for _, l in contigs], dtype=np.int64)
+    h = C.c_void_p()
+    engine._check(self._L.mg_bam_open(engine._h, str(bam).encode(), str(bai).encode() if bai else None, len(names), self._names, _ptr(self._lens),
+                                      header_text.encode(), str(sample).encode(), int(level), int(threads), int(run_bytes or 0), C.byref(h)))
+    self._h = h
+
+  def add(self, fq1, fq2=None):
+    """-> (templates encoded, consumed bytes of fq1, of fq2).  A read the BAM cannot hold raises ValueError
+    with (file, record in this chunk, reason) as ``args[1:]``."""
+    n, c1, c2, bi, bc = C.c_int64(0), C.c_int64(0), C.c_int64(0), C.c_int64(-1), C.c_int32(0)
+    rc = self._L.mg_bam_add(self._h, _ptr(fq1) if fq1.size else _ptr(np.zeros(1, np.uint8)), fq1.size, _ptr(fq2) if fq2 is not None else None,
+                            fq2.size if fq2 is not None else 0, C.byref(n), C.byref(c1), C.byref(c2), C.byref(bi), C.byref(bc))
+    if rc == _lib.MG_EVALUE and bi.value >= 0:
+      nf = 2 if fq2 is not None else 1
+      raise ValueError('not writable as a BAM record', bi.value % nf, bi.value // nf, BAM_CODES.get(bc.value, str(bc.value)))
+    self.engine._check(rc)
+    return n.value, c1.value, c2.value
+
+  def close(self):
+    """Sort / merge the last run, write BAM + BAI -> (records, sorted runs, {'device_ms', 'd2h_ms', 'write_ms'})."""
+    n, runs, t = C.c_int64(0), C.c_int64(0), np.zeros(3, dtype=np.float64)
+    h, self._h = self._h, None
+    self.engine._check(self._L.mg_bam_close(h, C.byref(n), C.byref(runs), _ptr(t)))
+    return n.value, runs.value, {'device_ms': t[0], 'd2h_ms': t[1], 'write_ms': t[2]}
+
+  def abort(self):
+    if self._h:
+      self._L.mg_bam_abort(self._h)
+      self._h = None
+
+
+def write_sorted_bam(bam, bai, contigs, header_text, records, level=6, threads=1):
+  """The BGZF writer + BAI builder without a device: ``records`` = encoded BAM records already in
+  coordinate order (bytes).  -> number of records."""
+  L = _lib.lib()
+  names = (C.c_char_p * max(1, len(contigs)))(*[str(n).encode() for n, _ in contigs])
+  lens = np.ascontiguousarray([int(l) for _, l in contigs] or [0], dtype=np.int64)
+  buf = np.frombuffer(bytes(records) or b'\0', dtype=np.uint8)
+  n = C.c_int64(0)
+  rc = L.mg_bam_write_sorted(str(bam).encode(), str(bai).encode() if bai else None, len(contigs), names, _ptr(lens), header_text.encode(),
+                             _ptr(buf), len(records), int(level), int(threads), C.byref(n))
+  if rc != 0:
+    raise (ValueError if rc == _lib.MG_EVALUE else RuntimeError)('mitty_b200: cannot write {} (rc={})'.format(bam, rc))
+  return n.value
+
+
 class Sink(object):
   """The native output sink (mg_sink_*): writer threads inside the library put the units into the two
   FASTQ files in schedule order -- pwrite for regular files, ordered sequential writes for FIFOs /

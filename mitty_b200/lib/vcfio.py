@@ -541,6 +541,10 @@ class FastaFile(object):
   def references(self):
     return list(self._lengths) if self._h is not None else list(self._seqs)
 
+  def get_reference_length(self, reference):
+    """Length of a contig (pysam.FastaFile.get_reference_length)."""
+    return self._lengths[reference] if self._h is not None else len(self._contig(reference))
+
   def close(self):
     if self._h is not None:
       self._L.mg_fasta_close(self._h)
