@@ -221,29 +221,30 @@ MG_HD uint32_t mg_permute(uint32_t i, uint32_t n, uint32_t bits, uint32_t k0, ui
 // ------------------------------------------------------------------------------------------
 // Decimal helpers
 
-MG_HD uint32_t mg_pow10(int d) {   // 10^d for d in 0..9
-  switch (d) {
-    case 0: return 1u; case 1: return 10u; case 2: return 100u; case 3: return 1000u; case 4: return 10000u;
-    case 5: return 100000u; case 6: return 1000000u; case 7: return 10000000u; case 8: return 100000000u;
-    default: return 1000000000u;
-  }
+// No branch and no table in the digit counts below: a switch, or a table indexed per lane, serialises the lanes
+// of a warp that hold numbers of different lengths.
+MG_HD uint32_t mg_pow10(uint32_t d) {   // 10^d for d in 0..9, selected by the bits of d
+  return ((d & 1u) ? 10u : 1u) * ((d & 2u) ? 100u : 1u) * ((d & 4u) ? 10000u : 1u) * ((d & 8u) ? 100000000u : 1u);
 }
 
-// decimal digits of v, and (ones) the number 11..1 with as many ones: no branch, no table (a switch or a table
-// indexed per lane serialises the lanes of a warp that hold numbers of different lengths)
+MG_HD uint32_t mg_bit_length(uint32_t v) {   // bits of v, v != 0
+#if defined(__CUDA_ARCH__)
+  return 32u - (uint32_t)__clz((int)v);
+#else
+  return 32u - (uint32_t)__builtin_clz(v);
+#endif
+}
+
+// decimal digits of v, and (ones) the number 11..1 with as many ones.  With b = bits of v, t = floor(b log10 2)
+// (1233 / 4096 is log10 2 rounded down, exact enough for b <= 32) and v has t or t + 1 digits: t + 1 when
+// v >= 10^t.  v | 1 has the digits of v (a power of ten above 1 is even) and makes 0 one digit.
 MG_HD int mg_ndigits_ones(uint32_t v, uint32_t &ones) {
-  int d = 1; uint32_t o = 1u;
-  if (v >= 10u) { d++; o += 10u; }
-  if (v >= 100u) { d++; o += 100u; }
-  if (v >= 1000u) { d++; o += 1000u; }
-  if (v >= 10000u) { d++; o += 10000u; }
-  if (v >= 100000u) { d++; o += 100000u; }
-  if (v >= 1000000u) { d++; o += 1000000u; }
-  if (v >= 10000000u) { d++; o += 10000000u; }
-  if (v >= 100000000u) { d++; o += 100000000u; }
-  if (v >= 1000000000u) { d++; o += 1000000000u; }
-  ones = o;
-  return d;
+  const uint32_t w = v | 1u;
+  const uint32_t t = (mg_bit_length(w) * 1233u) >> 12;
+  const uint32_t p = mg_pow10(t);
+  const bool up = w >= p;
+  ones = (p - 1u) / 9u + (up ? p : 0u);                     // 11..1 with t ones, plus 10^t for one digit more
+  return (int)(t + (up ? 1u : 0u));
 }
 
 MG_HD int mg_ndigits32(uint32_t v) { uint32_t o; return mg_ndigits_ones(v, o); }
@@ -519,7 +520,10 @@ MG_HD void mg_put_i32(W &w, int32_t v) {
   if (v < 0) { w.put('-'); mg_put_u32(w, (uint32_t)(-(int64_t)v)); } else mg_put_u32(w, (uint32_t)v);
 }
 
-MG_HD int mg_nchars_i32(int32_t v) { return v < 0 ? 1 + mg_ndigits32((uint32_t)(-(int64_t)v)) : mg_ndigits32((uint32_t)v); }
+MG_HD int mg_nchars_i32(int32_t v) {   // one digit count for either sign
+  const bool neg = v < 0;
+  return (neg ? 1 : 0) + mg_ndigits32(neg ? (uint32_t)(-(int64_t)v) : (uint32_t)v);
+}
 
 // length of '|strand|pos|rlen|cigar|vlist' for one read; L_nd = decimal digits of L
 template <class NP>

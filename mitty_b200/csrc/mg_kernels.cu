@@ -621,64 +621,103 @@ struct Agg { unsigned long long c1, c2, by; };
 #define DESC_MASK62 ((1ull << 62) - 1ull)
 
 // Exclusive prefix of (c1, c2, bytes) over all tiles before `tile` (decoupled look-back), computed
-// by one whole warp; every lane returns the same sums.
+// by one whole warp; every lane returns the same sums.  One round reads a window of LOOKBACK_WIN
+// descriptors (LOOKBACK_WIN / 32 per lane, all loads in flight at once) and stops at the nearest
+// inclusive one.  The window bounds how fast inclusive prefixes can propagate: about one window of tiles
+// per L2 round trip.  At 32 tiles that is close to the rate at which tiles finish on 148 SMs.
+#define LOOKBACK_WIN 128
 __device__ Agg tile_lookback(const MgUnitParams &P, int tile, int lane) {
+  constexpr int Q = LOOKBACK_WIN / 32;
   Agg ex = {0, 0, 0};
   int idx = tile - 1;
   while (true) {
-    int t = idx - lane;
-    unsigned long long a = 0, b = 0;
-    uint32_t fl = 2;  // tiles before 0 behave like an all-zero inclusive prefix
-    if (t >= 0) {
-      do {
-        a = ld_vol64(P.descA + t);
-        b = ld_vol64(P.descB + t);
-      } while (DESC_FLAG(a) == 0 || DESC_FLAG(a) != DESC_FLAG(b));
-      fl = DESC_FLAG(a);
+    unsigned long long a[Q], b[Q];
+#pragma unroll
+    for (int q = 0; q < Q; q++) {
+      const int t = idx - 32 * q - lane;
+      a[q] = 2ull << 62; b[q] = 2ull << 62;   // tiles before 0 behave like an all-zero inclusive prefix
+      if (t >= 0) { a[q] = ld_vol64(P.descA + t); b[q] = ld_vol64(P.descB + t); }
+    }
+#pragma unroll
+    for (int q = 0; q < Q; q++) {
+      const int t = idx - 32 * q - lane;
+      while (t >= 0 && (DESC_FLAG(a[q]) == 0 || DESC_FLAG(a[q]) != DESC_FLAG(b[q]))) {
+        a[q] = ld_vol64(P.descA + t); b[q] = ld_vol64(P.descB + t);
+      }
     }
     __syncwarp();
-    uint32_t pm = __ballot_sync(FULL, fl == 2);
-    int first = __ffs(pm) - 1;
-    bool take = (t >= 0) && (first < 0 || lane <= first);
-    unsigned long long c1 = take ? ((a >> 31) & 0x7FFFFFFFull) : 0;
-    unsigned long long c2 = take ? (a & 0x7FFFFFFFull) : 0;
-    unsigned long long by = take ? (b & DESC_MASK62) : 0;
+    int stop = LOOKBACK_WIN;   // window position (32 q + lane) of the nearest inclusive descriptor
+#pragma unroll
+    for (int q = Q - 1; q >= 0; q--) {
+      const uint32_t pm = __ballot_sync(FULL, DESC_FLAG(a[q]) == 2);
+      if (pm) stop = 32 * q + __ffs(pm) - 1;
+    }
+    unsigned long long c1 = 0, c2 = 0, by = 0;
+#pragma unroll
+    for (int q = 0; q < Q; q++) {
+      if (32 * q + lane <= stop) {   // (the all-zero stand-ins before tile 0 add nothing)
+        c1 += (a[q] >> 31) & 0x7FFFFFFFull; c2 += a[q] & 0x7FFFFFFFull; by += b[q] & DESC_MASK62;
+      }
+    }
     ex.c1 += warp_sum_u64(c1); ex.c2 += warp_sum_u64(c2); ex.by += warp_sum_u64(by);
-    if (first >= 0) break;
-    idx -= 32;
+    if (stop < LOOKBACK_WIN) break;
+    idx -= LOOKBACK_WIN;
   }
   return ex;
 }
 
 // ---- k_unit_plan ---------------------------------------------------------------------------
-// Phase 1 of a unit: one candidate per thread (sampling, te < p_max, N filter, node lookup, record
+// Phase 1 of a unit: one candidate per thread (sampling, te < p_max / N filter, node lookup, record
 // size), block scan, decoupled look-back, and one 32-byte MgPlan per KEPT template at its final
-// rank.  Small per-thread state, no staging memory: runs at high occupancy, which hides the
-// dependent L2 loads of the node / template-start gathers.
+// rank.  Small per-thread state: runs at high occupancy, which hides the dependent L2 loads of the
+// node / template-start gathers.
+//
+// One block barrier per tile, and no warp waits for a look-back right after its tile's aggregate went
+// out.  Iteration k of a CTA does the candidates of its tile T_k; warp 0 then does the look-back of
+// T_{k-1}, whose aggregate went out one iteration earlier.  After the barrier every thread writes its
+// plan of T_{k-1} (parked in shared memory since then) and thread 0 publishes T_k's aggregate.  So
+// the other warps spend the look-back on their next candidates, and a look-back starts a whole tile
+// of work after the aggregates it reads were due.  The next tile is claimed one iteration ahead,
+// off the barrier.
+//
+// Deadlock freedom: tiles are claimed from an atomic counter, so every tile below a claimed one has
+// been claimed by a CTA that is running (a CTA exits only after the plans of all its tiles).  The
+// look-back of a tile T waits only for aggregates of tiles below T.  The aggregate of a tile U goes
+// out once its CTA has done the look-back of its previous tile, which is below U.  By induction on the
+// tile index every look-back ends, whichever CTAs are resident.
 #define PLAN_THREADS 256
 
-__global__ void __launch_bounds__(PLAN_THREADS) k_unit_plan(const __grid_constant__ MgUnitParams P) {
+// 40 registers, six CTAs per SM (the look-back's window spills a few words to L1 at that bound; eight CTAs at
+// 32 registers spill 68 bytes and measured slower)
+__global__ void __launch_bounds__(PLAN_THREADS, 6) k_unit_plan(const __grid_constant__ MgUnitParams P) {
   __shared__ uint32_t s_tlen[MG_TLEN_K];
-  __shared__ uint32_t s_wc[PLAN_THREADS / 32], s_ws[PLAN_THREADS / 32];
-  __shared__ unsigned long long s_base[3];
-  __shared__ uint32_t s_tile;
+  // each thread's candidate of T_{k-1}: {xa, xb, n0a, n0b}, {dn, fo << 31 | ta << 30 | tb << 29 | sz}, and its
+  // exclusive (ec, es) inside the tile
+  __shared__ uint4 s_hold[2][PLAN_THREADS];
+  __shared__ uint2 s_hold2[2][PLAN_THREADS], s_ex[PLAN_THREADS];
+  __shared__ uint32_t s_wc[2][PLAN_THREADS / 32], s_ws[2][PLAN_THREADS / 32];
+  __shared__ unsigned long long s_base[2][3];
+  __shared__ uint32_t s_tile[2];
   const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
   const int L = P.rlen;
   if (P.mode == MG_MODE_PHILOX && P.tlen_alias) {
 #pragma unroll 1
     for (int i = t; i < MG_TLEN_K; i += PLAN_THREADS) s_tlen[i] = P.tlen_alias[i];
   }
-  while (true) {
-    __syncthreads();
-    if (t == 0) s_tile = atomicAdd(P.tile_counter, 1u);
-    __syncthreads();
-    const int tile = (int)s_tile;
-    if (tile >= P.n_tiles) break;
+  if (t == 0) s_tile[0] = atomicAdd(P.tile_counter, 1u);
+  __syncthreads();
+  int tile = (int)s_tile[0], prev = -1;
+  uint32_t prev_c1 = 0, prev_c2 = 0, prev_sz = 0;       // aggregate of T_{k-1}
+#pragma unroll 1
+  for (int k = 0;; k++) {
+    const int cur = k & 1;
+    const bool live = tile < P.n_tiles;
+    if (t == 0 && live) s_tile[cur ^ 1] = atomicAdd(P.tile_counter, 1u);
     const uint32_t j = (uint32_t)tile * PLAN_THREADS + t;
     bool k1 = false, k2 = false, ta = false, tb = false;
     uint32_t xa = 0, xb = 0, fo = 0, sz = 0;
     int n0a = 0, n1a = 0, n0b = 0, n1b = 0;
-    if (j < P.n_cand) {
+    if (live && j < P.n_cand) {
       Cand c = sample_candidate(P, s_tlen, j);
       k1 = c.k1; fo = c.fo;
       if (k1) {
@@ -699,57 +738,79 @@ __global__ void __launch_bounds__(PLAN_THREADS) k_unit_plan(const __grid_constan
         }
       }
     }
-    // block scan of (k1 | k2 << 16, sz)
+    s_hold[cur][t] = make_uint4(xa, xb, (uint32_t)n0a, (uint32_t)n0b);
+    s_hold2[cur][t] = make_uint2((uint32_t)(n1a - n0a) | ((uint32_t)(n1b - n0b) << 16),
+                                 (fo << 31) | ((ta ? 1u : 0u) << 30) | ((tb ? 1u : 0u) << 29) | sz);
+    // warp scans of (k1 | k2 << 16, sz) over T_k
     const uint32_t cpk = (k1 ? 1u : 0u) | (k2 ? 0x10000u : 0u);
     const uint32_t ic = warp_incl_scan_u32(cpk, lane), is = warp_incl_scan_u32(sz, lane);
-    if (lane == 31) { s_wc[wid] = ic; s_ws[wid] = is; }
+    if (lane == 31) { s_wc[cur][wid] = ic; s_ws[cur][wid] = is; }
+    // warp 0: exclusive prefix of T_{k-1}, and its inclusive descriptor
+    if (wid == 0 && prev >= 0) {
+      Agg ex = {0, 0, 0};
+      if (prev > 0) ex = tile_lookback(P, prev, lane);
+      if (lane == 0) {
+        const unsigned long long i1 = ex.c1 + prev_c1, i2 = ex.c2 + prev_c2, ib = ex.by + prev_sz;
+        if (prev > 0) {                                                          // tile 0 went out inclusive
+          st_vol64(P.descA + prev, (2ull << 62) | (i1 << 31) | i2);
+          st_vol64(P.descB + prev, (2ull << 62) | ib);
+        }
+        s_base[cur ^ 1][0] = ex.c1; s_base[cur ^ 1][1] = ex.c2; s_base[cur ^ 1][2] = ex.by;
+        if (prev == P.n_tiles - 1) { P.totals[0] = i1; P.totals[1] = i2; P.totals[2] = ib + mg_digit_sum(i2); }
+      }
+    }
     __syncthreads();
+    // the plans of T_{k-1}
+    if (prev >= 0) {
+      const uint2 h1 = s_hold2[cur ^ 1][t];
+      if (h1.y & 0x1FFFFFFFu) {                                                  // sz != 0: kept
+        const uint4 h0 = s_hold[cur ^ 1][t];
+        const uint2 ex = s_ex[t];
+        const unsigned long long base1 = s_base[cur ^ 1][0], base2 = s_base[cur ^ 1][1];
+        const unsigned long long rank = base2 + (ex.x >> 16);                    // cnt - 1, readgenerate.py:209
+        // the serial's digits change the record size: offset = scanned bytes + sum of digits of 1..rank
+        const unsigned long long off = s_base[cur ^ 1][2] + ex.y + mg_digit_sum(rank);
+        const uint32_t my_fo = (P.mode == MG_MODE_PHILOX) ? h1.y >> 31 : (uint32_t)(P.fo_in[base1 + (ex.x & 0xFFFFu)] & 1);   // illumina.py:93
+        MgPlan pl;
+        pl.xa = h0.x; pl.xb = h0.y; pl.n0a = (int32_t)h0.z; pl.n0b = (int32_t)h0.w;
+        pl.dn = h1.x;
+        pl.fo_sz = (my_fo << 31) | ((h1.y & 0x7FFFFFFFu) + (uint32_t)mg_ndigits32((uint32_t)(rank + 1)));
+        pl.off = off;
+        P.plan[rank] = pl;
+      }
+    }
+    if (!live) break;
+    // T_k: offsets inside the tile, its aggregate; tile 0 has its inclusive prefix already
     uint32_t oc = 0, os = 0, tc = 0, ts_ = 0;
 #pragma unroll
     for (int w = 0; w < PLAN_THREADS / 32; w++) {
-      if (w < wid) { oc += s_wc[w]; os += s_ws[w]; }
-      tc += s_wc[w]; ts_ += s_ws[w];
+      if (w < wid) { oc += s_wc[cur][w]; os += s_ws[cur][w]; }
+      tc += s_wc[cur][w]; ts_ += s_ws[cur][w];
     }
     const uint32_t ec = oc + ic - cpk, es = os + is - sz;   // exclusive
-    const uint32_t tile_c1 = tc & 0xFFFFu, tile_c2 = tc >> 16, tile_sz = ts_;
-    if (wid == 0) {
-      Agg ex = {0, 0, 0};
-      if (tile > 0) {
-        if (lane == 0) {
-          st_vol64(P.descA + tile, (1ull << 62) | ((unsigned long long)tile_c1 << 31) | tile_c2);
-          st_vol64(P.descB + tile, (1ull << 62) | tile_sz);
-        }
-        ex = tile_lookback(P, tile, lane);
-      }
-      if (lane == 0) {
-        const unsigned long long i1 = ex.c1 + tile_c1, i2 = ex.c2 + tile_c2, ib = ex.by + tile_sz;
-        st_vol64(P.descA + tile, (2ull << 62) | (i1 << 31) | i2);
-        st_vol64(P.descB + tile, (2ull << 62) | ib);
-        s_base[0] = ex.c1; s_base[1] = ex.c2; s_base[2] = ex.by;
-        if (tile == P.n_tiles - 1) { P.totals[0] = i1; P.totals[1] = i2; P.totals[2] = ib + mg_digit_sum(i2); }
-      }
+    prev_c1 = tc & 0xFFFFu; prev_c2 = tc >> 16; prev_sz = ts_;
+    if (t == 0) {
+      const unsigned long long fl = tile == 0 ? 2ull << 62 : 1ull << 62;
+      st_vol64(P.descA + tile, fl | ((unsigned long long)prev_c1 << 31) | prev_c2);
+      st_vol64(P.descB + tile, fl | prev_sz);
     }
-    __syncthreads();
-    if (k2) {
-      const unsigned long long base1 = s_base[0], base2 = s_base[1];
-      const unsigned long long rank = base2 + (ec >> 16);                        // cnt - 1, readgenerate.py:209
-      // the serial's digits change the record size: offset = scanned bytes + sum of digits of 1..rank
-      const unsigned long long off = s_base[2] + es + mg_digit_sum(rank);
-      const uint32_t my_fo = (P.mode == MG_MODE_PHILOX) ? fo : (uint32_t)(P.fo_in[base1 + (ec & 0xFFFFu)] & 1);   // illumina.py:93
-      MgPlan pl;
-      pl.xa = xa; pl.xb = xb; pl.n0a = n0a; pl.n0b = n0b;
-      pl.dn = (uint32_t)(n1a - n0a) | ((uint32_t)(n1b - n0b) << 16);
-      pl.fo_sz = (my_fo << 31) | ((ta ? 1u : 0u) << 30) | ((tb ? 1u : 0u) << 29) | (sz + (uint32_t)mg_ndigits32((uint32_t)(rank + 1)));
-      pl.off = off;
-      P.plan[rank] = pl;
-    }
+    s_ex[t] = make_uint2(ec, es);
+    prev = tile;
+    tile = (int)s_tile[cur ^ 1];
   }
 }
 
 void mg_launch_plan(const MgUnitParams &P, cudaStream_t st) {
   if (P.n_tiles == 0) return;
-  int grid = P.n_tiles < 148 * 8 ? P.n_tiles : 148 * 8;
-  k_unit_plan<<<grid, PLAN_THREADS, 0, st>>>(P);
+  // as many CTAs as are resident at once: a later one would find the tile counter exhausted
+  static const int resident = [] {
+    int dev = 0, sms = 0, per_sm = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_unit_plan, PLAN_THREADS, 0);
+    return std::max(1, sms * per_sm);
+  }();
+  k_unit_plan<<<std::min(P.n_tiles, resident), PLAN_THREADS, 0, st>>>(P);
 }
 
 // ---- k_batch_plan --------------------------------------------------------------------------
