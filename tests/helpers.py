@@ -106,6 +106,36 @@ def model(name):
   return load_model(name)
 
 
+def dense_variant_region(seed, alt_n=True):
+  """A 6 kb contig with N / IUPAC / soft-masked bytes and a variant set built to stress the greedy skip
+  rule (rpc.py:55): long deletions that swallow runs of later variants, chains of overlapping deletions,
+  several records at one POS, non-ACGT bytes in ALT alleles.  seed 1..4 sets the density and the longest
+  deletion.  alt_n=False puts Y where the ALT alleles would have N (same positions and lengths), so that
+  reads are not dropped by the N filter.  -> (region bytes, BED start, VariantList, number of records)."""
+  rs = np.random.RandomState(seed)
+  n = 6000
+  ref = synth.synth_contig(n, seed=100 + seed)
+  ref[1000:1100] = ord('N'); ref[3000] = ord('R'); ref[3500:3503] = ord('n')
+  bed_start = 40
+  recs = []
+  for _ in range([400, 1500, 3000, 800][seed - 1]):
+    pos = int(rs.randint(1, n - 560))                 # no deletion reaches the region end
+    kind = rs.randint(0, 3)
+    r0 = chr(ref[pos - 1]).upper()
+    r0 = r0 if r0 in 'ACGT' else 'A'
+    if kind == 0:
+      recs.append((pos, r0, ('ACGTN' if alt_n else 'ACGTY')[rs.randint(0, 5)], 'X', 0))
+    elif kind == 1:
+      ol = int(rs.randint(1, 40))
+      recs.append((pos, r0, r0 + ''.join(('ACGTRN' if alt_n else 'ACGTRY')[i] for i in rs.randint(0, 6, size=ol)), 'I', ol))
+    else:
+      ol = int(rs.randint(1, [8, 30, 50, 200][seed - 1]))
+      recs.append((pos, 'A' * (ol + 1), 'A', 'D', ol))
+  recs.sort(key=lambda t: t[0])                       # stable: records at one POS keep their order
+  vl = vcfio.VariantList.from_variants([vcfio.Variant(*t) for t in recs])
+  return np.ascontiguousarray(ref[bed_start:n - 300]), bed_start, vl, len(recs)
+
+
 # ---- god-aligner style round trip -------------------------------------------------------------------
 
 class HaplotypeIndex(object):

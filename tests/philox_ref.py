@@ -3,6 +3,8 @@ MgCorruptCtx in mitty_b200/csrc/mg_core.cuh): one Philox4x32-7 block per four cy
 word and one lookup in a Vose alias row over the joint outcomes (quality, substitution) per base.
 Test infrastructure: lets the fused GPU path and the standalone corrupt kernel be checked byte for
 byte, not only statistically."""
+import re
+
 import numpy as np
 
 M0, M1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57)
@@ -152,9 +154,17 @@ BASES = b'ACGT'
 CODE = {65: 0, 67: 1, 71: 2, 84: 3}
 
 
-def corrupt_file(fq, f, tables, k0, k1, serials=None):
+def record_name(header):
+  """FastxFile's .name of a header line: the bytes after its first one, up to the first space, tab or CR."""
+  return re.split(b'[ \t\r]', header[1:], maxsplit=1)[0]
+
+
+def corrupt_file(fq, f, tables, k0, k1, serials=None, names_from=None):
   """Corrupt a perfect FASTQ buffer (file index f) -> bytes.  tables = (alias, kshift, code9).
-  serials: per-record template serial (default 0..n-1, the standalone kernel's numbering)."""
+  serials: per-record template serial (default 0..n-1, the standalone kernel's numbering).
+  names_from: FASTQ buffer whose record names head the output records, '@' + record_name() -- the
+  standalone corrupt-reads writes read 1's name on both files (readcorrupt.py:113); default: every
+  record keeps its own header line, as the fused emit kernel does."""
   alias, kshift, code9 = tables
   qb = 7 if code9 else 6
   cb = 9 if code9 else 8
@@ -162,6 +172,10 @@ def corrupt_file(fq, f, tables, k0, k1, serials=None):
   n_rec = (len(lines) - 1) // 4
   if serials is None:
     serials = np.arange(n_rec, dtype=np.uint64)
+  heads = [lines[4 * rec] for rec in range(n_rec)]
+  if names_from is not None:
+    src = names_from.split(b'\n')
+    heads = [b'@' + record_name(src[4 * rec]) for rec in range(n_rec)]
   out = []
   L = max(len(lines[4 * r + 1]) for r in range(n_rec)) if n_rec else 0
   ng = (L + 3) // 4
@@ -184,5 +198,5 @@ def corrupt_file(fq, f, tables, k0, k1, serials=None):
     for n in np.flatnonzero(s):
       c = CODE.get(seq[n])
       seq[n] = ord('N') if c is None else BASES[c ^ int(s[n])]
-    out.append(lines[4 * rec] + b'\n' + bytes(seq) + b'\n+\n' + (q + 33).astype(np.uint8).tobytes() + b'\n')
+    out.append(heads[rec] + b'\n' + bytes(seq) + b'\n+\n' + (q + 33).astype(np.uint8).tobytes() + b'\n')
   return b''.join(out)

@@ -88,30 +88,9 @@ def test_device_walk_dense_overlapping_variants(eng, seed):
   runs of later variants, chains of overlapping deletions, several records at one POS, variants
   before the region start, non-ACGT bytes in ALT alleles and in the reference."""
   import mitty_b200.simulation.rpc as rpc
-  rs = np.random.RandomState(seed)
-  n = 6000
-  ref = synth.synth_contig(n, seed=100 + seed)
-  ref[1000:1100] = ord('N'); ref[3000] = ord('R'); ref[3500:3503] = ord('n')
-  bed_start = 40
-  recs = []
-  for _ in range([400, 1500, 3000, 800][seed - 1]):
-    pos = int(rs.randint(1, n - 560))                 # no deletion reaches the region end (that case is rejected, below)
-    kind = rs.randint(0, 3)
-    r0 = chr(ref[pos - 1]).upper()
-    r0 = r0 if r0 in 'ACGT' else 'A'
-    if kind == 0:
-      recs.append((pos, r0, 'ACGTN'[rs.randint(0, 5)], 'X', 0))
-    elif kind == 1:
-      ol = int(rs.randint(1, 40))
-      recs.append((pos, r0, r0 + ''.join('ACGTRN'[i] for i in rs.randint(0, 6, size=ol)), 'I', ol))
-    else:
-      ol = int(rs.randint(1, [8, 30, 50, 200][seed - 1]))
-      recs.append((pos, 'A' * (ol + 1), 'A', 'D', ol))
-  recs.sort(key=lambda t: t[0])                       # stable: records at one POS keep their order
-  region = ref[bed_start:n - 300]
-  vl = vcfio.VariantList.from_variants([vcfio.Variant(*t) for t in recs])
+  region, bed_start, vl, n_recs = H.dense_variant_region(seed)
   want = oracle.create_node_list(region, bed_start + 1, H.oracle_cv(vl))
-  assert want[-1][2] == '=' and sum(1 for w in want if w[2] != '=') < len(recs)     # some records were skipped
+  assert want[-1][2] == '=' and sum(1 for w in want if w[2] != '=') < n_recs     # some records were skipped
   nl = rpc.create_node_list(region, bed_start + 1, vl, engine=eng)
   assert nl.tuples() == want
   # the materialised haplotype (with its non-ACGT exception runs) is the concatenation of the node sequences
@@ -155,7 +134,7 @@ def test_generate_reads_plugin_golden(eng):
 
 # ---- explicit templates: every corner of the emit kernel -------------------------------------------
 
-@pytest.mark.parametrize('L', [150, 37, 16, 1, 250])
+@pytest.mark.parametrize('L', [150, 37, 16, 1, 250, 161, 162, 305, 306])   # 161/162, 305/306: both sides of the register-window switches
 def test_edge_units_explicit(eng, L):
   from mitty_b200.engine import MODE_EXPLICIT
   regs = H.workload_regions(synth.edge_workload())
@@ -428,14 +407,23 @@ def test_tumor_normal_viral_mix(tmp_path):
   assert 0.006 < frac < 0.014, frac
 
 
-def test_corrupt_reads_edge_inputs(tmp_path):
+def test_corrupt_reads_edge_inputs(eng, tmp_path):
   """corrupt-reads on the inputs the reference's reader loop meets (readcorrupt.py:49-55): empty
   files, single-end input, ragged read lengths in one file, a second file with fewer records (zip
-  truncation), a last record without a trailing newline -- deterministic mode == the oracle."""
+  truncation), a last record without a trailing newline -- deterministic mode == the oracle, production
+  mode == the numpy specification."""
   import mitty_b200.simulation.illumina as il
   import mitty_b200.simulation.readcorrupt as rc
+  from tests import philox_ref as PR
   m = H.model('hiseq-X-v2.5-Garvan.pkl')
+  eng.load_model(m)
+  tables = eng.model_tables(1)
   rs = np.random.RandomState(3)
+
+  def first_records(b, n):
+    """The first n records of a FASTQ buffer, newline-terminated."""
+    lines = (b if b.endswith(b'\n') else b + b'\n').split(b'\n')
+    return b''.join(x + b'\n' for x in lines[:4 * n])
 
   def fq(lengths, tag, newline=True):
     recs = []
@@ -464,14 +452,17 @@ def test_corrupt_reads_edge_inputs(tmp_path):
     assert open(o1, 'rb').read() == want1, name
     if b2 is not None:
       assert open(o2, 'rb').read() == want2, name
-    # production mode: same framing (names, lengths), deterministic for a seed, independent of the chunk size
+    # production mode: == the numpy specification (key 0x636f7232, read 1's name on both files), independent of the chunk size
     p1, p2 = str(tmp_path / (name + '.1.p.fq')), (str(tmp_path / (name + '.2.p.fq')) if b2 is not None else None)
     q1, q2 = str(tmp_path / (name + '.1.q.fq')), (str(tmp_path / (name + '.2.q.fq')) if b2 is not None else None)
     rc.multi_process(il, m, i1, p1, i2, p2, processes=1, seed=11)
     rc.multi_process(il, m, i1, q1, i2, q2, processes=1, seed=11, chunk_bytes=700)
     assert open(p1, 'rb').read() == open(q1, 'rb').read(), name
-    got = open(p1, 'rb').read().split(b'\n')
-    assert [len(x) for x in got] == [len(x) for x in want1.split(b'\n')] and got[0::4] == want1.split(b'\n')[0::4], name
+    r1 = first_records(b1, n)
+    assert open(p1, 'rb').read() == PR.corrupt_file(r1, 0, tables, 11, 0x636f7232, names_from=r1), name
+    if b2 is not None:
+      assert open(p2, 'rb').read() == open(q2, 'rb').read(), name
+      assert open(p2, 'rb').read() == PR.corrupt_file(first_records(b2, n), 1, tables, 11, 0x636f7232, names_from=r1), name
 
 
 def test_bed_cutting_through_a_deletion(tmp_path, caplog):

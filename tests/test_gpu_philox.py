@@ -178,7 +178,10 @@ def test_philox_large_unit_exact(eng):
                                                   (synth.softmask_workload, 0, 'hiseq-X-v2.5-Garvan.pkl'),
                                                   (synth.edge_workload, 0, '1kg-pcr-free.pkl'),   # 2x250: the wide register window, 256-entry rows
                                                   (synth.edge_workload, 1, 'hiseq-2500-v1-pcr-free.pkl'),
-                                                  (synth.edge_workload, 1, 'hiseq-X-v2.5-Garvan.pkl:200')])   # reads longer than max_rlen: BQ 93, 9-bit codes
+                                                  (synth.edge_workload, 1, 'hiseq-X-v2.5-Garvan.pkl:200'),   # reads longer than max_rlen: BQ 93, 9-bit codes
+                                                  (synth.edge_workload, 1, 'hiseq-X-v2.5-Garvan.pkl:161'),   # both sides of the first register-window switch
+                                                  (synth.edge_workload, 1, 'hiseq-X-v2.5-Garvan.pkl:162'),
+                                                  (synth.edge_workload, 1, 'hiseq-X-v2.5-Garvan.pkl:300')])   # the wide window at the model's last cycle
 def test_philox_corruption_exact_vs_numpy_spec(eng, wl_fn, cpy, model_name):
   """Production-mode corruption is fully specified (Philox counters, one joint alias row per (mate,
   cycle)): the fused emit kernel and the standalone corrupt kernel must reproduce the numpy
