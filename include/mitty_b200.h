@@ -273,6 +273,32 @@ void mg_bam_abort(mg_bam *b);
 int mg_bam_write_sorted(const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
                         const char *header_text, const uint8_t *records, int64_t len, int32_t level, int32_t threads, int64_t *n_records);
 
+/* ---- bam2illumina: replaces mitty/empirical/bam2illumina.py -- the per-base counts of an Illumina read model
+ * over every alignment record of a BGZF BAM file or FIFO (any sort order, no index).  Host threads
+ * (`threads`) inflate the BGZF members into page-locked chunks of about chunk_bytes; each chunk of whole
+ * records is copied to the device and counted there while the next one is inflated.  Record k (0-based,
+ * file order) is considered iff k % every == 0; it is skipped for flag & 0xB04, mapq < min_mq, l_seq == 0,
+ * missing QUAL (0xFF) or l_seq > max_bp, in that order; otherwise mate = (flag & 0xC1) == 0x81, base i of
+ * SEQ is cycle l_seq - 1 - i on the reverse strand (else i), and
+ *   bq_mat[mate][cycle][min(qual, 93)] += 1   u64[2][max_bp][94]
+ *   len_hist[l_seq] += 1                      u64[max_bp + 1]
+ *   tlen[|TLEN|] += 1 for (flag & 0xC1) == 0x41 and |TLEN| < max_tlen      u64[max_tlen]
+ * counts[12]: records, considered, counted, skipped for flag / mapq / empty SEQ / missing QUAL / length,
+ * inflated bytes, compressed bytes, EOF member present (1 / 0), chunks.  times[6] ms: reading the file,
+ * inflating (wall), walking the record chain, host-to-device copies, kernels (CUDA events), the whole call.  thread_ms[threads]
+ * (may be NULL): busy time of each inflate thread.  Malformed input is MG_EVALUE with bad_code (1 not gzip,
+ * 2 no BC subfield, 3 corrupt or truncated member, 4 CRC32, 5 ISIZE, 6 not a BAM header, 7 file ends in the
+ * header, 10 read error: bad_where = compressed offset of the member; 8 block_size < 32, 9 file ends inside
+ * the record, 11 / 12 / 13 / 14 read name / CIGAR / SEQ / QUAL overrun block_size: bad_where = record
+ * ordinal); the first bad record in file order is reported, and no chunk after the one holding it is read.
+ * 1 <= max_bp <= 50000, 1 <= max_tlen <= 2^20 and 1 <= every <= 2^32 - 1 (MG_EINVAL otherwise).
+ * mg_bam_scan: the same reader without a device: stats[4] = records, inflated bytes, compressed bytes, EOF
+ * member present; record errors 11-14 are not checked.                                            */
+int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, int32_t max_tlen, int32_t min_mq, int64_t every, int32_t threads,
+                     int64_t chunk_bytes, uint64_t *bq_mat, uint64_t *len_hist, uint64_t *tlen, int64_t *counts, double *times,
+                     double *thread_ms, int64_t *bad_where, int32_t *bad_code);
+int mg_bam_scan(const char *path, int32_t threads, int64_t chunk_bytes, int64_t *stats, int64_t *bad_where, int32_t *bad_code);
+
 /* ---- profiling: device time (CUDA events on the launch stream) of the emit / corrupt kernel
  * (emit_ms over emit_launches launches, emit_bytes written) and of the planning kernel (plan_ms);
  * total_launches counts every kernel this context launched since the last reset.               */

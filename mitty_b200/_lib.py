@@ -11,7 +11,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_HERE, 'csrc')
 SO_PATH = os.path.join(_HERE, 'libmitty_b200.so')
-SOURCES = ['mg_api.cu', 'mg_kernels.cu', 'mg_check.cu', 'mg_bam.cu', 'mg_sink.cpp', 'mg_bgzf.cpp', 'mg_fasta.cpp']
+SOURCES = ['mg_api.cu', 'mg_kernels.cu', 'mg_check.cu', 'mg_bam.cu', 'mg_readmodel.cu', 'mg_sink.cpp', 'mg_bgzf.cpp', 'mg_fasta.cpp']
 HEADERS = ['mg_core.cuh', 'mg_internal.h', 'mg_qname.cuh', 'mg_bgzf.h', 'mg_deflate.h', 'mg_sink.cpp', 'mg_check.cu', 'mg_fasta.cpp', os.path.join('..', '..', 'include', 'mitty_b200.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared', '-lz']
@@ -28,7 +28,8 @@ SYMBOLS = ['mg_device_count', 'mg_ctx_create', 'mg_ctx_destroy', 'mg_last_error'
            'mg_batch_build', 'mg_batch_free', 'mg_batch_generate',
            'mg_fasta_open', 'mg_fasta_close', 'mg_fasta_n_contigs', 'mg_fasta_contig', 'mg_fasta_fetch',
            'mg_check_open', 'mg_check_close', 'mg_check_add_copy', 'mg_check_fastq',
-           'mg_bam_open', 'mg_bam_add', 'mg_bam_close', 'mg_bam_abort', 'mg_bam_write_sorted']
+           'mg_bam_open', 'mg_bam_add', 'mg_bam_close', 'mg_bam_abort', 'mg_bam_write_sorted',
+           'mg_bam_scan', 'mg_readmodel_bam']
 
 
 class UnitDesc(C.Structure):
@@ -143,5 +144,8 @@ def lib():
     L.mg_bam_abort.restype = None
     L.mg_bam_write_sorted.argtypes = [C.c_char_p, C.c_char_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64, C.c_int32,
                                       C.c_int32, C.POINTER(C.c_int64)]
+    L.mg_bam_scan.argtypes = [C.c_char_p, C.c_int32, C.c_int64, C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int32)]
+    L.mg_readmodel_bam.argtypes = [C.c_void_p, C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int32)]
     _lib = L
   return _lib

@@ -1,5 +1,5 @@
 """Command line with the reference's ``generate-reads`` / ``corrupt-reads`` / ``qname`` commands
-(mitty/cli.py:106-157) and ``god-aligner`` (mitty/cli.py:191-204): same positional arguments and options, plus ``--deterministic`` (consume
+(mitty/cli.py:106-157), ``god-aligner`` (mitty/cli.py:191-204) and ``create-read-model bam2illumina``: same positional arguments and options, plus ``--deterministic`` (consume
 the reference's numpy draws; byte-exact against ``mitty ... --threads 1``) and, for
 generate-reads, ``--corrupt`` (fuse the corruption model into the emit kernel)."""
 import logging
@@ -127,6 +127,35 @@ def god_aligner(fasta, fastq1, bam, fastq2, threads, device, level):
   import mitty_b200.benchmarking.god_aligner as ga
   res = ga.process_multi_threaded(fasta, bam, fastq1, fastq2, threads=threads, device=device, level=level)
   click.echo('{} records written to {} in {:0.2f}s'.format(res['records'], bam, res['seconds']))
+
+
+@cli.group('create-read-model')
+def create_read_model():
+  """Create a read model from data"""
+
+
+@create_read_model.command('bam2illumina', short_help='Create an Illumina read model from a BAM')
+@click.argument('bam', type=click.Path(exists=True))
+@click.argument('pkl', type=click.Path())
+@click.argument('description')
+@click.option('--every', type=click.IntRange(1, (1 << 32) - 1), default=1, help='Count only every Nth record (file order)')
+@click.option('--min-mq', type=click.IntRange(0), default=0, help='Skip reads with a lower mapping quality')
+@click.option('--threads', type=int, default=None, help='host inflate threads (default: the cores of the box)')
+@click.option('--max-bp', type=click.IntRange(1, 50000), default=300, help='Longest read counted (longer ones are skipped)')
+@click.option('--max-tlen', type=click.IntRange(1, 1 << 20), default=1000, help='Template lengths at or above this are not counted')
+@click.option('--device', default=0, help='CUDA device')
+def bam2illumina(bam, pkl, description, every, min_mq, threads, max_bp, max_tlen, device):
+  """Count base qualities per (mate, cycle), read lengths and template lengths of the alignments of BAM
+  (a BGZF file or FIFO, any sort order) and write them as an Illumina read model PKL for generate-reads and
+  corrupt-reads."""
+  import mitty_b200.empirical.bam2illumina as b2i
+  res = b2i.process_bam_parallel(bam, pkl, description, every=every, min_mq=min_mq, threads=threads, max_bp=max_bp, max_tlen=max_tlen,
+                                 device=device)
+  skipped = ', '.join('{} {}'.format(res['skip_' + k], why) for k, why in (
+    ('flag', 'unmapped / secondary / QC-fail / supplementary'), ('mapq', 'below --min-mq'), ('empty', 'without SEQ'),
+    ('noqual', 'without QUAL'), ('long', 'longer than --max-bp')))
+  click.echo('{} of {} records counted ({} considered) in {:0.2f}s; skipped: {}'.format(
+    res['counted'], res['records'], res['considered'], res['seconds'], skipped))
 
 
 @cli.command('corrupt-reads', short_help='Apply corruption model to FASTQ file of reads')

@@ -15,8 +15,11 @@
 #include <unistd.h>
 #include <zlib.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cerrno>
+#include <chrono>
+#include <cstdlib>
 #include <cstdio>
 #include <cstring>
 
@@ -272,4 +275,230 @@ extern "C" int mg_bam_write_sorted(const char *bam_path, const char *bai_path, i
   if (!w.open(bam_path, bai_path, mg_bam_header(header_text, names, lens), n_ref, level, threads)) { w.discard(); return MG_EVALUE; }
   if (!w.records(records, len)) { w.discard(); return MG_EVALUE; }
   return w.close(n_records) ? MG_OK : MG_EVALUE;
+}
+
+// ---- BGZF BAM reader -----------------------------------------------------------------------------
+
+namespace {
+
+double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+const int64_t kMaxMember = 65536;
+
+// -> 0: a whole member at p[0, m.bsize); > 0: bytes needed to decide; < 0: -MG_RD_* of a malformed member
+int64_t parse_member(const uint8_t *p, int64_t avail, int &hdr, int &bsize) {
+  if (avail < 12) return 12;
+  if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) return -MG_RD_GZIP;
+  const int xlen = p[10] | p[11] << 8;
+  if (avail < 12 + xlen) return 12 + xlen;
+  bsize = -1;
+  for (int i = 12; i + 4 <= 12 + xlen;) {            // subfields: SI1 SI2 SLEN data
+    const int slen = p[i + 2] | p[i + 3] << 8;
+    if (p[i] == 'B' && p[i + 1] == 'C' && slen == 2 && i + 6 <= 12 + xlen) bsize = (p[i + 4] | p[i + 5] << 8) + 1;
+    i += 4 + slen;
+  }
+  if (bsize < 0) return -MG_RD_BC;
+  if (avail < bsize) return bsize;
+  hdr = 12 + xlen;
+  for (int f : {8, 16}) {                              // FNAME, FCOMMENT: zero-terminated
+    if (!(p[3] & f)) continue;
+    while (hdr < bsize && p[hdr]) hdr++;
+    hdr++;
+  }
+  if (p[3] & 2) hdr += 2;                              // FHCRC
+  return hdr + 8 > bsize ? -MG_RD_DATA : 0;
+}
+
+}  // namespace
+
+MgBamReader::~MgBamReader() {
+  if (fd_ >= 0) ::close(fd_);
+  for (int s = 0; s < 2; s++) {
+    if (buf_[s]) release_(buf_[s]);
+    if (off_[s]) release_(off_[s]);
+  }
+}
+
+bool MgBamReader::open(const char *path, int threads, int64_t chunk_bytes, Alloc alloc, Release release) {
+  alloc_ = alloc; release_ = release;
+  threads_ = std::max(1, threads);
+  thread_ms.assign((size_t)threads_, 0.0);
+  fd_ = ::open(path, O_RDONLY);
+  if (fd_ < 0) { err = std::string("cannot open ") + path + ": " + strerror(errno); return false; }
+  const int64_t cap = std::min<int64_t>(std::max<int64_t>(chunk_bytes, 2 * kMaxMember), 1ll << 31);
+  z_.resize((size_t)(cap + 2 * kMaxMember));
+  return grow(0, cap, 0) && grow(1, cap, 0);
+}
+
+// buffer `slot` of at least `need` bytes, its first `keep` bytes kept; records are at least 36 bytes
+bool MgBamReader::grow(int slot, int64_t need, int64_t keep) {
+  if (need <= cap_[slot]) return true;
+  if (need >= (1ll << 32)) { err = "a BAM record larger than 4 GB"; return false; }
+  uint8_t *b = static_cast<uint8_t *>(alloc_((size_t)need));
+  uint32_t *o = static_cast<uint32_t *>(alloc_((size_t)(need / 36 + 2) * 4));
+  if (!b || !o) {
+    if (b) release_(b);
+    if (o) release_(o);
+    err = "out of host memory for a chunk of " + std::to_string(need) + " bytes";
+    return false;
+  }
+  if (keep) memcpy(b, buf_[slot], (size_t)keep);
+  if (buf_[slot]) { release_(buf_[slot]); release_(off_[slot]); }
+  buf_[slot] = b; off_[slot] = o; cap_[slot] = need;
+  return true;
+}
+
+// moves the unparsed compressed bytes to the front and reads until the buffer is full or the input ends
+void MgBamReader::read_more() {
+  const double t0 = now_ms();
+  memmove(z_.data(), z_.data() + zpos_, (size_t)(zend_ - zpos_));
+  zoff_ += zpos_; zend_ -= zpos_; zpos_ = 0;
+  while (zend_ < (int64_t)z_.size() && !in_eof_) {
+    const ssize_t r = ::read(fd_, z_.data() + zend_, z_.size() - (size_t)zend_);
+    if (r < 0 && errno == EINTR) continue;
+    if (r < 0) { fail(MG_RD_IO, zoff_ + zend_); in_eof_ = true; break; }
+    if (r == 0) in_eof_ = true;
+    zend_ += r;
+  }
+  read_ms += now_ms() - t0;
+}
+
+// appends whole members to b[n, cap), inflated by the thread team.  -> 1 when the next member does not fit,
+// 0 when the input has ended or a member is bad (code set; n then ends where that member's bytes would start)
+int MgBamReader::fill(uint8_t *b, int64_t &n, int64_t cap) {
+  while (true) {
+    batch_.clear();
+    int64_t out = n;
+    int state = 2;                                     // 2: the compressed buffer needs refilling
+    while (true) {
+      Member m;
+      const int64_t r = parse_member(z_.data() + zpos_, zend_ - zpos_, m.hdr, m.bsize);
+      if (r < 0) { fail((int)-r, zoff_ + zpos_); state = 0; break; }
+      if (r > 0) {
+        if (in_eof_) {
+          if (zend_ > zpos_) fail(MG_RD_DATA, zoff_ + zpos_);
+          state = 0;
+          break;
+        }
+        if (!batch_.empty()) break;
+        read_more();
+        continue;
+      }
+      m.z = z_.data() + zpos_;
+      m.crc = rd32(m.z + m.bsize - 8); m.isize = rd32(m.z + m.bsize - 4);
+      m.comp = zoff_ + zpos_;
+      if (m.isize > kMaxMember) { fail(MG_RD_ISIZE, m.comp); state = 0; break; }
+      if (out + m.isize > cap) { state = 1; break; }
+      m.out = out; out += m.isize;
+      eof_marker = m.bsize == 28 && !memcmp(m.z, kEof, 28);
+      zpos_ += m.bsize; comp_bytes += m.bsize;
+      batch_.push_back(m);
+    }
+    const int nm = (int)batch_.size();
+    if (nm) {
+      const double t0 = now_ms();
+      std::vector<int> st((size_t)nm, 0);
+      std::atomic<int> next{0};
+      auto work = [&](int t) {
+        const double w0 = now_ms();
+        for (int i; (i = next++) < nm;) {
+          const Member &m = batch_[(size_t)i];
+          const int rc = mg_inflate(m.z + m.hdr, m.bsize - m.hdr - 8, b + m.out, m.isize);
+          st[(size_t)i] = rc == 1 ? MG_RD_DATA : rc == 2 ? MG_RD_ISIZE
+                        : (uint32_t)crc32(crc32(0L, Z_NULL, 0), b + m.out, (uInt)m.isize) != m.crc ? MG_RD_CRC : MG_RD_OK;
+        }
+        thread_ms[(size_t)t] += now_ms() - w0;
+      };
+      std::vector<std::thread> team;
+      for (int t = 1; t < std::min(threads_, nm); t++) team.emplace_back(work, t);
+      work(0);
+      for (auto &x : team) x.join();
+      inflate_ms += now_ms() - t0;
+      for (int i = 0; i < nm; i++) {
+        if (st[(size_t)i] == MG_RD_OK) continue;
+        code = MG_RD_OK;                               // a bad member comes before any later framing error
+        fail(st[(size_t)i], batch_[(size_t)i].comp);
+        out = batch_[(size_t)i].out;
+        state = 0;
+        break;
+      }
+    }
+    raw_bytes += out - n;
+    n = out;
+    if (state != 2) return state;
+  }
+}
+
+// consumes BAM header bytes of b[pos, n) (magic, l_text, text, n_ref, the references) -> the new position
+int64_t MgBamReader::header(const uint8_t *b, int64_t pos, int64_t n) {
+  while (hstate_ != 3 || hskip_) {
+    if (hskip_) {
+      const int64_t t = std::min(hskip_, n - pos);
+      pos += t; hskip_ -= t;
+      if (hskip_) return pos;
+      continue;
+    }
+    if (n - pos < (hstate_ == 0 ? 8 : 4)) return pos;
+    const int32_t v = (int32_t)rd32(b + pos + (hstate_ == 0 ? 4 : 0));
+    if ((hstate_ == 0 && memcmp(b + pos, "BAM\1", 4)) || v < 0) { fail(MG_RD_MAGIC, 0); hstate_ = 3; return pos; }
+    pos += hstate_ == 0 ? 8 : 4;
+    if (hstate_ == 0) { hskip_ = v; hstate_ = 1; }
+    else if (hstate_ == 1) { hrefs_ = v; hstate_ = v ? 2 : 3; }
+    else { hskip_ = (int64_t)v + 4; if (--hrefs_ == 0) hstate_ = 3; }
+  }
+  return pos;
+}
+
+bool MgBamReader::next(int slot, MgBamChunk &c) {
+  if (code || !err.empty() || (done_ && !carry_n_)) return false;
+  if (carry_slot_ != slot && !grow(slot, carry_n_, 0)) return false;
+  if (carry_n_) memmove(buf_[slot], buf_[carry_slot_] + carry_at_, (size_t)carry_n_);
+  int64_t n = carry_n_, pos = 0, k = 0;
+  carry_n_ = 0;
+  bool stop = false;
+  while (true) {
+    const int more = done_ ? 0 : fill(buf_[slot], n, cap_[slot]);
+    if (hstate_ != 3 || hskip_) pos = header(buf_[slot], pos, n);
+    if (code == MG_RD_MAGIC) { done_ = true; break; }
+    const double t0 = now_ms();
+    while (hstate_ == 3 && !hskip_ && !stop && n - pos >= 4) {
+      __builtin_prefetch(buf_[slot] + std::min(pos + 4096, n - 1));      // the chain runs forward through memory the inflate threads wrote
+      const int32_t bs = (int32_t)rd32(buf_[slot] + pos);
+      if (bs < 32) { code = MG_RD_BLOCK; where = records + k; stop = true; break; }   // before any framing error found further on
+      if (4 + (int64_t)bs > n - pos) break;
+      off_[slot][k++] = (uint32_t)pos;
+      pos += 4 + (int64_t)bs;
+    }
+    walk_ms += now_ms() - t0;
+    if (stop || !more) { done_ = true; break; }
+    if (k) break;
+    if (pos) { memmove(buf_[slot], buf_[slot] + pos, (size_t)(n - pos)); n -= pos; pos = 0; continue; }   // header bytes only
+    if (!grow(slot, 2 * cap_[slot], n)) return false;                                               // a record larger than the buffer
+  }
+  if (done_ && !code) {
+    if (hstate_ != 3 || hskip_) fail(MG_RD_HEADER, zoff_ + zend_);
+    else if (pos < n) fail(MG_RD_CUT, records + k);
+  }
+  carry_slot_ = slot; carry_at_ = pos; carry_n_ = done_ ? 0 : n - pos;
+  if (!k) return false;
+  c.data = buf_[slot]; c.bytes = pos; c.off = off_[slot]; c.n = k; c.first = records;
+  records += k;
+  return true;
+}
+
+namespace {
+void *host_alloc(size_t n) { return malloc(n); }
+void host_release(void *p) { free(p); }
+}  // namespace
+
+extern "C" int mg_bam_scan(const char *path, int32_t threads, int64_t chunk_bytes, int64_t *stats, int64_t *bad_where, int32_t *bad_code) {
+  if (!path || !stats || !bad_where || !bad_code) return MG_EINVAL;
+  *bad_where = -1; *bad_code = 0;
+  MgBamReader rd;
+  if (!rd.open(path, threads, chunk_bytes, host_alloc, host_release)) return MG_EVALUE;
+  MgBamChunk c;
+  for (int k = 0; rd.next(k & 1, c); k++) {}
+  stats[0] = rd.records; stats[1] = rd.raw_bytes; stats[2] = rd.comp_bytes; stats[3] = rd.eof_marker;
+  if (rd.code) { *bad_where = rd.where; *bad_code = rd.code; return MG_EVALUE; }
+  return rd.err.empty() ? MG_OK : MG_EVALUE;
 }

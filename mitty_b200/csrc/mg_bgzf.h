@@ -1,5 +1,6 @@
-// BGZF writer and BAI builder of the god-aligner (SAM spec v1 §4.1, §5.2), host code only: the device
-// encodes and sorts the BAM records (mg_bam.cu), these write them.
+// BGZF writer and BAI builder of the god-aligner (SAM spec v1 §4.1, §5.2) and the BGZF BAM reader of
+// bam2illumina, host code only: the device encodes and sorts the BAM records (mg_bam.cu) or counts them
+// (mg_readmodel.cu), these write or read them.
 #pragma once
 #include <stdint.h>
 
@@ -70,4 +71,68 @@ class MgBamWriter {
   std::string bam_, bai_path_;
   std::vector<uint8_t> pend_;                   // the record that straddles two calls
   int64_t n_ = 0;
+};
+
+// Reader errors (MgBamReader::code; the device adds MG_RD_NAME .. MG_RD_QUAL).  `where` is the compressed
+// file offset of the member for the framing codes, the record ordinal (0-based, over the whole file) for
+// the record codes.
+enum {
+  MG_RD_OK = 0,
+  MG_RD_GZIP = 1,      // offset: not a gzip member (magic, method, or no FEXTRA flag)
+  MG_RD_BC = 2,        // offset: the gzip extra field has no 'BC' subfield
+  MG_RD_DATA = 3,      // offset: corrupt or truncated member
+  MG_RD_CRC = 4,       // offset: CRC32 of the inflated bytes differs
+  MG_RD_ISIZE = 5,     // offset: ISIZE differs from the inflated length, or exceeds 65536
+  MG_RD_MAGIC = 6,     // offset 0: the stream does not start with BAM\1
+  MG_RD_HEADER = 7,    // offset: the file ends inside the BAM header
+  MG_RD_BLOCK = 8,     // record: block_size < 32
+  MG_RD_CUT = 9,       // record: the file ends inside the record
+  MG_RD_IO = 10,       // offset: read error
+  MG_RD_NAME = 11,     // record: read name overruns block_size (checked on the device)
+  MG_RD_CIGAR = 12,    // record: CIGAR overruns block_size
+  MG_RD_SEQ = 13,      // record: SEQ overruns block_size (or l_seq < 0)
+  MG_RD_QUAL = 14,     // record: QUAL overruns block_size
+};
+
+// Whole BAM records of a chunk: data[0, bytes) holds them (a chunk may start with header bytes, which no
+// offset points at); off[i] = offset of record first + i.
+struct MgBamChunk { const uint8_t *data; int64_t bytes; const uint32_t *off; int64_t n; int64_t first; };
+
+// Sequential reader of a BGZF BAM file or FIFO.  Members are parsed in order (any XLEN; the 'BC'
+// subfield gives the member size); the ISIZE of each member gives its output offset before anything is
+// inflated, so `threads` host threads inflate a batch of members straight into the chunk buffer and check
+// CRC32 and ISIZE.  next() walks the block_size chain of the inflated stream and hands out the whole
+// records; the cut record carries over to the next chunk.  Two chunk buffers alternate (slot 0 / 1), so
+// the caller may still be copying one while the next one is inflated; `alloc` / `release` provide them
+// (page-locked memory for copies to a device).  A record larger than the buffer grows it.
+class MgBamReader {
+ public:
+  typedef void *(*Alloc)(size_t);
+  typedef void (*Release)(void *);
+  ~MgBamReader();
+  bool open(const char *path, int threads, int64_t chunk_bytes, Alloc alloc, Release release);
+  // the next chunk (n >= 1) in buffer `slot`; false at the end of the input or at the first error (code)
+  bool next(int slot, MgBamChunk &c);
+  int code = MG_RD_OK; int64_t where = -1;
+  std::string err;                             // open() failure
+  int64_t records = 0, raw_bytes = 0, comp_bytes = 0;
+  bool eof_marker = false;                     // the last member is the 28-byte EOF member
+  double read_ms = 0, inflate_ms = 0, walk_ms = 0;   // reading the file; inflating (wall time); walking the record chain
+  std::vector<double> thread_ms;               // busy time of each inflate thread
+ private:
+  struct Member { const uint8_t *z; int hdr, bsize; uint32_t crc, isize; int64_t out, comp; };
+  int fill(uint8_t *b, int64_t &n, int64_t cap);          // 1: next member does not fit, 0: input ended or failed
+  void read_more();
+  int64_t header(const uint8_t *b, int64_t pos, int64_t n);
+  void fail(int c, int64_t w) { if (!code) { code = c; where = w; } }
+  bool grow(int slot, int64_t need, int64_t keep);
+  int fd_ = -1, threads_ = 1;
+  Alloc alloc_ = nullptr; Release release_ = nullptr;
+  uint8_t *buf_[2] = {nullptr, nullptr}; uint32_t *off_[2] = {nullptr, nullptr};
+  int64_t cap_[2] = {0, 0};
+  std::vector<uint8_t> z_; int64_t zpos_ = 0, zend_ = 0, zoff_ = 0;
+  bool in_eof_ = false, done_ = false;
+  int carry_slot_ = -1; int64_t carry_at_ = 0, carry_n_ = 0;
+  int hstate_ = 0; int64_t hskip_ = 0, hrefs_ = 0;          // BAM header walk
+  std::vector<Member> batch_;
 };

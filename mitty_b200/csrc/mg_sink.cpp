@@ -55,6 +55,26 @@ void mg_deflate(const uint8_t *in, int64_t n, int level, int window_bits, std::v
   deflateEnd(&z);
 }
 
+int mg_inflate(const uint8_t *in, int64_t n, uint8_t *out, int64_t out_len) {
+  z_stream z; memset(&z, 0, sizeof z);
+  if (inflateInit2(&z, -15) != Z_OK) return 1;
+  z.next_in = const_cast<Bytef *>(in); z.avail_in = (uInt)n;
+  uint8_t spare;                                  // a stream longer than out_len lands here and is caught
+  z.next_out = out_len ? out : &spare; z.avail_out = out_len ? (uInt)out_len : 1;
+  int rc = inflate(&z, Z_FINISH);
+  if (rc == Z_BUF_ERROR && z.avail_out == 0) {
+    z.next_out = &spare; z.avail_out = 1;
+    rc = inflate(&z, Z_FINISH);
+    rc = rc == Z_STREAM_END || (rc == Z_BUF_ERROR && z.avail_out == 0) ? 2 : 1;
+  } else if (rc == Z_STREAM_END) {
+    rc = z.avail_in != 0 ? 1 : (int64_t)z.total_out != out_len ? 2 : 0;
+  } else {
+    rc = 1;
+  }
+  inflateEnd(&z);
+  return rc;
+}
+
 namespace {
 
 struct Slot { uint8_t *buf[2]; int producer; int refs; bool pinned; };

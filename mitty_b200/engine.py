@@ -111,6 +111,28 @@ class Engine(object):
     self._check(self._L.mg_model_tables(self._h, int(which), _ptr(alias), alias.size, C.byref(ks), C.byref(c9), C.byref(nr)))
     return alias.reshape(nm, nc, 1 << ks.value), ks.value, c9.value
 
+  # -- bam2illumina -----------------------------------------------------------------------------
+  def read_model_counts(self, path, max_bp=300, max_tlen=1000, min_mq=0, every=1, threads=1, chunk_bytes=64 << 20):
+    """mg_readmodel_bam: the per-base counts of an Illumina read model over a BGZF BAM (file or FIFO).
+    -> dict with bq_mat u64[2, max_bp, 94], len_hist u64[max_bp + 1], tlen u64[max_tlen], the counters of
+    READ_MODEL_COUNTS, 'times' (ms: read, inflate, walk, h2d, kernel, total) and 'thread_ms' (busy time of each
+    inflate thread).  Malformed input raises ValueError naming the record ordinal or compressed offset."""
+    threads = max(1, int(threads))
+    bq = np.zeros((2, int(max_bp), 94), dtype=np.uint64)
+    lh = np.zeros(int(max_bp) + 1, dtype=np.uint64)
+    tl = np.zeros(int(max_tlen), dtype=np.uint64)
+    cnt, times, tms = np.zeros(12, dtype=np.int64), np.zeros(6, dtype=np.float64), np.zeros(threads, dtype=np.float64)
+    bw, bc = C.c_int64(-1), C.c_int32(0)
+    rc = self._L.mg_readmodel_bam(self._h, str(path).encode(), int(max_bp), int(max_tlen), int(min_mq), int(every), threads, int(chunk_bytes),
+                                  _ptr(bq), _ptr(lh), _ptr(tl), _ptr(cnt), _ptr(times), _ptr(tms), C.byref(bw), C.byref(bc))
+    if rc == _lib.MG_EVALUE and bc.value:
+      raise bam_read_error(path, bc.value, bw.value)
+    self._check(rc)
+    out = {'bq_mat': bq, 'len_hist': lh, 'tlen': tl, 'thread_ms': tms,
+           'times': dict(zip(('read_ms', 'inflate_ms', 'walk_ms', 'h2d_ms', 'kernel_ms', 'total_ms'), (float(x) for x in times)))}
+    out.update(zip(READ_MODEL_COUNTS, (int(x) for x in cnt)))
+    return out
+
   # -- haplotypes --------------------------------------------------------------------------------
   def load_region(self, ref_bytes, bed_start):
     ref = np.ascontiguousarray(ref_bytes, dtype=np.uint8)
@@ -426,6 +448,38 @@ def write_sorted_bam(bam, bai, contigs, header_text, records, level=6, threads=1
   if rc != 0:
     raise (ValueError if rc == _lib.MG_EVALUE else RuntimeError)('mitty_b200: cannot write {} (rc={})'.format(bam, rc))
   return n.value
+
+
+# mg_readmodel_bam / mg_bam_scan errors: (what, whether bad_where is a record ordinal rather than a compressed offset)
+BAM_READ_ERRORS = {1: ('not a gzip member', False), 2: ("a gzip member without a BGZF 'BC' extra subfield", False),
+                   3: ('corrupt or truncated BGZF member', False), 4: ('CRC32 mismatch', False),
+                   5: ('ISIZE differs from the inflated length', False), 6: ('not a BAM file (magic or header lengths)', False),
+                   7: ('the file ends inside the BAM header', False), 8: ('block_size < 32', True),
+                   9: ('the file ends inside the record', True), 10: ('read error', False),
+                   11: ('read name overruns block_size', True), 12: ('CIGAR overruns block_size', True),
+                   13: ('SEQ overruns block_size', True), 14: ('QUAL overruns block_size', True)}
+READ_MODEL_COUNTS = ('records', 'considered', 'counted', 'skip_flag', 'skip_mapq', 'skip_empty', 'skip_noqual', 'skip_long',
+                     'inflated_bytes', 'compressed_bytes', 'eof_marker', 'chunks')
+
+
+def bam_read_error(path, code, where):
+  """The ValueError of a malformed BAM: names the record ordinal (0-based, file order) or the compressed offset."""
+  what, is_record = BAM_READ_ERRORS.get(code, ('error {}'.format(code), False))
+  return ValueError('{}: {} {}: {}'.format(path, 'record' if is_record else 'compressed offset', where, what))
+
+
+def scan_bam(path, threads=1, chunk_bytes=64 << 20):
+  """The BGZF BAM reader of ``read_model_counts`` without a device: inflate, check the framing and walk the
+  record chain.  -> {'records', 'inflated_bytes', 'compressed_bytes', 'eof_marker'}; malformed input raises
+  ValueError (record overruns inside block_size are checked on the device only)."""
+  L = _lib.lib()
+  st, bw, bc = np.zeros(4, dtype=np.int64), C.c_int64(-1), C.c_int32(0)
+  rc = L.mg_bam_scan(str(path).encode(), int(threads), int(chunk_bytes), _ptr(st), C.byref(bw), C.byref(bc))
+  if rc == _lib.MG_EVALUE and bc.value:
+    raise bam_read_error(path, bc.value, bw.value)
+  if rc != 0:
+    raise (ValueError if rc == _lib.MG_EVALUE else RuntimeError)('mitty_b200: cannot read {} (rc={})'.format(path, rc))
+  return dict(zip(('records', 'inflated_bytes', 'compressed_bytes', 'eof_marker'), (int(x) for x in st)))
 
 
 class Sink(object):
