@@ -37,7 +37,7 @@ typedef struct mg_ctx mg_ctx;
 int mg_device_count(void);   /* number of CUDA devices (0 if none / no driver) */
 int mg_ctx_create(int device, void *stream, mg_ctx **out);
 void mg_ctx_destroy(mg_ctx *ctx);
-const char *mg_last_error(mg_ctx *ctx);
+const char *mg_last_error(mg_ctx *ctx);   /* NULL: the last failed mg_bam_write_sorted of this thread */
 int mg_synchronize(mg_ctx *ctx);
 
 /* page-locked host memory for the caller's FASTQ buffers (makes the D2H copies of
@@ -262,7 +262,8 @@ int mg_check_fastq(mg_checker *k, const uint8_t *in1, int64_t len1, const uint8_
  * writes BAM + BAI (n_runs: sorted runs used; times[3] ms: device work incl. ingest, device-to-host copies,
  * writing); on error nothing is left behind.  mg_bam_abort drops everything, temporary files included.
  * mg_bam_write_sorted: the BGZF writer + BAI builder alone, without a device, over records already encoded
- * and in coordinate order.                                                                            */
+ * and in coordinate order.  Both reject a contig of 2^31 bases or more (MG_EVALUE, before any file is
+ * created): BAM keeps its length, POS, PNEXT and TLEN in int32.                                       */
 typedef struct mg_bam mg_bam;
 int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
                 const char *header_text, const char *sample, int32_t level, int32_t threads, int64_t run_bytes, mg_bam **out);

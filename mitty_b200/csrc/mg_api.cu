@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/mitty_b200.h"
+#include "mg_bgzf.h"
 #include "mg_internal.h"
 
 namespace {
@@ -351,7 +352,7 @@ void mg_ctx_destroy(mg_ctx *ctx) {
   delete ctx;
 }
 
-const char *mg_last_error(mg_ctx *ctx) { return ctx ? ctx->err.c_str() : "null context"; }
+const char *mg_last_error(mg_ctx *ctx) { return ctx ? ctx->err.c_str() : mg_bam_host_error(); }
 
 int mg_synchronize(mg_ctx *ctx) {
   if (!ctx) return MG_EINVAL;

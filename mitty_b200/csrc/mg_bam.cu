@@ -573,11 +573,6 @@ struct mg_bam { Bam b; };
 int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
                 const char *header_text, const char *sample, int32_t level, int32_t threads, int64_t run_bytes, mg_bam **out) {
   if (!ctx || !bam_path || n_ref <= 0 || !ref_names || !ref_len || !header_text || !sample || level < 0 || level > 9 || !out) return MG_EINVAL;
-  cudaSetDevice(mg_internal_device(ctx));
-  mg_bam *h = new mg_bam();
-  Bam &b = h->b;
-  b.ctx = ctx; b.bam = bam_path; b.bai = bai_path ? bai_path : ""; b.n_ref = n_ref; b.level = level; b.threads = std::max(1, (int)threads);
-  b.rg = sample;
   std::vector<std::string> names; std::vector<int64_t> lens;
   std::vector<uint8_t> pool; std::vector<int32_t> noff(1, 0);
   int64_t max_len = 1;
@@ -586,6 +581,14 @@ int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t
     pool.insert(pool.end(), names.back().begin(), names.back().end()); noff.push_back((int32_t)pool.size());
     max_len = std::max(max_len, ref_len[i]);
   }
+  // with every contig below 2^31, pos + span <= ref_len bounds POS, PNEXT and TLEN to int32
+  const std::string bad = mg_bam_check_contigs(names, lens);
+  if (!bad.empty()) return mg_internal_fail(ctx, MG_EVALUE, ("mg_bam_open: " + bad).c_str());
+  cudaSetDevice(mg_internal_device(ctx));
+  mg_bam *h = new mg_bam();
+  Bam &b = h->b;
+  b.ctx = ctx; b.bam = bam_path; b.bai = bai_path ? bai_path : ""; b.n_ref = n_ref; b.level = level; b.threads = std::max(1, (int)threads);
+  b.rg = sample;
   b.header = mg_bam_header(header_text, names, lens);
   b.pos_bits = bit_length((uint64_t)max_len);
   b.key_bits = bit_length((uint64_t)(n_ref - 1)) + b.pos_bits + 1;

@@ -71,6 +71,16 @@ inline uint32_t reg2bin(int64_t beg, int64_t end) {
 
 }  // namespace
 
+std::string mg_bam_check_contigs(const std::vector<std::string> &names, const std::vector<int64_t> &lens) {
+  for (size_t i = 0; i < names.size(); i++)
+    if (lens[i] < 0 || lens[i] > INT32_MAX)
+      return "contig " + names[i] + " has " + std::to_string(lens[i]) + " bases: a BAM file addresses 0 .. 2^31 - 1";
+  return "";
+}
+
+static thread_local std::string host_err;
+const char *mg_bam_host_error() { return host_err.c_str(); }
+
 std::vector<uint8_t> mg_bam_header(const std::string &text, const std::vector<std::string> &names, const std::vector<int64_t> &lens) {
   std::vector<uint8_t> h = {'B', 'A', 'M', 1};
   app32(h, (uint32_t)text.size());
@@ -271,10 +281,17 @@ extern "C" int mg_bam_write_sorted(const char *bam_path, const char *bai_path, i
   if (!bam_path || n_ref < 0 || (n_ref && (!ref_names || !ref_len)) || !header_text || (len && !records) || level < 0 || level > 9) return MG_EINVAL;
   std::vector<std::string> names; std::vector<int64_t> lens;
   for (int i = 0; i < n_ref; i++) { names.push_back(ref_names[i]); lens.push_back(ref_len[i]); }
+  host_err = mg_bam_check_contigs(names, lens);
+  if (!host_err.empty()) return MG_EVALUE;
   MgBamWriter w;
-  if (!w.open(bam_path, bai_path, mg_bam_header(header_text, names, lens), n_ref, level, threads)) { w.discard(); return MG_EVALUE; }
-  if (!w.records(records, len)) { w.discard(); return MG_EVALUE; }
-  return w.close(n_records) ? MG_OK : MG_EVALUE;
+  if (!w.open(bam_path, bai_path, mg_bam_header(header_text, names, lens), n_ref, level, threads) || !w.records(records, len)) {
+    host_err = w.err;
+    w.discard();
+    return MG_EVALUE;
+  }
+  if (w.close(n_records)) return MG_OK;
+  host_err = w.err;
+  return MG_EVALUE;
 }
 
 // ---- BGZF BAM reader -----------------------------------------------------------------------------

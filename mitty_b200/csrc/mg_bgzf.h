@@ -11,6 +11,12 @@
 
 #define MG_BGZF_BLOCK 65280   // uncompressed bytes per BGZF member (htslib's BGZF_BLOCK_SIZE)
 
+// BAM keeps l_ref, POS, PNEXT and TLEN in int32, so a contig of 2^31 bases or more cannot be written:
+// -> "" or the error naming the first such contig.
+std::string mg_bam_check_contigs(const std::vector<std::string> &names, const std::vector<int64_t> &lens);
+// The message of the last failed mg_bam_write_sorted on this thread (mg_last_error(NULL)).
+const char *mg_bam_host_error();
+
 // Binary BAM header: magic, l_text, text, then the reference list.
 std::vector<uint8_t> mg_bam_header(const std::string &text, const std::vector<std::string> &names, const std::vector<int64_t> &lens);
 

@@ -446,7 +446,7 @@ def write_sorted_bam(bam, bai, contigs, header_text, records, level=6, threads=1
   rc = L.mg_bam_write_sorted(str(bam).encode(), str(bai).encode() if bai else None, len(contigs), names, _ptr(lens), header_text.encode(),
                              _ptr(buf), len(records), int(level), int(threads), C.byref(n))
   if rc != 0:
-    raise (ValueError if rc == _lib.MG_EVALUE else RuntimeError)('mitty_b200: cannot write {} (rc={})'.format(bam, rc))
+    raise (ValueError if rc == _lib.MG_EVALUE else RuntimeError)('mitty_b200: cannot write {} (rc={}): {}'.format(bam, rc, L.mg_last_error(None).decode()))
   return n.value
 
 

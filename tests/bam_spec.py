@@ -86,10 +86,56 @@ def encode_record(name, seq, qual, info, mate, file_index, ref_id, sample):
     q = q[::-1]
   packed = bytes((codes[i] << 4 | (codes[i + 1] if i + 1 < len(codes) else 0)) for i in range(0, len(codes), 2))
   ops = cigar_ops(info.cigar)
-  body = struct.pack('<iiBBHHHiiii', ref_id, pos, len(name) + 1, 60, reg2bin(pos, end), len(ops), flag, len(seq), next_ref, next_pos, tlen)
+  # past 2^29 the SAM spec's bin does not fit the 16-bit field: its low 16 bits, as htslib's uint16_t bin keeps
+  body = struct.pack('<iiBBHHHiiii', ref_id, pos, len(name) + 1, 60, reg2bin(pos, end) & 0xFFFF, len(ops), flag, len(seq), next_ref, next_pos, tlen)
   body += name + b'\0' + b''.join(struct.pack('<I', n << 4 | CIGAR_OPS[o]) for n, o in ops) + packed + bytes(x & 0xFF for x in q)
   body += b'RGZ' + sample.encode() + b'\0'
   return struct.pack('<i', len(body)) + body
+
+
+def read_layout(pos0, span, rlen=None):
+  """(pos (1-based), cigar, rlen) of a read that covers [pos0, pos0 + span) with few bases: span 0 is a read
+  inside an insertion ('>p:nI'), a longer span a deletion between two matched bases."""
+  if span == 0:
+    n = rlen or 3
+    return pos0 + 1, '>{}:{}I'.format(pos0, n), n
+  if span <= 2:
+    return pos0 + 1, '{}='.format(span), span
+  return pos0 + 1, '1={}D1='.format(span - 2), 2
+
+
+def fastq(templates, sample='S', pad=None):
+  """Hand-built FASTQ in qname format.  templates = [(chrom, [read] or [read1, read2])], read = (strand, pos
+  (1-based), cigar, seq, qual); one read per template gives a single-end file.  pad[t]: extra leading zeros of
+  template t's serial (longer names).  -> (fq1, fq2 or None)"""
+  files = [[], []]
+  for t, (chrom, reads) in enumerate(templates):
+    serial = '0' * (pad[t] if pad else 0) + str(t)
+    name = '{}:0:0:{}|{}|0|'.format(sample, serial, chrom) + '|'.join('{}|{}|{}|{}|'.format(s, p, len(seq), c) for s, p, c, seq, _ in reads)
+    for f, (_, _, _, seq, qual) in enumerate(reads):
+      files[f].append(b'@' + name.encode() + b'\n' + seq + b'\n+\n' + qual + b'\n')
+  return b''.join(files[0]), (b''.join(files[1]) if files[1] else None)
+
+
+def bin_edge_spans(length, shifts=(14, 17, 20, 23, 26)):
+  """[(pos0, span)] of alignments that start or end on each side of multiples of 2^14 .. 2^26 (the first three
+  and the last below ``length``) and that end on the last base, spans 0 .. 2^s + 1: every level of the
+  binning scheme, bins 0 - 8 included."""
+  out = set()
+  for s in shifts:
+    bounds = sorted({m << s for m in (1, 2, 3, (length - 1) >> s)} - {0})
+    for b in bounds:
+      for sp in (1, 2, 3, (1 << s) - 1, 1 << s, (1 << s) + 1):
+        for beg in (b - sp - 1, b - sp, b - sp + 1, b - 1, b, b + 1):
+          if 0 <= beg and beg + sp <= length:
+            out.add((beg, sp))
+      for beg in (b - 1, b, b + 1):
+        if beg < length:
+          out.add((beg, 0))
+  for sp in (0, 1, 2, 3, 1 << 14, (1 << 17) + 1, 1 << 23, (1 << 26) + 1):
+    if sp <= length:
+      out.add((length - max(sp, 1), sp))
+  return sorted(out)
 
 
 def fastq_records(buf):
@@ -285,3 +331,26 @@ def decode_reads(raw):
     out.append((name, flag, bytes(ord('=ACMGRSVTWYHKDBN'[c]) for c in codes), bytes(qual)))
     u += 4 + bs
   return out
+
+
+def check_queries(data, bai, regions):
+  """Every record that overlaps a query region lies in a chunk the index returns for it."""
+  index = parse_bai(bai)
+  recs = record_offsets(data)
+  for ref, beg, end in regions:
+    chunks = query(index, ref, beg, end)
+    hits = [v for v, r, pos, e in recs if r == ref and pos < end and e > beg]
+    for v in hits:
+      assert any(a <= v < b for a, b in chunks), (ref, beg, end, v)
+
+
+def edge_queries(ref, length, shifts=(14, 17, 20, 23, 26)):
+  """Query regions on bin and 16 kb window edges of one contig: 1, 2 and 2^s bases around each multiple
+  of 2^s that bin_edge_spans uses (16 kb windows are the s = 14 case)."""
+  out = []
+  for s in shifts:
+    for b in sorted({m << s for m in (1, 2, 3, (length - 1) >> s)} - {0}):
+      for beg, end in ((b - 1, b), (b, b + 1), (b - 1, b + 1), (b - (1 << s), b), (b, b + (1 << s)), (b - 1, b + (1 << s) + 1)):
+        if 0 <= beg and end <= length:
+          out.append((ref, beg, end))
+  return out + [(ref, length - 1, length), (ref, 0, length)]

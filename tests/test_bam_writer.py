@@ -136,15 +136,131 @@ def test_index_query_finds_every_overlapping_record(tmp_path, synthetic):
   from mitty_b200.engine import write_sorted_bam
   p = str(tmp_path / 'q.bam')
   write_sorted_bam(p, p + '.bai', CONTIGS, S.header_text(CONTIGS, 'T'), b''.join(synthetic), level=1, threads=2)
-  data = open(p, 'rb').read()
-  index = S.parse_bai(open(p + '.bai', 'rb').read())
-  recs = S.record_offsets(data)
   rng = random.Random(11)
+  regions = []
   for _ in range(200):
     ref = rng.randrange(len(CONTIGS))
     beg = rng.randrange(CONTIGS[ref][1] - 10)
-    end = min(CONTIGS[ref][1], beg + rng.choice([1, 50, 1000, 20000, 100000]))
-    chunks = S.query(index, ref, beg, end)
-    hits = [v for v, r, pos, e in recs if r == ref and pos < end and e > beg]
-    for v in hits:
-      assert any(a <= v < b for a, b in chunks), (ref, beg, end, v)
+    regions.append((ref, beg, min(CONTIGS[ref][1], beg + rng.choice([1, 50, 1000, 20000, 100000]))))
+  S.check_queries(open(p, 'rb').read(), open(p + '.bai', 'rb').read(), regions)
+
+
+# ---- block, record-size and bin edges of the writer -------------------------------------------------
+
+EDGE_CONTIGS = [('1', 20000), ('big', 3 * (1 << 26) + 12345), ('empty', 5000), ('last', 1 << 27)]
+
+
+def _reads(rng, chrom, n, length, L=60):
+  """n single-end templates of L bases at random positions of chrom, in coordinate order."""
+  return sorted(((chrom, [(rng.randrange(2), rng.randrange(1, length - L), '%d=' % L, bytes(rng.choice(b'ACGT') for _ in range(L)), b'I' * L)])
+                 for _ in range(n)), key=lambda t: t[1][0][1::-1])
+
+
+def _stream(templates, pad=None):
+  """-> (header + records, records) of the spec for single-end templates."""
+  fq1, _ = S.fastq(templates, sample='T', pad=pad)
+  _, recs = S.records(EDGE_CONTIGS, fq1)
+  return S.header_bytes(EDGE_CONTIGS, 'T') + b''.join(recs), recs
+
+
+def _bin_edge_templates(rng):
+  out = []
+  for ref in (1, 3):
+    chrom, length = EDGE_CONTIGS[ref]
+    for beg, sp in S.bin_edge_spans(length):
+      pos, cig, rlen = S.read_layout(beg, sp)
+      out.append((chrom, [(rng.randrange(2), pos, cig, bytes(rng.choice(b'ACGT') for _ in range(rlen)), b'5' * rlen)]))
+  return out
+
+
+def _padded_to(templates, target):
+  """Pads the names of the first templates (in coordinate order) so that a record ends exactly at
+  uncompressed offset ``target``.  -> pad"""
+  raw, recs = _stream(templates)
+  u = len(raw) - sum(len(r) for r in recs)
+  ends = []
+  for r in recs:
+    u += len(r)
+    ends.append(u)
+  short = max(e for e in ends if e <= target)       # the last record end at or before target, moved up to it
+  need, pad = target - short, [0] * len(templates)
+  for t in range(len(templates)):
+    pad[t] = min(need, 150)
+    need -= pad[t]
+  assert need == 0
+  return pad
+
+
+def _edge_case(case):
+  rng = random.Random(case)
+  if case == 'bins_0_to_72':
+    t = _bin_edge_templates(rng) + _reads(rng, '1', 300, 20000)
+    return t, None
+  if case == 'record_over_64k':
+    L = 100000
+    big = ('big', [(1, 5000, '%d=' % L, bytes(rng.choice(b'ACGTN') for _ in range(L)), bytes(rng.randrange(33, 75) for _ in range(L)))])
+    return _reads(rng, 'big', 400, 20000) + [big] + _reads(rng, 'big', 200, 200000), None
+  t = _reads(rng, '1', 1500, 20000)
+  raw, _ = _stream(t)
+  if case == 'record_ends_on_block':
+    return t, _padded_to(t, S.BLOCK)
+  assert case == 'stream_is_whole_blocks'
+  return t, _padded_to(t, (len(raw) // S.BLOCK + 1) * S.BLOCK)
+
+
+@pytest.mark.parametrize('case', ['bins_0_to_72', 'record_ends_on_block', 'stream_is_whole_blocks', 'record_over_64k'])
+def test_native_writer_block_record_and_bin_edges(tmp_path, case):
+  """The native writer and index against the specification where blocks, records and bins meet their edges;
+  each case asserts that its records reach the edge it is named after."""
+  from mitty_b200.engine import write_sorted_bam
+  templates, pad = _edge_case(case)
+  raw, recs = _stream(templates, pad)
+  ends, u = set(), len(raw) - sum(len(r) for r in recs)
+  for r in recs:
+    u += len(r)
+    ends.add(u)
+  bins = {struct.unpack_from('<H', r, 14)[0] for r in recs}
+  if case == 'bins_0_to_72':
+    assert 0 in bins and bins & set(range(1, 9)) and bins & set(range(9, 73)) and bins & set(range(73, 585)), sorted(bins)[:20]
+  elif case == 'record_ends_on_block':
+    assert S.BLOCK in ends and len(raw) > 2 * S.BLOCK
+  elif case == 'stream_is_whole_blocks':
+    assert len(raw) % S.BLOCK == 0 and len(raw) // S.BLOCK >= 2
+  else:
+    assert max(len(r) for r in recs) > 1 << 16
+  p = str(tmp_path / 'e.bam')
+  assert write_sorted_bam(p, p + '.bai', EDGE_CONTIGS, S.header_text(EDGE_CONTIGS, 'T'), b''.join(recs), level=1, threads=3) == len(recs)
+  data, bai = open(p, 'rb').read(), open(p + '.bai', 'rb').read()
+  assert S.decompress(data) == raw
+  assert bai == S.build_bai(data, len(EDGE_CONTIGS))
+  if case == 'stream_is_whole_blocks':
+    assert [len(m) for _, m in S.members(data)] == [S.BLOCK] * (len(raw) // S.BLOCK) + [0]
+  if case == 'bins_0_to_72':
+    S.check_queries(data, bai, S.edge_queries(1, EDGE_CONTIGS[1][1]) + S.edge_queries(3, EDGE_CONTIGS[3][1]) + [(2, 0, 5000)])
+
+
+def test_writer_rejects_contigs_bam_cannot_address(tmp_path):
+  """BAM keeps a contig's length, POS, PNEXT and TLEN in int32: a contig of 2^31 bases or more is an error
+  naming it, raised before any file exists; 2^31 - 1 bases are written."""
+  from mitty_b200.engine import write_sorted_bam
+  p = str(tmp_path / 'x.bam')
+  for length in (1 << 31, 1 << 40):
+    contigs = [('1', 100), ('huge', length)]
+    with pytest.raises(ValueError, match='huge'):
+      write_sorted_bam(p, p + '.bai', contigs, 'x', b'')
+    assert os.listdir(str(tmp_path)) == []
+  contigs = [('1', 100), ('huge', (1 << 31) - 1)]
+  assert write_sorted_bam(p, None, contigs, S.header_text(contigs, 'T'), b'') == 0
+  assert S.decompress(open(p, 'rb').read()) == S.header_bytes(contigs, 'T')
+
+
+def test_spec_bin_past_2_29_keeps_its_low_16_bits():
+  """Past 2^29 the SAM spec's bin no longer fits the record's 16-bit field (from 4681 + 997 048 320 >> 14):
+  the record keeps its low 16 bits, as htslib's uint16_t field does."""
+  for pos0, sp, full in ((1 << 29, 10, 4681 + (1 << 15)), (997048320 - 1, 1, 65535), (997048320, 1, 65536),
+                         ((1 << 31) - 2, 1, 4681 + ((1 << 31) - 2 >> 14)), ((1 << 30) + 3, 1 << 16, 585 + (1 << 13))):
+    assert S.reg2bin(pos0, pos0 + sp) == full
+    name = b'T:0:0:1|h|0|0|%d|%d|%d=|' % (pos0 + 1, sp, sp)
+    r = S.encode_record(name, b'A' * sp, b'I' * sp, parse_qname(name.decode())[0], None, 0, 0, 'T')
+    assert struct.unpack_from('<i', r, 8)[0] == pos0
+    assert struct.unpack_from('<H', r, 14)[0] == full & 0xFFFF
