@@ -3,7 +3,7 @@
 
 Every read becomes one BAM record at the POS / CIGAR its qname states (``parse_qname``): POS = qname pos
 - 1, the qname's CIGAR ('>p:nI' becomes 'nI'), strand-1 reads reverse-complemented back and their
-qualities reversed.  The FASTQ files are streamed in chunks through page-locked buffers; the device
+qualities reversed.  The FASTQ files are read in chunks through page-locked buffers (``lib.fastqio``); the device
 parses, validates, encodes and sorts the records (``k_bam_size``, ``k_bam_encode``, ``k_radix_*``,
 ``k_gather_*``) in runs of at most ``run_bytes`` of device memory; host threads deflate the BGZF blocks
 and build the BAI.  The bytes written do not depend on ``run_bytes``, the chunk size, ``threads`` or the
@@ -13,8 +13,8 @@ import os
 import time
 
 from mitty_b200.engine import BamWriter, Engine
+from mitty_b200.lib.fastqio import FastqStream, for_each_chunk, qname_of
 from mitty_b200.lib.vcfio import FastaFile
-from mitty_b200.simulation.readcorrupt import _Stream
 
 logger = logging.getLogger(__name__)
 
@@ -37,15 +37,6 @@ def sample_of(buf):
   return line[1:].split('|', 1)[0].split(':', 1)[0].strip() if line.startswith('@') else ''
 
 
-def _record(buf, rec):
-  """The qname line of record ``rec`` of a FASTQ chunk."""
-  pos = 0
-  for _ in range(4 * rec):
-    pos = buf.index(b'\n', pos) + 1
-  end = buf.find(b'\n', pos)
-  return buf[pos:end if end >= 0 else len(buf)].decode(errors='replace')
-
-
 def process_multi_threaded(fasta, bam_fname, fastq1, fastq2=None, threads=None, device=0, level=6, run_bytes=None,
                            chunk_bytes=256 << 20, sample=None):
   """Write ``bam_fname`` and ``bam_fname + '.bai'`` from the FASTQ (pair).  ``threads``: host deflate threads;
@@ -66,43 +57,33 @@ def process_multi_threaded(fasta, bam_fname, fastq1, fastq2=None, threads=None, 
   threads = default_threads() if threads is None else max(1, int(threads))
   engine = Engine(device)
   bw = None
-  paired = fastq2 is not None
-  ins = []
   try:
-    # one open() per input (they may be FIFOs): the sample is read from the first chunk, not peeked
-    ins = [_Stream(fastq1, engine.pinned(chunk_bytes))] + ([_Stream(fastq2, engine.pinned(chunk_bytes))] if paired else [])
+    ins = [FastqStream(f, engine.pinned(chunk_bytes)) for f in (fastq1, fastq2) if f is not None]
     templates = 0
-    while True:
-      for st in ins:
-        st.refill()
+
+    def writer(first):      # the BamWriter, opened at the first chunk: the @RG sample is its first qname's
+      nonlocal bw
       if bw is None:
-        sample = sample_of(ins[0].buf[:ins[0].fill]) if sample is None else sample
-        bw = BamWriter(engine, bam_fname, bai, contigs, header_text(contigs, sample), sample, level=level, threads=threads, run_bytes=run_bytes)
-      a1 = ins[0].buf[:ins[0].fill]
-      a2 = ins[1].buf[:ins[1].fill] if paired else None
-      if a1.size == 0 or (paired and a2.size == 0):
-        break
+        s = sample_of(first) if sample is None else sample
+        bw = BamWriter(engine, bam_fname, bai, contigs, header_text(contigs, s), s, level=level, threads=threads, run_bytes=run_bytes)
+      return bw
+
+    def step(a1, a2):
+      nonlocal templates
       try:
-        n, c1, c2 = bw.add(a1, a2)
+        n, c1, c2 = writer(a1).add(a1, a2)
       except ValueError as e:
         if len(e.args) < 4:
           raise
         f, rec, why = e.args[1:]
-        buf = (a1 if f == 0 else a2).tobytes()
-        raise ValueError('{} record {}: {}: {}'.format(fastq1 if f == 0 else fastq2, templates + rec + 1, why, _record(buf, rec)))
-      if n == 0:
-        if all(st.eof for st in ins):
-          break
-        raise ValueError('a FASTQ record is larger than the chunk size ({} bytes)'.format(chunk_bytes))
+        raise ValueError('{} record {}: {}: {}'.format(fastq1 if f == 0 else fastq2, templates + rec + 1, why, qname_of(a1 if f == 0 else a2, rec)))
       templates += n
-      ins[0].consume(c1)
-      if paired:
-        ins[1].consume(c2)
-    records, runs, times = bw.close()
+      return n, c1, c2
+
+    for_each_chunk(ins, step)
+    records, runs, times = writer(ins[0].buf[:ins[0].fill]).close()      # an empty input still gets an empty BAM and BAI
     bw = None
   finally:
-    for st in ins:
-      st.close()
     if bw is not None:
       bw.abort()
     engine.close()

@@ -22,35 +22,6 @@
 
 namespace {
 
-struct DevBuf {  // grow-only device buffer
-  void *p = nullptr;
-  size_t cap = 0;
-  ~DevBuf() { if (p) cudaFree(p); }
-  cudaError_t need(size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) { cudaFree(p); p = nullptr; cap = 0; }
-    size_t want = bytes + bytes / 8 + 256;
-    cudaError_t e = cudaMalloc(&p, want);
-    if (e == cudaSuccess) cap = want;
-    return e;
-  }
-  template <class T> T *as() { return reinterpret_cast<T *>(p); }
-};
-
-struct HostBuf {  // grow-only page-locked staging buffer
-  void *p = nullptr;
-  size_t cap = 0;
-  ~HostBuf() { if (p) cudaFreeHost(p); }
-  cudaError_t need(size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) { cudaFreeHost(p); p = nullptr; cap = 0; }
-    size_t want = bytes + bytes / 4 + 4096;
-    cudaError_t e = cudaHostAlloc(&p, want, cudaHostAllocPortable);
-    if (e == cudaSuccess) cap = want;
-    return e;
-  }
-};
-
 struct ExcRun { int64_t start, len; uint8_t byte; };
 
 struct Region {
@@ -109,7 +80,8 @@ struct mg_ctx {
   int64_t next_id = 1;
   // scratch
   DevBuf s_raw, s_exc, s_ts, s_u, s_fo, s_tsorted, s_partial, s_state, s_out[2][2], s_str, s_plan, s_sample[3];
-  DevBuf c_in[2], c_out[2], c_nl[2], c_cnt, c_sz[2], c_off[2], c_tmp, c_draw[4];
+  MgFastqChunk fq;                                 // corrupt-reads: the input chunk and its newline index
+  DevBuf c_out[2], c_sz[2], c_off[2], c_draw[4];
   DevBuf b_units, b_arr;                           // a batch of small units: unit table; per-unit counts and their prefixes
   HostBuf h_stage;                                 // the variant arrays of a build on their way to the device (one DMA from page-locked memory)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr;
@@ -143,8 +115,6 @@ int fail(mg_ctx *c, int code, const char *fmt, ...) {
   if (c) c->err = buf;
   return code;
 }
-
-#define CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx, MG_ECUDA, "%s: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); } while (0)
 
 // Vose's alias method over K outcomes with probabilities q (sum 1): entry i = prob << alias_bits | alias,
 // prob quantised to prob_bits.  A draw takes idx uniform in [0, K) and frac uniform in [0, 2^prob_bits):
@@ -239,12 +209,6 @@ struct Timer {   // MG_TIMING=1: host-side section timings on stderr
   static double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
   explicit Timer(const char *n) : name(n), t0(now()), on(getenv("MG_TIMING") != nullptr) {}
   void lap(const char *what) { if (on) { double t = now(); fprintf(stderr, "[mg] %s/%s %.2f ms\n", name, what, t - t0); t0 = t; } }
-};
-
-struct DeviceGuard {
-  int prev = -1;
-  explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
-  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
 }  // namespace
@@ -357,23 +321,23 @@ const char *mg_last_error(mg_ctx *ctx) { return ctx ? ctx->err.c_str() : mg_bam_
 int mg_synchronize(mg_ctx *ctx) {
   if (!ctx) return MG_EINVAL;
   DeviceGuard g(ctx->device);
-  CU(cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
   return MG_OK;
 }
 
 int mg_host_alloc(mg_ctx *ctx, int64_t bytes, void **out) {
   if (!ctx || !out || bytes <= 0) return fail(ctx, MG_EINVAL, "mg_host_alloc: bad arguments");
   DeviceGuard g(ctx->device);
-  CU(cudaHostAlloc(out, (size_t)bytes, cudaHostAllocPortable));
+  MG_CK(ctx, cudaHostAlloc(out, (size_t)bytes, cudaHostAllocPortable));
   return MG_OK;
 }
 
 int mg_host_free(mg_ctx *ctx, void *p) {
   if (!ctx) return MG_EINVAL;
   DeviceGuard g(ctx->device);
-  CU(cudaStreamSynchronize(ctx->stream));
-  if (ctx->copy_stream) CU(cudaStreamSynchronize(ctx->copy_stream));   // the pinned FASTQ buffers are written by this stream
-  CU(cudaFreeHost(p));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  if (ctx->copy_stream) MG_CK(ctx, cudaStreamSynchronize(ctx->copy_stream));   // the pinned FASTQ buffers are written by this stream
+  MG_CK(ctx, cudaFreeHost(p));
   return MG_OK;
 }
 
@@ -382,12 +346,12 @@ int mg_model_load(mg_ctx *ctx, const double *cum_tlen, int n_tlen, const double 
   if (!ctx || !cum_tlen || !cum_bq_mat || !phred_p || n_tlen <= 0 || n_mates < 1 || n_cycles <= 0 || n_bq <= 0 || rlen <= 0)
     return fail(ctx, MG_EINVAL, "mg_model_load: bad arguments");
   DeviceGuard g(ctx->device);
-  CU(ctx->m_tlen.need(sizeof(double) * n_tlen));
-  CU(ctx->m_bq.need(sizeof(double) * (size_t)n_mates * n_cycles * n_bq));
-  CU(ctx->m_phred.need(sizeof(double) * 100));
-  CU(cudaMemcpyAsync(ctx->m_tlen.p, cum_tlen, sizeof(double) * n_tlen, cudaMemcpyHostToDevice, ctx->stream));
-  CU(cudaMemcpyAsync(ctx->m_bq.p, cum_bq_mat, sizeof(double) * (size_t)n_mates * n_cycles * n_bq, cudaMemcpyHostToDevice, ctx->stream));
-  CU(cudaMemcpyAsync(ctx->m_phred.p, phred_p, sizeof(double) * 100, cudaMemcpyHostToDevice, ctx->stream));
+  MG_CK(ctx, ctx->m_tlen.need(sizeof(double) * n_tlen));
+  MG_CK(ctx, ctx->m_bq.need(sizeof(double) * (size_t)n_mates * n_cycles * n_bq));
+  MG_CK(ctx, ctx->m_phred.need(sizeof(double) * 100));
+  MG_CK(ctx, cudaMemcpyAsync(ctx->m_tlen.p, cum_tlen, sizeof(double) * n_tlen, cudaMemcpyHostToDevice, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(ctx->m_bq.p, cum_bq_mat, sizeof(double) * (size_t)n_mates * n_cycles * n_bq, cudaMemcpyHostToDevice, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(ctx->m_phred.p, phred_p, sizeof(double) * 100, cudaMemcpyHostToDevice, ctx->stream));
   // production-mode tables: one joint (quality, substitution) alias row per (mate, cycle).  Built
   // twice: for the emit kernel over the cycles a read of this model has (rlen), and for the standalone
   // corrupt kernel over every cycle (reads of any length up to n_cycles; the rows beyond the model's
@@ -412,17 +376,17 @@ int mg_model_load(mg_ctx *ctx, const double *cum_tlen, int n_tlen, const double 
         const size_t r = (size_t)m * n_cycles + c;
         build_joint_row(cum_bq_mat + r * n_bq, n_bq, phred_p, K, code9, ctx->h_alias[t].data() + r * K);
       }
-    CU(ctx->m_alias[t].need(4 * ctx->h_alias[t].size()));
-    CU(cudaMemcpyAsync(ctx->m_alias[t].p, ctx->h_alias[t].data(), 4 * ctx->h_alias[t].size(), cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, ctx->m_alias[t].need(4 * ctx->h_alias[t].size()));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->m_alias[t].p, ctx->h_alias[t].data(), 4 * ctx->h_alias[t].size(), cudaMemcpyHostToDevice, ctx->stream));
   }
   ctx->has_tlen_alias = (n_tlen + 1 <= MG_TLEN_K);
   if (ctx->has_tlen_alias) {
     std::vector<uint32_t> ta(MG_TLEN_K);
     vose(ss_left_probs(cum_tlen, n_tlen, MG_TLEN_K, n_tlen), MG_TLEN_K, 22, 10, ta.data());
-    CU(ctx->m_tlen_alias.need(4 * MG_TLEN_K));
-    CU(cudaMemcpy(ctx->m_tlen_alias.p, ta.data(), 4 * MG_TLEN_K, cudaMemcpyHostToDevice));
+    MG_CK(ctx, ctx->m_tlen_alias.need(4 * MG_TLEN_K));
+    MG_CK(ctx, cudaMemcpy(ctx->m_tlen_alias.p, ta.data(), 4 * MG_TLEN_K, cudaMemcpyHostToDevice));
   }
-  CU(cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->n_tlen = n_tlen; ctx->n_mates = n_mates; ctx->n_cycles = n_cycles; ctx->n_bq = n_bq; ctx->rlen = rlen;
   return MG_OK;
 }
@@ -452,28 +416,28 @@ static int load_packed(mg_ctx *ctx, const uint8_t *ref_bytes, int64_t len, int64
   R->len = len; R->bed_start = bed_start;
   int64_t words = (len + 15) / 16;
   R->owner = ctx;
-  CU(pool_get(ctx, (void **)&R->d_ref, sizeof(uint32_t) * (words + 2 * MG_HAP_PAD)));
-  CU(cudaMemsetAsync(R->d_ref, 0, sizeof(uint32_t) * (words + 2 * MG_HAP_PAD), ctx->stream));
+  MG_CK(ctx, pool_get(ctx, (void **)&R->d_ref, sizeof(uint32_t) * (words + 2 * MG_HAP_PAD)));
+  MG_CK(ctx, cudaMemsetAsync(R->d_ref, 0, sizeof(uint32_t) * (words + 2 * MG_HAP_PAD), ctx->stream));
   if (len > 0) {
-    CU(ctx->s_raw.need((size_t)len + 32));
-    CU(cudaMemcpyAsync(ctx->s_raw.p, ref_bytes, (size_t)len, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, ctx->s_raw.need((size_t)len + 32));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->s_raw.p, ref_bytes, (size_t)len, cudaMemcpyHostToDevice, ctx->stream));
     uint32_t cnt[2] = {0, 0};
     int64_t *d_start = nullptr, *d_end = nullptr;
     uint8_t *d_byte = nullptr;
     for (int attempt = 0; attempt < 2; attempt++) {
       // exception scratch: [cnt u32 x2 (padded to 16 B)][start i64 x cap][end i64 x cap][byte u8 x cap]
-      CU(ctx->s_exc.need(16 + (size_t)exc_cap * 17));
+      MG_CK(ctx, ctx->s_exc.need(16 + (size_t)exc_cap * 17));
       uint8_t *eb = ctx->s_exc.as<uint8_t>();
       uint32_t *d_cnt = reinterpret_cast<uint32_t *>(eb);
       d_start = reinterpret_cast<int64_t *>(eb + 16);
       d_end = d_start + exc_cap;
       d_byte = reinterpret_cast<uint8_t *>(d_end + exc_cap);
-      CU(cudaMemsetAsync(d_cnt, 0, 16, ctx->stream));
+      MG_CK(ctx, cudaMemsetAsync(d_cnt, 0, 16, ctx->stream));
       mg_launch_pack_ref(ctx->s_raw.as<uint8_t>(), len, R->d_ref + MG_HAP_PAD, d_cnt, d_start, d_byte, d_end, exc_cap, ctx->stream);
       ctx->total_launches++;
-      CU(cudaGetLastError());
-      CU(cudaMemcpyAsync(cnt, d_cnt, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      CU(cudaStreamSynchronize(ctx->stream));
+      MG_CK(ctx, cudaGetLastError());
+      MG_CK(ctx, cudaMemcpyAsync(cnt, d_cnt, 8, cudaMemcpyDeviceToHost, ctx->stream));
+      MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
       if (cnt[0] != cnt[1]) return fail(ctx, MG_ECUDA, "internal: exception run starts (%u) != ends (%u)", cnt[0], cnt[1]);
       if (cnt[0] <= exc_cap) break;
       if (attempt == 1 || cnt[0] > (1u << 27))
@@ -483,9 +447,9 @@ static int load_packed(mg_ctx *ctx, const uint8_t *ref_bytes, int64_t len, int64
     if (cnt[0]) {
       std::vector<int64_t> st(cnt[0]), en(cnt[0]);
       std::vector<uint8_t> by(cnt[0]);
-      CU(cudaMemcpy(st.data(), d_start, 8 * (size_t)cnt[0], cudaMemcpyDeviceToHost));
-      CU(cudaMemcpy(en.data(), d_end, 8 * (size_t)cnt[0], cudaMemcpyDeviceToHost));
-      CU(cudaMemcpy(by.data(), d_byte, (size_t)cnt[0], cudaMemcpyDeviceToHost));
+      MG_CK(ctx, cudaMemcpy(st.data(), d_start, 8 * (size_t)cnt[0], cudaMemcpyDeviceToHost));
+      MG_CK(ctx, cudaMemcpy(en.data(), d_end, 8 * (size_t)cnt[0], cudaMemcpyDeviceToHost));
+      MG_CK(ctx, cudaMemcpy(by.data(), d_byte, (size_t)cnt[0], cudaMemcpyDeviceToHost));
       std::vector<uint32_t> order(cnt[0]);
       for (uint32_t i = 0; i < cnt[0]; i++) order[i] = i;
       std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return st[a] < st[b]; });
@@ -496,8 +460,8 @@ static int load_packed(mg_ctx *ctx, const uint8_t *ref_bytes, int64_t len, int64
         R->exc[i] = ExcRun{st[order[i]], en[i] - st[order[i]] + 1, by[order[i]]};
         dev[i] = MgExc{(uint32_t)R->exc[i].start, (uint32_t)R->exc[i].len, R->exc[i].byte, 0};
       }
-      CU(pool_get(ctx, (void **)&R->d_exc, sizeof(MgExc) * cnt[0]));
-      CU(cudaMemcpy(R->d_exc, dev.data(), sizeof(MgExc) * cnt[0], cudaMemcpyHostToDevice));
+      MG_CK(ctx, pool_get(ctx, (void **)&R->d_exc, sizeof(MgExc) * cnt[0]));
+      MG_CK(ctx, cudaMemcpy(R->d_exc, dev.data(), sizeof(MgExc) * cnt[0], cudaMemcpyHostToDevice));
     }
   }
   return MG_OK;
@@ -572,10 +536,10 @@ static int build_segments(mg_ctx *ctx, const uint32_t *d_ref, const MgExc *d_rex
   const size_t o_eoff = o; o += al(8 * (max_nodes + 3));
   const size_t o_sum = o; o += al(sizeof(MgWalkSummary));
   const size_t o_segout = o; o += al(sizeof(MgSegOut) * ns);
-  CU(ctx->s_str.need(o));
+  MG_CK(ctx, ctx->s_str.need(o));
   uint8_t *sb = ctx->s_str.as<uint8_t>();
-  CU(pool_get(ctx, (void **)&C.d_nodes, sizeof(MgNode) * std::max<size_t>(max_nodes, 1)));
-  CU(ctx->h_stage.need(in_bytes));
+  MG_CK(ctx, pool_get(ctx, (void **)&C.d_nodes, sizeof(MgNode) * std::max<size_t>(max_nodes, 1)));
+  MG_CK(ctx, ctx->h_stage.need(in_bytes));
   {
     uint8_t *hs = static_cast<uint8_t *>(ctx->h_stage.p);
     if (V) {
@@ -584,7 +548,7 @@ static int build_segments(mg_ctx *ctx, const uint32_t *d_ref, const MgExc *d_rex
       if (alt_bytes) memcpy(hs + o_alt, alt_pool, (size_t)alt_bytes);
     }
     memcpy(hs + o_seg, segs.data(), sizeof(MgSeg) * ns);
-    CU(cudaMemcpyAsync(sb, hs, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(sb, hs, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
   }
   MgWalkParams W;
   W.pos = reinterpret_cast<int64_t *>(sb + o_pos); W.oplen = reinterpret_cast<int64_t *>(sb + o_oplen);
@@ -603,15 +567,15 @@ static int build_segments(mg_ctx *ctx, const uint32_t *d_ref, const MgExc *d_rex
   int64_t *e_cnt = reinterpret_cast<int64_t *>(sb + o_ecnt), *e_off = reinterpret_cast<int64_t *>(sb + o_eoff);
   mg_launch_exc_count(C.d_nodes, W.node_alt, W.sum, (int)max_nodes, sb + o_alt, d_rexc, n_rexc, e_cnt, ctx->stream);
   mg_launch_scan_i64(e_cnt, e_off, (int64_t)max_nodes, W.scan_tmp, ctx->stream);
-  CU(cudaGetLastError());
+  MG_CK(ctx, cudaGetLastError());
   MgWalkSummary sum;
   int64_t n_exc = 0;
   seg_out.resize(ns);
-  CU(cudaMemcpyAsync(&sum, W.sum, sizeof sum, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(&n_exc, e_off + max_nodes, 8, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(seg_out.data(), W.seg_out, sizeof(MgSegOut) * ns, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(&sum, W.sum, sizeof sum, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(&n_exc, e_off + max_nodes, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(seg_out.data(), W.seg_out, sizeof(MgSegOut) * ns, cudaMemcpyDeviceToHost, ctx->stream));
   tm.lap("enqueue walk");
-  CU(cudaStreamSynchronize(ctx->stream));             // also: the caller's arrays have been consumed
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));             // also: the caller's arrays have been consumed
   tm.lap("walk");
 
   if (sum.err != ~0ull) {
@@ -636,23 +600,23 @@ static int build_segments(mg_ctx *ctx, const uint32_t *d_ref, const MgExc *d_rex
   // -- device builds that need the sizes: exception runs, haplotype, block table
   C.hap_words = (hap_len + 15) / 16;
   C.n_blk = (int)((hap_len >> BLK_SHIFT) + 1);
-  CU(pool_get(ctx, (void **)&C.d_hap, sizeof(uint32_t) * (C.hap_words + 2 * MG_HAP_PAD)));
-  CU(pool_get(ctx, (void **)&C.d_blk, sizeof(uint32_t) * C.n_blk));
-  CU(pool_get(ctx, (void **)&C.d_exc, sizeof(MgExc) * std::max<size_t>(1, (size_t)n_exc)));
+  MG_CK(ctx, pool_get(ctx, (void **)&C.d_hap, sizeof(uint32_t) * (C.hap_words + 2 * MG_HAP_PAD)));
+  MG_CK(ctx, pool_get(ctx, (void **)&C.d_blk, sizeof(uint32_t) * C.n_blk));
+  MG_CK(ctx, pool_get(ctx, (void **)&C.d_exc, sizeof(MgExc) * std::max<size_t>(1, (size_t)n_exc)));
   if (n_exc) {
     mg_launch_exc_write(C.d_nodes, W.node_alt, W.sum, (int)max_nodes, sb + o_alt, d_rexc, n_rexc, e_off, C.d_exc, ctx->stream);
-    CU(pool_get(ctx, (void **)&C.d_eblk, sizeof(uint32_t) * ((size_t)C.n_blk + 1)));
+    MG_CK(ctx, pool_get(ctx, (void **)&C.d_eblk, sizeof(uint32_t) * ((size_t)C.n_blk + 1)));
     mg_launch_eblk_table(C.d_exc, (int)n_exc, C.d_eblk, C.n_blk + 1, BLK_SHIFT, ctx->stream);
     ctx->total_launches++;
   }
-  CU(cudaMemsetAsync(C.d_hap, 0, sizeof(uint32_t) * MG_HAP_PAD, ctx->stream));
-  CU(cudaMemsetAsync(C.d_hap + MG_HAP_PAD + C.hap_words, 0, sizeof(uint32_t) * MG_HAP_PAD, ctx->stream));
+  MG_CK(ctx, cudaMemsetAsync(C.d_hap, 0, sizeof(uint32_t) * MG_HAP_PAD, ctx->stream));
+  MG_CK(ctx, cudaMemsetAsync(C.d_hap + MG_HAP_PAD + C.hap_words, 0, sizeof(uint32_t) * MG_HAP_PAD, ctx->stream));
   mg_launch_blk_table(C.d_nodes, (int)nn, C.d_blk, C.n_blk, BLK_SHIFT, ctx->stream);
   if (hap_len > 0)
     mg_launch_hap_build(d_ref, sb + o_alt, C.d_nodes, W.node_alt, (int)nn, C.d_blk, BLK_SHIFT, C.n_blk, (uint32_t)hap_len, C.d_hap + MG_HAP_PAD,
                         C.hap_words, ctx->stream);
   ctx->total_launches += 2 + (n_exc ? 1 : 0);
-  CU(cudaGetLastError());
+  MG_CK(ctx, cudaGetLastError());
   tm.lap("enqueue build");                            // stream-ordered: units launched next wait for these kernels
   return MG_OK;
 }
@@ -702,8 +666,8 @@ int mg_copy_nodes(mg_ctx *ctx, int64_t copy_id, int64_t *ps, int64_t *pr, uint8_
   DeviceGuard g(ctx->device);
   const Copy &C = *it->second;
   std::vector<MgNode> dn((size_t)C.n_nodes);
-  CU(cudaStreamSynchronize(ctx->stream));
-  CU(cudaMemcpy(dn.data(), C.d_nodes, sizeof(MgNode) * dn.size(), cudaMemcpyDeviceToHost));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaMemcpy(dn.data(), C.d_nodes, sizeof(MgNode) * dn.size(), cudaMemcpyDeviceToHost));
   for (size_t k = 0; k < dn.size(); k++) {   // the device table back in the reference's terms (rpc.py:5-35)
     ps[k] = C.p_min + (int64_t)dn[k].key - (dn[k].op == 'D' ? 1 : 0);
     pr[k] = dn[k].pr; op[k] = (uint8_t)dn[k].op; oplen[k] = dn[k].oplen;
@@ -720,11 +684,11 @@ int mg_copy_haplotype(mg_ctx *ctx, int64_t copy_id, uint8_t *out, int64_t cap) {
   const int64_t n = C.p_max - C.p_min;
   if (cap < n) return fail(ctx, MG_ECAP, "haplotype needs %lld bytes", (long long)n);
   std::vector<uint32_t> w((size_t)C.hap_words);
-  CU(cudaStreamSynchronize(ctx->stream));
-  if (C.hap_words) CU(cudaMemcpy(w.data(), C.d_hap + MG_HAP_PAD, 4 * (size_t)C.hap_words, cudaMemcpyDeviceToHost));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  if (C.hap_words) MG_CK(ctx, cudaMemcpy(w.data(), C.d_hap + MG_HAP_PAD, 4 * (size_t)C.hap_words, cudaMemcpyDeviceToHost));
   for (int64_t i = 0; i < n; i++) out[i] = (uint8_t)("ACGT"[(w[i >> 4] >> (2 * (i & 15))) & 3]);
   std::vector<MgExc> exc((size_t)C.n_exc);
-  if (C.n_exc) CU(cudaMemcpy(exc.data(), C.d_exc, sizeof(MgExc) * exc.size(), cudaMemcpyDeviceToHost));
+  if (C.n_exc) MG_CK(ctx, cudaMemcpy(exc.data(), C.d_exc, sizeof(MgExc) * exc.size(), cudaMemcpyDeviceToHost));
   for (const MgExc &e : exc)
     for (uint32_t q = 0; q < e.len; q++) out[e.start + q] = e.byte == MG_EXC_CASE ? (uint8_t)(out[e.start + q] | 0x20) : (uint8_t)e.byte;
   return MG_OK;
@@ -758,8 +722,8 @@ static int fill_unit_params(mg_ctx *ctx, const mg_unit_desc *d, MgUnitParams &P,
   if (d->mode == MG_MODE_PHILOX) {
     if (!(d->p > 0.0 && d->p < 1.0)) return fail(ctx, MG_EINVAL, "PHILOX mode needs 0 < p < 1");
     if (n) {
-      CU(ctx->s_tsorted.need(4 * n + 64));
-      CU(ctx->s_partial.need(8 * (n / 2048 + 2)));
+      MG_CK(ctx, ctx->s_tsorted.need(4 * n + 64));
+      MG_CK(ctx, ctx->s_partial.need(8 * (n / 2048 + 2)));
       const MgUnitKeys K0 = mg_unit_keys(d->unit_seed, (uint32_t)n);
       mg_launch_gap_scan((uint32_t)n, d->p, K0.gap0, K0.gap1, ctx->s_tsorted.as<uint32_t>(),
                          ctx->s_partial.as<unsigned long long>(), ctx->stream);
@@ -773,10 +737,10 @@ static int fill_unit_params(mg_ctx *ctx, const mg_unit_desc *d, MgUnitParams &P,
   } else if (d->mode == MG_MODE_DET || d->mode == MG_MODE_EXPLICIT) {
     if (n && (!d->ts || (!d->fo && !sample_only) || (d->mode == MG_MODE_DET ? !d->u_tlen : !d->tl))) return fail(ctx, MG_EINVAL, "deterministic mode needs ts, fo and u_tlen/tl arrays");
     if (n) {
-      CU(ctx->s_ts.need(8 * n)); CU(ctx->s_u.need(8 * n)); CU(ctx->s_fo.need(n));
-      CU(cudaMemcpyAsync(ctx->s_ts.p, d->ts, 8 * n, cudaMemcpyHostToDevice, ctx->stream));
-      CU(cudaMemcpyAsync(ctx->s_u.p, d->mode == MG_MODE_DET ? (const void *)d->u_tlen : (const void *)d->tl, 8 * n, cudaMemcpyHostToDevice, ctx->stream));
-      if (d->fo) CU(cudaMemcpyAsync(ctx->s_fo.p, d->fo, n, cudaMemcpyHostToDevice, ctx->stream));
+      MG_CK(ctx, ctx->s_ts.need(8 * n)); MG_CK(ctx, ctx->s_u.need(8 * n)); MG_CK(ctx, ctx->s_fo.need(n));
+      MG_CK(ctx, cudaMemcpyAsync(ctx->s_ts.p, d->ts, 8 * n, cudaMemcpyHostToDevice, ctx->stream));
+      MG_CK(ctx, cudaMemcpyAsync(ctx->s_u.p, d->mode == MG_MODE_DET ? (const void *)d->u_tlen : (const void *)d->tl, 8 * n, cudaMemcpyHostToDevice, ctx->stream));
+      if (d->fo) MG_CK(ctx, cudaMemcpyAsync(ctx->s_fo.p, d->fo, n, cudaMemcpyHostToDevice, ctx->stream));
     }
     P.ts_in = ctx->s_ts.as<int64_t>();
     if (d->mode == MG_MODE_DET) P.u_tlen = ctx->s_u.as<double>(); else P.tl_in = ctx->s_u.as<int64_t>();
@@ -795,15 +759,15 @@ int mg_sample_templates(mg_ctx *ctx, const mg_unit_desc *d, int64_t *ts_out, int
   if (rc) return rc;
   const size_t n = (size_t)d->n_candidates;
   if (!n) return MG_OK;
-  CU(ctx->s_sample[0].need(8 * n)); CU(ctx->s_sample[1].need(8 * n)); CU(ctx->s_sample[2].need(n));
+  MG_CK(ctx, ctx->s_sample[0].need(8 * n)); MG_CK(ctx, ctx->s_sample[1].need(8 * n)); MG_CK(ctx, ctx->s_sample[2].need(n));
   S.ts_out = ctx->s_sample[0].as<int64_t>(); S.te_out = ctx->s_sample[1].as<int64_t>(); S.fo_out = ctx->s_sample[2].as<int8_t>();
   mg_launch_sample(S, ctx->stream);
   ctx->total_launches++;
-  CU(cudaGetLastError());
-  CU(cudaMemcpyAsync(ts_out, S.ts_out, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(te_out, S.te_out, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(fo_out, S.fo_out, n, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaGetLastError());
+  MG_CK(ctx, cudaMemcpyAsync(ts_out, S.ts_out, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(te_out, S.te_out, 8 * n, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(fo_out, S.fo_out, n, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
   return MG_OK;
 }
 
@@ -848,13 +812,13 @@ static int unit_generate(mg_ctx *ctx, const mg_unit_desc *d, uint8_t *out1, uint
 
   // scan state: [totals 4 x u64][tile counter (16 B)][descA][descB]
   const size_t state_bytes = 48 + 16 * (size_t)std::max(P.n_tiles, 1);
-  CU(ctx->s_state.need(state_bytes));
+  MG_CK(ctx, ctx->s_state.need(state_bytes));
   uint8_t *sb = ctx->s_state.as<uint8_t>();
   P.totals = reinterpret_cast<unsigned long long *>(sb);
   P.tile_counter = reinterpret_cast<uint32_t *>(sb + 32);
   P.descA = reinterpret_cast<unsigned long long *>(sb + 48);
   P.descB = P.descA + std::max(P.n_tiles, 1);
-  CU(ctx->s_plan.need(sizeof(MgPlan) * std::max<size_t>(n, 1)));
+  MG_CK(ctx, ctx->s_plan.need(sizeof(MgPlan) * std::max<size_t>(n, 1)));
   P.plan = ctx->s_plan.as<MgPlan>();
 
   // device output buffers: sized from an estimate, regrown to the exact size on overflow (the plan
@@ -862,10 +826,10 @@ static int unit_generate(mg_ctx *ctx, const mg_unit_desc *d, uint8_t *out1, uint
   size_t est = n * (size_t)(2 * L + 5 + pl + ml + 12 + 2 * 36) / 6 * 5 + 4096;   // ~5/6 of the candidates survive
   const bool want_out = (out1 != nullptr) || (out2 != nullptr);
   unsigned long long tot[4] = {0, 0, 0, 0};
-  CU(cudaMemsetAsync(sb, 0, state_bytes, ctx->stream));
-  CU(cudaEventRecord(ctx->ev2, ctx->stream));
+  MG_CK(ctx, cudaMemsetAsync(sb, 0, state_bytes, ctx->stream));
+  MG_CK(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
   mg_launch_plan(P, ctx->stream);
-  CU(cudaGetLastError());
+  MG_CK(ctx, cudaGetLastError());
   {   // a drain still reading this buffer set (the unit before last) must finish first
     std::unique_lock<std::mutex> lk(ctx->dmu);
     while (ctx->dbusy[ctx->ob] > 0 && !ctx->dfailed) ctx->dcv.wait(lk);
@@ -873,17 +837,17 @@ static int unit_generate(mg_ctx *ctx, const mg_unit_desc *d, uint8_t *out1, uint
   }
   for (int attempt = 0; attempt < 2; attempt++) {
     DevBuf *ob = ctx->s_out[ctx->ob];
-    if (ob[0].cap < est || ob[1].cap < est) CU(cudaStreamSynchronize(ctx->copy_stream));   // regrowing frees the old block
-    CU(ob[0].need(est)); CU(ob[1].need(est));
+    if (ob[0].cap < est || ob[1].cap < est) MG_CK(ctx, cudaStreamSynchronize(ctx->copy_stream));   // regrowing frees the old block
+    MG_CK(ctx, ob[0].need(est)); MG_CK(ctx, ob[1].need(est));
     P.out[0] = ob[0].as<uint8_t>(); P.out[1] = ob[1].as<uint8_t>();
     P.cap = std::min(ob[0].cap, ob[1].cap);
-    CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[ctx->ob], 0));   // this buffer set's previous D2H must be done
-    CU(cudaEventRecord(ctx->ev0, ctx->stream));
+    MG_CK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[ctx->ob], 0));   // this buffer set's previous D2H must be done
+    MG_CK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     mg_launch_unit(P, grid, smem, ctx->stream);
-    CU(cudaEventRecord(ctx->ev1, ctx->stream));
-    CU(cudaGetLastError());
-    CU(cudaMemcpyAsync(tot, P.totals, sizeof tot, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    MG_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    MG_CK(ctx, cudaGetLastError());
+    MG_CK(ctx, cudaMemcpyAsync(tot, P.totals, sizeof tot, cudaMemcpyDeviceToHost, ctx->stream));
+    MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
     if (P.n_tiles) {
       float ms = 0, ms_plan = 0;
       cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
@@ -894,7 +858,7 @@ static int unit_generate(mg_ctx *ctx, const mg_unit_desc *d, uint8_t *out1, uint
     if (!tot[3]) break;
     if (attempt == 1) return fail(ctx, MG_ECUDA, "internal: output overflow after regrow");
     est = (size_t)tot[2] + 4096;
-    CU(cudaMemsetAsync(P.totals + 3, 0, 8, ctx->stream));
+    MG_CK(ctx, cudaMemsetAsync(P.totals + 3, 0, 8, ctx->stream));
   }
   ctx->last_ob = ctx->ob; ctx->last_bytes = (int64_t)tot[2];
   if (n_bytes) *n_bytes = (int64_t)tot[2];
@@ -905,11 +869,11 @@ static int unit_generate(mg_ctx *ctx, const mg_unit_desc *d, uint8_t *out1, uint
     if ((int64_t)tot[2] > cap) return fail(ctx, MG_ECAP, "output needs %lld bytes per file, caller gave %lld", (long long)tot[2], (long long)cap);
     // the kernels have finished (totals were read back): the copies go to their own stream, so the
     // next unit's kernels overlap with them
-    if (out1 && tot[2]) CU(cudaMemcpyAsync(out1, P.out[0], (size_t)tot[2], cudaMemcpyDeviceToHost, ctx->copy_stream));
-    if (out2 && tot[2]) CU(cudaMemcpyAsync(out2, P.out[1], (size_t)tot[2], cudaMemcpyDeviceToHost, ctx->copy_stream));
-    CU(cudaEventRecord(ctx->ev_d2h[ctx->ob], ctx->copy_stream));
+    if (out1 && tot[2]) MG_CK(ctx, cudaMemcpyAsync(out1, P.out[0], (size_t)tot[2], cudaMemcpyDeviceToHost, ctx->copy_stream));
+    if (out2 && tot[2]) MG_CK(ctx, cudaMemcpyAsync(out2, P.out[1], (size_t)tot[2], cudaMemcpyDeviceToHost, ctx->copy_stream));
+    MG_CK(ctx, cudaEventRecord(ctx->ev_d2h[ctx->ob], ctx->copy_stream));
     ctx->ob ^= 1;
-    if (wait_copies) CU(cudaStreamSynchronize(ctx->copy_stream));
+    if (wait_copies) MG_CK(ctx, cudaStreamSynchronize(ctx->copy_stream));
   }
   return MG_OK;
 }
@@ -928,15 +892,15 @@ int mg_unit_read_async(mg_ctx *ctx, int32_t file, int64_t offset, int64_t bytes,
   if (!ctx || !dst || file < 0 || file > 1 || offset < 0 || bytes < 0) return fail(ctx, MG_EINVAL, "mg_unit_read_async: bad arguments");
   if (offset + bytes > ctx->last_bytes) return fail(ctx, MG_EINVAL, "mg_unit_read_async: range beyond the unit's %lld bytes", (long long)ctx->last_bytes);
   DeviceGuard g(ctx->device);
-  if (bytes) CU(cudaMemcpyAsync(dst, ctx->s_out[ctx->last_ob][file].as<uint8_t>() + offset, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->copy_stream));
-  CU(cudaEventRecord(ctx->ev_d2h[ctx->last_ob], ctx->copy_stream));   // the next unit into this buffer set waits for it
+  if (bytes) MG_CK(ctx, cudaMemcpyAsync(dst, ctx->s_out[ctx->last_ob][file].as<uint8_t>() + offset, (size_t)bytes, cudaMemcpyDeviceToHost, ctx->copy_stream));
+  MG_CK(ctx, cudaEventRecord(ctx->ev_d2h[ctx->last_ob], ctx->copy_stream));   // the next unit into this buffer set waits for it
   return MG_OK;
 }
 
 int mg_wait_copies(mg_ctx *ctx) {
   if (!ctx) return MG_EINVAL;
   DeviceGuard g(ctx->device);
-  CU(cudaStreamSynchronize(ctx->copy_stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->copy_stream));
   return MG_OK;
 }
 
@@ -957,26 +921,11 @@ int mg_corrupt_fastq(mg_ctx *ctx, const uint8_t *in1, int64_t len1, const uint8_
   if (nf > ctx->n_mates) return fail(ctx, MG_EINVAL, "paired corruption needs a 2-mate model");
   const uint8_t *in[2] = {in1, in2}; const int64_t len[2] = {len1, len2};
   MgCorruptParams P; memset(&P, 0, sizeof P);
-  int64_t n_lines[2] = {0, 0};
-  for (int f = 0; f < nf; f++) {
-    CU(ctx->c_in[f].need((size_t)len[f] + 16));
-    if (len[f]) CU(cudaMemcpyAsync(ctx->c_in[f].p, in[f], (size_t)len[f], cudaMemcpyHostToDevice, ctx->stream));
-    const int64_t chunks = mg_nl_chunks(len[f]);
-    CU(ctx->c_cnt.need(8 * (size_t)(2 * chunks + 4)));
-    CU(ctx->c_tmp.need(8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>(chunks, 1))));
-    int64_t *cnt = ctx->c_cnt.as<int64_t>(), *off = cnt + chunks + 1;
-    mg_launch_nl_count(ctx->c_in[f].as<uint8_t>(), len[f], cnt, ctx->stream);
-    mg_launch_scan_i64(cnt, off, chunks, ctx->c_tmp.as<int64_t>(), ctx->stream);
-    CU(cudaMemcpyAsync(&n_lines[f], off + chunks, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    CU(ctx->c_nl[f].need(8 * (size_t)(n_lines[f] + 1)));
-    mg_launch_nl_write(ctx->c_in[f].as<uint8_t>(), len[f], off, ctx->c_nl[f].as<int64_t>(), ctx->stream);
-    ctx->total_launches += 5;
-    CU(cudaGetLastError());
-    P.in[f] = ctx->c_in[f].as<uint8_t>(); P.nl[f] = ctx->c_nl[f].as<int64_t>();
-  }
-  int64_t n_rec = n_lines[0] / 4;                                   // zip() of the two readers, readcorrupt.py:53
-  if (nf == 2) n_rec = std::min(n_rec, n_lines[1] / 4);
+  MgFastqChunk &q = ctx->fq;
+  MG_CK(ctx, mg_fastq_load(q, in, len, nf, ctx->stream));
+  ctx->total_launches += 5 * nf;
+  for (int f = 0; f < nf; f++) { P.in[f] = q.in[f].as<uint8_t>(); P.nl[f] = q.nl[f].as<int64_t>(); }
+  const int64_t n_rec = q.n_tpl;                                    // zip() of the two readers, readcorrupt.py:53
   P.n_rec = n_rec; P.n_files = nf;
   P.cum_bq = ctx->m_bq.as<double>(); P.n_cycles = ctx->n_cycles; P.n_bq = ctx->n_bq; P.phred = ctx->m_phred.as<double>();
   P.mode = mode;
@@ -992,60 +941,60 @@ int mg_corrupt_fastq(mg_ctx *ctx, const uint8_t *in1, int64_t len1, const uint8_
   {  // bytes of each input that belong to the n_rec complete templates (the caller streams a large
      // file in chunks and carries the rest over)
     int64_t last[2] = {0, 0};
-    for (int f = 0; f < nf; f++) CU(cudaMemcpyAsync(&last[f], P.nl[f] + (4 * n_rec - 1), 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
+    MG_CK(ctx, mg_fastq_ends(q, n_rec, last, ctx->stream));
+    MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
     if (consumed1) *consumed1 = last[0] + 1;
     if (consumed2 && nf > 1) *consumed2 = last[1] + 1;
   }
 
-  CU(ctx->s_state.need(64));
+  MG_CK(ctx, ctx->s_state.need(64));
   P.err = ctx->s_state.as<unsigned long long>();
-  CU(cudaMemsetAsync(P.err, 0, 16, ctx->stream));
-  CU(ctx->c_tmp.need(8 * (size_t)mg_scan_tmp_elems(n_rec)));
-  for (int f = 0; f < nf; f++) { CU(ctx->c_sz[f].need(8 * (size_t)n_rec)); CU(ctx->c_off[f].need(8 * (size_t)(n_rec + 1))); }
+  MG_CK(ctx, cudaMemsetAsync(P.err, 0, 16, ctx->stream));
+  MG_CK(ctx, q.tmp.need(8 * (size_t)mg_scan_tmp_elems(n_rec)));
+  for (int f = 0; f < nf; f++) { MG_CK(ctx, ctx->c_sz[f].need(8 * (size_t)n_rec)); MG_CK(ctx, ctx->c_off[f].need(8 * (size_t)(n_rec + 1))); }
   mg_launch_corrupt_sizes(P, ctx->c_sz[0].as<int64_t>(), nf > 1 ? ctx->c_sz[1].as<int64_t>() : nullptr, ctx->stream);
   int64_t total[2] = {0, 0};
   for (int f = 0; f < nf; f++) {
-    mg_launch_scan_i64(ctx->c_sz[f].as<int64_t>(), ctx->c_off[f].as<int64_t>(), n_rec, ctx->c_tmp.as<int64_t>(), ctx->stream);
-    CU(cudaMemcpyAsync(&total[f], ctx->c_off[f].as<int64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    mg_launch_scan_i64(ctx->c_sz[f].as<int64_t>(), ctx->c_off[f].as<int64_t>(), n_rec, q.tmp.as<int64_t>(), ctx->stream);
+    MG_CK(ctx, cudaMemcpyAsync(&total[f], ctx->c_off[f].as<int64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, ctx->stream));
     P.out_off[f] = ctx->c_off[f].as<int64_t>();
     ctx->total_launches += 3;
   }
   unsigned long long errv[2] = {0, 0};
-  CU(cudaMemcpyAsync(errv, P.err, 16, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(errv, P.err, 16, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
   const unsigned long long err = errv[0];
   if (err) return fail(ctx, MG_EINDEX, "a read is longer than the model's %d cycles (IndexError in the reference, illumina.py:156)", ctx->n_cycles);
   if (out_len1) *out_len1 = total[0];
   if (out_len2) *out_len2 = total[1];
   if (std::max(total[0], total[1]) > cap) return fail(ctx, MG_ECAP, "output needs %lld bytes, caller gave %lld", (long long)std::max(total[0], total[1]), (long long)cap);
-  for (int f = 0; f < nf; f++) { CU(ctx->c_out[f].need((size_t)total[f] + 16)); P.out[f] = ctx->c_out[f].as<uint8_t>(); }
+  for (int f = 0; f < nf; f++) { MG_CK(ctx, ctx->c_out[f].need((size_t)total[f] + 16)); P.out[f] = ctx->c_out[f].as<uint8_t>(); }
 
   if (mode == MG_MODE_DET) {
     if (!bq_rnd || !call_rnd || !base_rnd || !draw_off) return fail(ctx, MG_EINVAL, "deterministic mode needs the draw arrays");
     const int64_t n_reads = n_rec * nf;
     const int64_t n_draws = draw_off[n_reads];
-    CU(ctx->c_draw[0].need(8 * (size_t)n_draws + 8)); CU(ctx->c_draw[1].need(8 * (size_t)n_draws + 8));
-    CU(ctx->c_draw[2].need((size_t)n_draws + 8)); CU(ctx->c_draw[3].need(8 * (size_t)(n_reads + 1)));
-    CU(cudaMemcpyAsync(ctx->c_draw[0].p, bq_rnd, 8 * (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->c_draw[1].p, call_rnd, 8 * (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->c_draw[2].p, base_rnd, (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->c_draw[3].p, draw_off, 8 * (size_t)(n_reads + 1), cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, ctx->c_draw[0].need(8 * (size_t)n_draws + 8)); MG_CK(ctx, ctx->c_draw[1].need(8 * (size_t)n_draws + 8));
+    MG_CK(ctx, ctx->c_draw[2].need((size_t)n_draws + 8)); MG_CK(ctx, ctx->c_draw[3].need(8 * (size_t)(n_reads + 1)));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->c_draw[0].p, bq_rnd, 8 * (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->c_draw[1].p, call_rnd, 8 * (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->c_draw[2].p, base_rnd, (size_t)n_draws, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->c_draw[3].p, draw_off, 8 * (size_t)(n_reads + 1), cudaMemcpyHostToDevice, ctx->stream));
     P.bq_rnd = ctx->c_draw[0].as<double>(); P.call_rnd = ctx->c_draw[1].as<double>();
     P.base_rnd = ctx->c_draw[2].as<uint8_t>(); P.draw_off = ctx->c_draw[3].as<int64_t>();
   }
-  CU(cudaEventRecord(ctx->ev0, ctx->stream));
+  MG_CK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
   {
     static const bool lsu = getenv("MG_COPYOUT_LSU") != nullptr, old = getenv("MG_CORRUPT_SIMPLE") != nullptr;
     // production mode, every record fits a warp's stage: the staged kernel; else (deterministic draws, giant names) the simple one
     if (mode == MG_MODE_PHILOX && !old && errv[1] + 16 <= (unsigned long long)mg_corrupt_stage_cap()) mg_launch_corrupt_staged(P, !lsu, ctx->stream);
     else mg_launch_corrupt(P, ctx->stream);
   }
-  CU(cudaEventRecord(ctx->ev1, ctx->stream));
-  CU(cudaGetLastError());
-  if (out1) CU(cudaMemcpyAsync(out1, P.out[0], (size_t)total[0], cudaMemcpyDeviceToHost, ctx->stream));
-  if (nf > 1 && out2) CU(cudaMemcpyAsync(out2, P.out[1], (size_t)total[1], cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
+  MG_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  MG_CK(ctx, cudaGetLastError());
+  if (out1) MG_CK(ctx, cudaMemcpyAsync(out1, P.out[0], (size_t)total[0], cudaMemcpyDeviceToHost, ctx->stream));
+  if (nf > 1 && out2) MG_CK(ctx, cudaMemcpyAsync(out2, P.out[1], (size_t)total[1], cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));
   float ms = 0; cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
   ctx->emit_ms += ms; ctx->emit_launches++; ctx->total_launches++;
   ctx->emit_bytes += 2 * (total[0] + total[1]);
@@ -1054,7 +1003,42 @@ int mg_corrupt_fastq(mg_ctx *ctx, const uint8_t *in1, int64_t len1, const uint8_
 
 }  // extern "C"
 
-// ---- internal views for mg_check.cu ----------------------------------------------------------------
+// ---- FASTQ ingest (corrupt-reads, check-reads, god-aligner) ----------------------------------------
+
+cudaError_t mg_fastq_load(MgFastqChunk &q, const uint8_t *const in[2], const int64_t len[2], int nf, cudaStream_t st) {
+#define TRY(call) do { const cudaError_t e_ = (call); if (e_ != cudaSuccess) return e_; } while (0)
+  int64_t n_lines[2] = {0, 0};
+  for (int f = 0; f < nf; f++) {
+    TRY(q.in[f].need((size_t)len[f] + 16));
+    if (len[f]) TRY(cudaMemcpyAsync(q.in[f].p, in[f], (size_t)len[f], cudaMemcpyHostToDevice, st));
+    const int64_t chunks = mg_nl_chunks(len[f]);
+    TRY(q.cnt.need(8 * (size_t)(2 * chunks + 4)));
+    TRY(q.tmp.need(8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>(chunks, 1))));
+    int64_t *cnt = q.cnt.as<int64_t>(), *off = cnt + chunks + 1;
+    mg_launch_nl_count(q.in[f].as<uint8_t>(), len[f], cnt, st);
+    mg_launch_scan_i64(cnt, off, chunks, q.tmp.as<int64_t>(), st);
+    TRY(cudaMemcpyAsync(&n_lines[f], off + chunks, 8, cudaMemcpyDeviceToHost, st));
+    TRY(cudaStreamSynchronize(st));
+    TRY(q.nl[f].need(8 * (size_t)(n_lines[f] + 1)));
+    mg_launch_nl_write(q.in[f].as<uint8_t>(), len[f], off, q.nl[f].as<int64_t>(), st);
+    TRY(cudaGetLastError());
+  }
+#undef TRY
+  q.nf = nf;
+  q.n_tpl = n_lines[0] / 4;
+  if (nf == 2) q.n_tpl = std::min(q.n_tpl, n_lines[1] / 4);
+  return cudaSuccess;
+}
+
+cudaError_t mg_fastq_ends(const MgFastqChunk &q, int64_t k, int64_t last[2], cudaStream_t st) {
+  for (int f = 0; f < q.nf; f++) {
+    const cudaError_t e = cudaMemcpyAsync(&last[f], q.nl[f].as<int64_t>() + (4 * k - 1), 8, cudaMemcpyDeviceToHost, st);
+    if (e != cudaSuccess) return e;
+  }
+  return cudaSuccess;
+}
+
+// ---- internal views for mg_check.cu, mg_bam.cu and mg_readmodel.cu ---------------------------------
 int mg_internal_copy_view(mg_ctx *ctx, int64_t copy_id, int64_t *region_id, const MgNode **nodes, int *n_nodes, const uint32_t **hap, uint32_t *hap_len,
                           const MgExc **exc, int *n_exc, int64_t *start1) {
   auto it = ctx->copies.find(copy_id);
@@ -1076,6 +1060,9 @@ int mg_internal_region_view(mg_ctx *ctx, int64_t region_id, const uint32_t **ref
 cudaStream_t mg_internal_stream(mg_ctx *ctx) { return ctx->stream; }
 int mg_internal_device(mg_ctx *ctx) { return ctx->device; }
 int mg_internal_fail(mg_ctx *ctx, int code, const char *msg) { return fail(ctx, code, "%s", msg); }
+int mg_internal_cuda_fail(mg_ctx *ctx, cudaError_t e, const char *call, const char *file, int line) {
+  return fail(ctx, MG_ECUDA, "%s: %s (%s:%d)", call, cudaGetErrorString(e), file, line);
+}
 
 extern "C" {
 
@@ -1312,42 +1299,42 @@ int mg_batch_generate(mg_ctx *ctx, int64_t batch_id, int64_t n_units, const int3
 
   // -- device tables: [units][unit_kept n+1][unit_bytes n+1][unit_te n+1][kept_base n+2][byte_base n+2][scan tmp]
   const size_t nu = (size_t)n_units;
-  CU(ctx->b_units.need(sizeof(MgBatchUnit) * nu));
+  MG_CK(ctx, ctx->b_units.need(sizeof(MgBatchUnit) * nu));
   const size_t tmp_elems = (size_t)mg_scan_tmp_elems((int64_t)nu);
-  CU(ctx->b_arr.need(8 * (3 * (nu + 1) + 2 * (nu + 2) + tmp_elems + 8)));
+  MG_CK(ctx, ctx->b_arr.need(8 * (3 * (nu + 1) + 2 * (nu + 2) + tmp_elems + 8)));
   long long *arr = ctx->b_arr.as<long long>();
   P.bunits = ctx->b_units.as<MgBatchUnit>(); P.n_bunits = (int)n_units;
   P.unit_kept = arr; P.unit_bytes = arr + (nu + 1); P.unit_te = arr + 2 * (nu + 1);
   long long *kept_base = arr + 3 * (nu + 1), *byte_base = kept_base + (nu + 2), *scan_tmp = byte_base + (nu + 2);
   P.kept_base = kept_base; P.byte_base = byte_base;
-  CU(ctx->s_state.need(64));
+  MG_CK(ctx, ctx->s_state.need(64));
   P.totals = ctx->s_state.as<unsigned long long>();
-  CU(cudaMemsetAsync(P.totals, 0, 64, ctx->stream));
-  CU(ctx->s_plan.need(sizeof(MgPlan) * std::max<size_t>((size_t)n_plan, 1)));
+  MG_CK(ctx, cudaMemsetAsync(P.totals, 0, 64, ctx->stream));
+  MG_CK(ctx, ctx->s_plan.need(sizeof(MgPlan) * std::max<size_t>((size_t)n_plan, 1)));
   P.plan = ctx->s_plan.as<MgPlan>();
-  CU(cudaMemcpyAsync(ctx->b_units.p, U.data(), sizeof(MgBatchUnit) * nu, cudaMemcpyHostToDevice, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(ctx->b_units.p, U.data(), sizeof(MgBatchUnit) * nu, cudaMemcpyHostToDevice, ctx->stream));
   if (mode == MG_MODE_DET && n_draws) {
     const size_t nd = (size_t)n_draws;
-    CU(ctx->s_ts.need(8 * nd)); CU(ctx->s_u.need(8 * nd)); CU(ctx->s_fo.need(nd));
-    CU(cudaMemcpyAsync(ctx->s_ts.p, ts, 8 * nd, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->s_u.p, u_tlen, 8 * nd, cudaMemcpyHostToDevice, ctx->stream));
-    CU(cudaMemcpyAsync(ctx->s_fo.p, fo, nd, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, ctx->s_ts.need(8 * nd)); MG_CK(ctx, ctx->s_u.need(8 * nd)); MG_CK(ctx, ctx->s_fo.need(nd));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->s_ts.p, ts, 8 * nd, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->s_u.p, u_tlen, 8 * nd, cudaMemcpyHostToDevice, ctx->stream));
+    MG_CK(ctx, cudaMemcpyAsync(ctx->s_fo.p, fo, nd, cudaMemcpyHostToDevice, ctx->stream));
   }
   P.ts_in = ctx->s_ts.as<int64_t>(); P.u_tlen = ctx->s_u.as<double>(); P.fo_in = ctx->s_fo.as<int8_t>();
 
-  CU(cudaEventRecord(ctx->ev2, ctx->stream));
+  MG_CK(ctx, cudaEventRecord(ctx->ev2, ctx->stream));
   mg_launch_batch_plan(P, ctx->stream);
   mg_launch_scan_i64(reinterpret_cast<const int64_t *>(P.unit_kept), reinterpret_cast<int64_t *>(kept_base), (int64_t)nu, reinterpret_cast<int64_t *>(scan_tmp), ctx->stream);
   mg_launch_scan_i64(reinterpret_cast<const int64_t *>(P.unit_bytes), reinterpret_cast<int64_t *>(byte_base), (int64_t)nu, reinterpret_cast<int64_t *>(scan_tmp), ctx->stream);
-  CU(cudaGetLastError());
+  MG_CK(ctx, cudaGetLastError());
   ctx->total_launches += 7;
   std::vector<long long> h_bytes(nu), h_kept(nu);
   long long tot_kept = 0, tot_bytes = 0;
-  CU(cudaMemcpyAsync(h_bytes.data(), P.unit_bytes, 8 * nu, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(h_kept.data(), P.unit_kept, 8 * nu, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(&tot_kept, kept_base + nu, 8, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaMemcpyAsync(&tot_bytes, byte_base + nu, 8, cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));             // the sizes: the one read-back of a batch
+  MG_CK(ctx, cudaMemcpyAsync(h_bytes.data(), P.unit_bytes, 8 * nu, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(h_kept.data(), P.unit_kept, 8 * nu, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(&tot_kept, kept_base + nu, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaMemcpyAsync(&tot_bytes, byte_base + nu, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));             // the sizes: the one read-back of a batch
 
   {   // a drain still reading this buffer set must finish first
     std::unique_lock<std::mutex> lk(ctx->dmu);
@@ -1356,16 +1343,16 @@ int mg_batch_generate(mg_ctx *ctx, int64_t batch_id, int64_t n_units, const int3
   }
   DevBuf *ob = ctx->s_out[ctx->ob];
   const size_t need = (size_t)tot_bytes + 4096;
-  if (ob[0].cap < need || ob[1].cap < need) CU(cudaStreamSynchronize(ctx->copy_stream));
-  CU(ob[0].need(need)); CU(ob[1].need(need));
+  if (ob[0].cap < need || ob[1].cap < need) MG_CK(ctx, cudaStreamSynchronize(ctx->copy_stream));
+  MG_CK(ctx, ob[0].need(need)); MG_CK(ctx, ob[1].need(need));
   P.out[0] = ob[0].as<uint8_t>(); P.out[1] = ob[1].as<uint8_t>();
   P.cap = std::min(ob[0].cap, ob[1].cap);
-  CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[ctx->ob], 0));
-  CU(cudaEventRecord(ctx->ev0, ctx->stream));
+  MG_CK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_d2h[ctx->ob], 0));
+  MG_CK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
   mg_launch_batch_emit(P, grid, smem, ctx->stream);
-  CU(cudaEventRecord(ctx->ev1, ctx->stream));
-  CU(cudaGetLastError());
-  CU(cudaStreamSynchronize(ctx->stream));             // the drain thread copies from another stream
+  MG_CK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  MG_CK(ctx, cudaGetLastError());
+  MG_CK(ctx, cudaStreamSynchronize(ctx->stream));             // the drain thread copies from another stream
   {
     float ms = 0, ms_plan = 0;
     cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1); cudaEventElapsedTime(&ms_plan, ctx->ev2, ctx->ev0);

@@ -2,7 +2,7 @@
 // mitty/benchmarking/god_aligner.py), encoded and sorted on the device.
 //
 // Per FASTQ chunk (both files of a pair in step):
-//   ingest    H2D, newline index (k_nl_count / scan / k_nl_write, as corrupt-reads and check-reads)
+//   ingest    H2D, newline index (mg_fastq_load, shared with corrupt-reads and check-reads)
 //   k_bam_size    one thread per read: qname parse (mg_qname.cuh), contig lookup, validation; record size,
 //                 sort key (refID, pos, reverse bit), error code
 //   scan          record offsets of the chunk
@@ -33,10 +33,6 @@
 #include "mg_bgzf.h"
 #include "mg_internal.h"
 #include "mg_qname.cuh"
-
-cudaStream_t mg_internal_stream(mg_ctx *ctx);
-int mg_internal_device(mg_ctx *ctx);
-int mg_internal_fail(mg_ctx *ctx, int code, const char *msg);
 
 namespace {
 
@@ -324,29 +320,6 @@ __global__ void __launch_bounds__(256) k_gather_copy(const uint32_t *__restrict_
 
 // ---- host side ---------------------------------------------------------------------------------------
 
-cudaError_t grow(void **p, size_t &cap, size_t bytes) {
-  if (bytes <= cap) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr; cap = 0;
-  const cudaError_t e = cudaMalloc(p, bytes + bytes / 8 + 256);
-  if (e == cudaSuccess) cap = bytes + bytes / 8 + 256;
-  return e;
-}
-
-// as grow, keeping the first `keep` bytes
-cudaError_t grow_keep(void **p, size_t &cap, size_t bytes, size_t keep, cudaStream_t st) {
-  if (bytes <= cap) return cudaSuccess;
-  void *q = nullptr;
-  const size_t c = bytes + bytes / 4 + 256;
-  cudaError_t e = cudaMalloc(&q, c);
-  if (e != cudaSuccess) return e;
-  if (keep) e = cudaMemcpyAsync(q, *p, keep, cudaMemcpyDeviceToDevice, st);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-  if (*p) cudaFree(*p);
-  *p = q; cap = c;
-  return e;
-}
-
 bool write_all(int fd, const void *p, size_t n) {
   const uint8_t *b = static_cast<const uint8_t *>(p);
   while (n > 0) {
@@ -409,68 +382,66 @@ struct Bam {
   std::vector<uint8_t> header;
   std::string rg;
   // contig table, RG value
-  void *d_names = nullptr, *d_name_off = nullptr, *d_len = nullptr, *d_rg = nullptr;
+  DevBuf d_names, d_name_off, d_len, d_rg;
   // chunk
-  void *d_in[2] = {nullptr, nullptr}, *d_nl[2] = {nullptr, nullptr}, *d_cnt = nullptr, *d_tmp = nullptr;
-  void *d_csz = nullptr, *d_ckey = nullptr, *d_coff = nullptr, *d_code = nullptr, *d_bad = nullptr;
-  size_t c_in[2] = {0, 0}, c_nl[2] = {0, 0}, c_cnt = 0, c_tmp = 0, c_csz = 0, c_ckey = 0, c_coff = 0, c_code = 0;
+  MgFastqChunk fq;
+  DevBuf d_csz, d_ckey, d_coff, d_code, d_bad;
   // run
-  void *d_rec = nullptr, *d_key = nullptr, *d_size = nullptr, *d_roff = nullptr;
-  size_t c_rec = 0, c_key = 0, c_size = 0, c_roff = 0;
+  DevBuf d_rec, d_key, d_size, d_roff;
   int64_t run_n = 0, run_rec = 0;
   // sort / gather
-  void *d_key2 = nullptr, *d_ord = nullptr, *d_ord2 = nullptr, *d_hist = nullptr, *d_hoff = nullptr, *d_stmp = nullptr, *d_ssize = nullptr,
-       *d_soff = nullptr, *d_out = nullptr;
-  size_t c_key2 = 0, c_ord = 0, c_ord2 = 0, c_hist = 0, c_hoff = 0, c_stmp = 0, c_ssize = 0, c_soff = 0, c_out = 0;
-  uint8_t *pin[2] = {nullptr, nullptr};
-  cudaEvent_t ev0[2], ev1[2];
+  DevBuf d_key2, d_ord, d_ord2, d_hist, d_hoff, d_stmp, d_ssize, d_soff, d_out;
+  HostBuf pin[2];
+  cudaEvent_t ev0[2] = {}, ev1[2] = {};
   std::vector<std::string> spills;
   int64_t n_runs = 0;
   double t_dev = 0, t_d2h = 0, t_out = 0;     // ms: ingest + encode + sort + gather; device-to-host copies; writing (deflate, spill, merge)
+  ~Bam() {
+    for (int k = 0; k < 2; k++) { if (ev0[k]) cudaEventDestroy(ev0[k]); if (ev1[k]) cudaEventDestroy(ev1[k]); }
+    for (const std::string &s : spills) unlink(s.c_str());
+  }
 };
 
 double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 int bam_fail(Bam &b, int code, const std::string &msg) { return mg_internal_fail(b.ctx, code, msg.c_str()); }
 
-#define CK(call) do { if ((call) != cudaSuccess) return bam_fail(b, MG_ECUDA, #call); } while (0)
-
 // sorts and gathers the current run into d_out (records in key order, d_key2 <- keys in key order)
 int sort_run(Bam &b) {
   cudaStream_t st = mg_internal_stream(b.ctx);
   const int64_t n = b.run_n;
   const int nb = (int)((n + RS_TILE - 1) / RS_TILE);
-  CK(grow(&b.d_key2, b.c_key2, 8 * (size_t)n + 8));
-  CK(grow(&b.d_ord, b.c_ord, 4 * (size_t)n + 4));
-  CK(grow(&b.d_ord2, b.c_ord2, 4 * (size_t)n + 4));
-  CK(grow(&b.d_hist, b.c_hist, 8 * (size_t)nb * 256 + 8));
-  CK(grow(&b.d_hoff, b.c_hoff, 8 * ((size_t)nb * 256 + 1)));
-  CK(grow(&b.d_stmp, b.c_stmp, 8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>({(int64_t)nb * 256, n, 1}))));
-  CK(grow(&b.d_ssize, b.c_ssize, 8 * (size_t)n + 8));
-  CK(grow(&b.d_soff, b.c_soff, 8 * ((size_t)n + 1)));
-  CK(grow(&b.d_out, b.c_out, (size_t)b.run_rec + 16));
+  MG_CK(b.ctx, b.d_key2.need(8 * (size_t)n + 8));
+  MG_CK(b.ctx, b.d_ord.need(4 * (size_t)n + 4));
+  MG_CK(b.ctx, b.d_ord2.need(4 * (size_t)n + 4));
+  MG_CK(b.ctx, b.d_hist.need(8 * (size_t)nb * 256 + 8));
+  MG_CK(b.ctx, b.d_hoff.need(8 * ((size_t)nb * 256 + 1)));
+  MG_CK(b.ctx, b.d_stmp.need(8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>({(int64_t)nb * 256, n, 1}))));
+  MG_CK(b.ctx, b.d_ssize.need(8 * (size_t)n + 8));
+  MG_CK(b.ctx, b.d_soff.need(8 * ((size_t)n + 1)));
+  MG_CK(b.ctx, b.d_out.need((size_t)b.run_rec + 16));
   const unsigned g = (unsigned)((n + 255) / 256);
-  uint64_t *k[2] = {static_cast<uint64_t *>(b.d_key), static_cast<uint64_t *>(b.d_key2)};
-  uint32_t *o[2] = {static_cast<uint32_t *>(b.d_ord), static_cast<uint32_t *>(b.d_ord2)};
+  uint64_t *k[2] = {b.d_key.as<uint64_t>(), b.d_key2.as<uint64_t>()};
+  uint32_t *o[2] = {b.d_ord.as<uint32_t>(), b.d_ord2.as<uint32_t>()};
   k_iota<<<g, 256, 0, st>>>(o[0], n);
   const int passes = std::max(1, (b.key_bits + 7) / 8);
   int s = 0;
   for (int p = 0; p < passes; p++, s ^= 1) {
-    k_radix_hist<<<nb, RS_THREADS, 0, st>>>(k[s], n, 8 * p, static_cast<int64_t *>(b.d_hist), nb);
-    mg_launch_scan_i64(static_cast<int64_t *>(b.d_hist), static_cast<int64_t *>(b.d_hoff), (int64_t)nb * 256, static_cast<int64_t *>(b.d_stmp), st);
-    k_radix_scatter<<<nb, RS_THREADS, 0, st>>>(k[s], o[s], k[s ^ 1], o[s ^ 1], n, 8 * p, static_cast<int64_t *>(b.d_hoff), nb);
+    k_radix_hist<<<nb, RS_THREADS, 0, st>>>(k[s], n, 8 * p, b.d_hist.as<int64_t>(), nb);
+    mg_launch_scan_i64(b.d_hist.as<int64_t>(), b.d_hoff.as<int64_t>(), (int64_t)nb * 256, b.d_stmp.as<int64_t>(), st);
+    k_radix_scatter<<<nb, RS_THREADS, 0, st>>>(k[s], o[s], k[s ^ 1], o[s ^ 1], n, 8 * p, b.d_hoff.as<int64_t>(), nb);
   }
   if (s == 0) {   // keep the sorted keys in d_key2 and the ordinals in d_ord2
-    CK(cudaMemcpyAsync(b.d_key2, b.d_key, 8 * (size_t)n, cudaMemcpyDeviceToDevice, st));
-    CK(cudaMemcpyAsync(b.d_ord2, b.d_ord, 4 * (size_t)n, cudaMemcpyDeviceToDevice, st));
+    MG_CK(b.ctx, cudaMemcpyAsync(b.d_key2.p, b.d_key.p, 8 * (size_t)n, cudaMemcpyDeviceToDevice, st));
+    MG_CK(b.ctx, cudaMemcpyAsync(b.d_ord2.p, b.d_ord.p, 4 * (size_t)n, cudaMemcpyDeviceToDevice, st));
   }
-  const uint32_t *ord = static_cast<const uint32_t *>(b.d_ord2);
-  k_gather_sizes<<<g, 256, 0, st>>>(ord, static_cast<int64_t *>(b.d_size), static_cast<int64_t *>(b.d_ssize), n);
-  mg_launch_scan_i64(static_cast<int64_t *>(b.d_ssize), static_cast<int64_t *>(b.d_soff), n, static_cast<int64_t *>(b.d_stmp), st);
-  k_gather_copy<<<(unsigned)((32 * n + 255) / 256), 256, 0, st>>>(ord, static_cast<int64_t *>(b.d_roff), static_cast<int64_t *>(b.d_soff),
-                                                                  static_cast<uint8_t *>(b.d_rec), static_cast<uint8_t *>(b.d_out), n);
-  CK(cudaGetLastError());
-  CK(cudaStreamSynchronize(st));
+  const uint32_t *ord = b.d_ord2.as<const uint32_t>();
+  k_gather_sizes<<<g, 256, 0, st>>>(ord, b.d_size.as<int64_t>(), b.d_ssize.as<int64_t>(), n);
+  mg_launch_scan_i64(b.d_ssize.as<int64_t>(), b.d_soff.as<int64_t>(), n, b.d_stmp.as<int64_t>(), st);
+  k_gather_copy<<<(unsigned)((32 * n + 255) / 256), 256, 0, st>>>(ord, b.d_roff.as<int64_t>(), b.d_soff.as<int64_t>(), b.d_rec.as<uint8_t>(),
+                                                                  b.d_out.as<uint8_t>(), n);
+  MG_CK(b.ctx, cudaGetLastError());
+  MG_CK(b.ctx, cudaStreamSynchronize(st));
   return MG_OK;
 }
 
@@ -482,15 +453,15 @@ int stream_out(Bam &b, const uint8_t *src, int64_t bytes, F sink) {
   for (int64_t off = 0; off < bytes || prev >= 0; off += kPiece, k ^= 1) {
     const int64_t m = std::min(kPiece, bytes - off);
     if (m > 0) {
-      CK(cudaEventRecord(b.ev0[k], st));
-      CK(cudaMemcpyAsync(b.pin[k], src + off, (size_t)m, cudaMemcpyDeviceToHost, st));
-      CK(cudaEventRecord(b.ev1[k], st));
+      MG_CK(b.ctx, cudaEventRecord(b.ev0[k], st));
+      MG_CK(b.ctx, cudaMemcpyAsync(b.pin[k].p, src + off, (size_t)m, cudaMemcpyDeviceToHost, st));
+      MG_CK(b.ctx, cudaEventRecord(b.ev1[k], st));
     }
     if (prev >= 0) {
-      CK(cudaEventSynchronize(b.ev1[k ^ 1]));
+      MG_CK(b.ctx, cudaEventSynchronize(b.ev1[k ^ 1]));
       float ms = 0; cudaEventElapsedTime(&ms, b.ev0[k ^ 1], b.ev1[k ^ 1]); b.t_d2h += ms;
       const double t = now_ms();
-      if (!sink(b.pin[k ^ 1], prev)) return MG_EVALUE;
+      if (!sink(b.pin[k ^ 1].as<const uint8_t>(), prev)) return MG_EVALUE;
       b.t_out += now_ms() - t;
     }
     prev = m > 0 ? m : -1;
@@ -512,8 +483,8 @@ int spill_run(Bam &b) {
   const int64_t hdr[2] = {b.run_n, b.run_rec};
   bool ok = write_all(fd, hdr, sizeof hdr);
   rc = MG_OK;
-  if (ok) rc = stream_out(b, static_cast<uint8_t *>(b.d_key2), 8 * b.run_n, [&](const uint8_t *p, int64_t n) { return write_all(fd, p, (size_t)n); });
-  if (ok && !rc) rc = stream_out(b, static_cast<uint8_t *>(b.d_out), b.run_rec, [&](const uint8_t *p, int64_t n) { return write_all(fd, p, (size_t)n); });
+  if (ok) rc = stream_out(b, b.d_key2.as<const uint8_t>(), 8 * b.run_n, [&](const uint8_t *p, int64_t n) { return write_all(fd, p, (size_t)n); });
+  if (ok && !rc) rc = stream_out(b, b.d_out.as<const uint8_t>(), b.run_rec, [&](const uint8_t *p, int64_t n) { return write_all(fd, p, (size_t)n); });
   ok = close(fd) == 0 && ok;
   if (!ok || rc) return bam_fail(b, MG_EVALUE, "cannot write the temporary run file " + b.spills.back());
   b.n_runs++;
@@ -551,17 +522,6 @@ int merge_runs(Bam &b, MgBamWriter &w) {
   return rc ? bam_fail(b, MG_EVALUE, "merging the sorted runs failed: " + w.err) : MG_OK;
 }
 
-void bam_free(Bam &b) {
-  cudaSetDevice(mg_internal_device(b.ctx));
-  cudaStreamSynchronize(mg_internal_stream(b.ctx));
-  for (void *p : {b.d_names, b.d_name_off, b.d_len, b.d_rg, b.d_in[0], b.d_in[1], b.d_nl[0], b.d_nl[1], b.d_cnt, b.d_tmp, b.d_csz, b.d_ckey, b.d_coff,
-                  b.d_code, b.d_bad, b.d_rec, b.d_key, b.d_size, b.d_roff, b.d_key2, b.d_ord, b.d_ord2, b.d_hist, b.d_hoff, b.d_stmp, b.d_ssize,
-                  b.d_soff, b.d_out}) if (p) cudaFree(p);
-  for (uint8_t *p : b.pin) if (p) cudaFreeHost(p);
-  for (int k = 0; k < 2; k++) { cudaEventDestroy(b.ev0[k]); cudaEventDestroy(b.ev1[k]); }
-  for (const std::string &s : b.spills) unlink(s.c_str());
-}
-
 int bit_length(uint64_t x) { int n = 0; while (x) { n++; x >>= 1; } return n; }
 
 }  // namespace
@@ -569,6 +529,12 @@ int bit_length(uint64_t x) { int n = 0; while (x) { n++; x >>= 1; } return n; }
 extern "C" {
 
 struct mg_bam { Bam b; };
+
+static void bam_delete(mg_bam *h) {       // once the stream is idle; the temporary run files go with it
+  DeviceGuard g(mg_internal_device(h->b.ctx));
+  cudaStreamSynchronize(mg_internal_stream(h->b.ctx));
+  delete h;
+}
 
 int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t n_ref, const char *const *ref_names, const int64_t *ref_len,
                 const char *header_text, const char *sample, int32_t level, int32_t threads, int64_t run_bytes, mg_bam **out) {
@@ -584,7 +550,7 @@ int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t
   // with every contig below 2^31, pos + span <= ref_len bounds POS, PNEXT and TLEN to int32
   const std::string bad = mg_bam_check_contigs(names, lens);
   if (!bad.empty()) return mg_internal_fail(ctx, MG_EVALUE, ("mg_bam_open: " + bad).c_str());
-  cudaSetDevice(mg_internal_device(ctx));
+  DeviceGuard g(mg_internal_device(ctx));
   mg_bam *h = new mg_bam();
   Bam &b = h->b;
   b.ctx = ctx; b.bam = bam_path; b.bai = bai_path ? bai_path : ""; b.n_ref = n_ref; b.level = level; b.threads = std::max(1, (int)threads);
@@ -601,19 +567,19 @@ int mg_bam_open(mg_ctx *ctx, const char *bam_path, const char *bai_path, int32_t
   cudaStream_t st = mg_internal_stream(ctx);
   int rc = MG_OK;
   pool.push_back(0);
-  auto up = [&](void **d, const void *src, size_t n) {
-    if (cudaMalloc(d, std::max<size_t>(n, 8)) != cudaSuccess || cudaMemcpyAsync(*d, src, n, cudaMemcpyHostToDevice, st) != cudaSuccess) rc = MG_ECUDA;
+  auto up = [&](DevBuf &d, const void *src, size_t n) {
+    if (d.need(std::max<size_t>(n, 8)) != cudaSuccess || cudaMemcpyAsync(d.p, src, n, cudaMemcpyHostToDevice, st) != cudaSuccess) rc = MG_ECUDA;
   };
-  up(&b.d_names, pool.data(), pool.size());
-  up(&b.d_name_off, noff.data(), 4 * noff.size());
-  up(&b.d_len, lens.data(), 8 * lens.size());
-  up(&b.d_rg, b.rg.data(), b.rg.size() + 1);
+  up(b.d_names, pool.data(), pool.size());
+  up(b.d_name_off, noff.data(), 4 * noff.size());
+  up(b.d_len, lens.data(), 8 * lens.size());
+  up(b.d_rg, b.rg.data(), b.rg.size() + 1);
   for (int k = 0; k < 2 && !rc; k++) {
-    if (cudaMallocHost((void **)&b.pin[k], (size_t)kPiece) != cudaSuccess) rc = MG_ECUDA;
+    if (b.pin[k].need((size_t)kPiece) != cudaSuccess) rc = MG_ECUDA;
     cudaEventCreate(&b.ev0[k]); cudaEventCreate(&b.ev1[k]);
   }
   if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = MG_ECUDA;
-  if (rc) { bam_free(b); delete h; return mg_internal_fail(ctx, MG_ECUDA, "mg_bam_open: out of device or page-locked memory"); }
+  if (rc) { bam_delete(h); return mg_internal_fail(ctx, MG_ECUDA, "mg_bam_open: out of device or page-locked memory"); }
   *out = h;
   return MG_OK;
 }
@@ -622,7 +588,7 @@ int mg_bam_add(mg_bam *h, const uint8_t *in1, int64_t len1, const uint8_t *in2, 
                int64_t *consumed2, int64_t *bad_index, int32_t *bad_code) {
   if (!h || !in1 || len1 < 0 || (in2 && len2 < 0)) return MG_EINVAL;
   Bam &b = h->b;
-  cudaSetDevice(mg_internal_device(b.ctx));
+  DeviceGuard g(mg_internal_device(b.ctx));
   cudaStream_t st = mg_internal_stream(b.ctx);
   const double t0 = now_ms();
   if (n_templates) *n_templates = 0;
@@ -632,51 +598,35 @@ int mg_bam_add(mg_bam *h, const uint8_t *in1, int64_t len1, const uint8_t *in2, 
   if (bad_code) *bad_code = 0;
   const int nf = in2 ? 2 : 1;
   const uint8_t *in[2] = {in1, in2}; const int64_t len[2] = {len1, len2};
-  int64_t n_lines[2] = {0, 0};
-  BamParams P; memset(&P, 0, sizeof P);
-  for (int f = 0; f < nf; f++) {
-    CK(grow(&b.d_in[f], b.c_in[f], (size_t)len[f] + 16));
-    if (len[f]) CK(cudaMemcpyAsync(b.d_in[f], in[f], (size_t)len[f], cudaMemcpyHostToDevice, st));
-    const int64_t chunks = mg_nl_chunks(len[f]);
-    CK(grow(&b.d_cnt, b.c_cnt, 8 * (size_t)(2 * chunks + 4)));
-    CK(grow(&b.d_tmp, b.c_tmp, 8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>(chunks, 1))));
-    int64_t *cnt = static_cast<int64_t *>(b.d_cnt), *off = cnt + chunks + 1;
-    mg_launch_nl_count(static_cast<uint8_t *>(b.d_in[f]), len[f], cnt, st);
-    mg_launch_scan_i64(cnt, off, chunks, static_cast<int64_t *>(b.d_tmp), st);
-    CK(cudaMemcpyAsync(&n_lines[f], off + chunks, 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    CK(grow(&b.d_nl[f], b.c_nl[f], 8 * (size_t)(n_lines[f] + 1)));
-    mg_launch_nl_write(static_cast<uint8_t *>(b.d_in[f]), len[f], off, static_cast<int64_t *>(b.d_nl[f]), st);
-    P.fq[f] = static_cast<uint8_t *>(b.d_in[f]); P.nl[f] = static_cast<int64_t *>(b.d_nl[f]);
-  }
-  int64_t n_tpl = n_lines[0] / 4;
-  if (nf == 2) n_tpl = std::min(n_tpl, n_lines[1] / 4);
+  MG_CK(b.ctx, mg_fastq_load(b.fq, in, len, nf, st));
+  const int64_t n_tpl = b.fq.n_tpl;
   if (n_tpl == 0) return MG_OK;
   const int64_t n = n_tpl * nf;
+  BamParams P; memset(&P, 0, sizeof P);
+  for (int f = 0; f < nf; f++) { P.fq[f] = b.fq.in[f].as<uint8_t>(); P.nl[f] = b.fq.nl[f].as<int64_t>(); }
   P.n_reads = n; P.nf = nf;
-  P.names = static_cast<uint8_t *>(b.d_names); P.name_off = static_cast<int32_t *>(b.d_name_off); P.ref_len = static_cast<int64_t *>(b.d_len);
+  P.names = b.d_names.as<uint8_t>(); P.name_off = b.d_name_off.as<int32_t>(); P.ref_len = b.d_len.as<int64_t>();
   P.n_ref = b.n_ref; P.pos_bits = b.pos_bits;
-  P.rg = static_cast<uint8_t *>(b.d_rg); P.rg_len = (int)b.rg.size();
-  CK(grow(&b.d_csz, b.c_csz, 8 * (size_t)n));
-  CK(grow(&b.d_ckey, b.c_ckey, 8 * (size_t)n));
-  CK(grow(&b.d_coff, b.c_coff, 8 * ((size_t)n + 1)));
-  CK(grow(&b.d_code, b.c_code, (size_t)n));
-  CK(grow(&b.d_tmp, b.c_tmp, 8 * (size_t)mg_scan_tmp_elems(n)));
-  if (!b.d_bad) CK(cudaMalloc(&b.d_bad, 8));
-  CK(cudaMemsetAsync(b.d_bad, 0xFF, 8, st));
-  P.size = static_cast<int64_t *>(b.d_csz); P.key = static_cast<uint64_t *>(b.d_ckey); P.code = static_cast<uint8_t *>(b.d_code);
-  P.first_bad = static_cast<unsigned long long *>(b.d_bad);
-  const unsigned g = (unsigned)((n + 255) / 256);
-  k_bam_size<<<g, 256, 0, st>>>(P);
-  CK(cudaGetLastError());
-  mg_launch_scan_i64(P.size, static_cast<int64_t *>(b.d_coff), n, static_cast<int64_t *>(b.d_tmp), st);
+  P.rg = b.d_rg.as<uint8_t>(); P.rg_len = (int)b.rg.size();
+  MG_CK(b.ctx, b.d_csz.need(8 * (size_t)n));
+  MG_CK(b.ctx, b.d_ckey.need(8 * (size_t)n));
+  MG_CK(b.ctx, b.d_coff.need(8 * ((size_t)n + 1)));
+  MG_CK(b.ctx, b.d_code.need((size_t)n));
+  MG_CK(b.ctx, b.fq.tmp.need(8 * (size_t)mg_scan_tmp_elems(n)));
+  MG_CK(b.ctx, b.d_bad.need(8));
+  MG_CK(b.ctx, cudaMemsetAsync(b.d_bad.p, 0xFF, 8, st));
+  P.size = b.d_csz.as<int64_t>(); P.key = b.d_ckey.as<uint64_t>(); P.code = b.d_code.as<uint8_t>();
+  P.first_bad = b.d_bad.as<unsigned long long>();
+  k_bam_size<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(P);
+  MG_CK(b.ctx, cudaGetLastError());
+  mg_launch_scan_i64(P.size, b.d_coff.as<int64_t>(), n, b.fq.tmp.as<int64_t>(), st);
   unsigned long long first_bad = 0; int64_t total = 0;
-  CK(cudaMemcpyAsync(&first_bad, b.d_bad, 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(&total, static_cast<int64_t *>(b.d_coff) + n, 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
+  MG_CK(b.ctx, cudaMemcpyAsync(&first_bad, b.d_bad.p, 8, cudaMemcpyDeviceToHost, st));
+  MG_CK(b.ctx, cudaMemcpyAsync(&total, b.d_coff.as<int64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
+  MG_CK(b.ctx, cudaStreamSynchronize(st));
   if (first_bad != ~0ull) {
     uint8_t code = 0;
-    CK(cudaMemcpy(&code, static_cast<uint8_t *>(b.d_code) + first_bad, 1, cudaMemcpyDeviceToHost));
+    MG_CK(b.ctx, cudaMemcpy(&code, b.d_code.as<uint8_t>() + first_bad, 1, cudaMemcpyDeviceToHost));
     if (bad_index) *bad_index = (int64_t)first_bad;
     if (bad_code) *bad_code = code;
     return bam_fail(b, MG_EVALUE, "a FASTQ record cannot be written as a BAM record");
@@ -686,7 +636,7 @@ int mg_bam_add(mg_bam *h, const uint8_t *in1, int64_t len1, const uint8_t *in2, 
   int64_t k = n_tpl, bytes = total;
   if (!fits(n, total)) {
     std::vector<int64_t> off((size_t)n + 1);
-    CK(cudaMemcpy(off.data(), b.d_coff, 8 * off.size(), cudaMemcpyDeviceToHost));
+    MG_CK(b.ctx, cudaMemcpy(off.data(), b.d_coff.p, 8 * off.size(), cudaMemcpyDeviceToHost));
     int64_t lo = 0, hi = n_tpl;              // largest k with fits(k templates)
     while (lo < hi) { const int64_t m = (lo + hi + 1) / 2; if (fits(m * nf, off[(size_t)(m * nf)])) lo = m; else hi = m - 1; }
     if (lo == 0) {
@@ -699,18 +649,18 @@ int mg_bam_add(mg_bam *h, const uint8_t *in1, int64_t len1, const uint8_t *in2, 
     k = lo; bytes = off[(size_t)(k * nf)];
   }
   const int64_t nk = k * nf;
-  CK(grow_keep(&b.d_rec, b.c_rec, (size_t)(b.run_rec + bytes) + 16, (size_t)b.run_rec, st));
-  CK(grow_keep(&b.d_key, b.c_key, 8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
-  CK(grow_keep(&b.d_size, b.c_size, 8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
-  CK(grow_keep(&b.d_roff, b.c_roff, 8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
+  MG_CK(b.ctx, b.d_rec.need_keep((size_t)(b.run_rec + bytes) + 16, (size_t)b.run_rec, st));
+  MG_CK(b.ctx, b.d_key.need_keep(8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
+  MG_CK(b.ctx, b.d_size.need_keep(8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
+  MG_CK(b.ctx, b.d_roff.need_keep(8 * (size_t)(b.run_n + nk), 8 * (size_t)b.run_n, st));
   P.n_reads = nk;
-  P.off = static_cast<int64_t *>(b.d_coff); P.run_rec = b.run_rec; P.run_n = b.run_n; P.rec = static_cast<uint8_t *>(b.d_rec);
-  P.run_key = static_cast<uint64_t *>(b.d_key); P.run_size = static_cast<int64_t *>(b.d_size); P.run_off = static_cast<int64_t *>(b.d_roff);
+  P.off = b.d_coff.as<int64_t>(); P.run_rec = b.run_rec; P.run_n = b.run_n; P.rec = b.d_rec.as<uint8_t>();
+  P.run_key = b.d_key.as<uint64_t>(); P.run_size = b.d_size.as<int64_t>(); P.run_off = b.d_roff.as<int64_t>();
   k_bam_encode<<<(unsigned)((nk + 255) / 256), 256, 0, st>>>(P);
-  CK(cudaGetLastError());
+  MG_CK(b.ctx, cudaGetLastError());
   int64_t last[2] = {0, 0};
-  for (int f = 0; f < nf; f++) CK(cudaMemcpyAsync(&last[f], P.nl[f] + (4 * k - 1), 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
+  MG_CK(b.ctx, mg_fastq_ends(b.fq, k, last, st));
+  MG_CK(b.ctx, cudaStreamSynchronize(st));
   b.run_n += nk; b.run_rec += bytes;
   if (n_templates) *n_templates = k;
   if (consumed1) *consumed1 = last[0] + 1;
@@ -720,15 +670,13 @@ int mg_bam_add(mg_bam *h, const uint8_t *in1, int64_t len1, const uint8_t *in2, 
 }
 
 void mg_bam_abort(mg_bam *h) {
-  if (!h) return;
-  bam_free(h->b);
-  delete h;
+  if (h) bam_delete(h);
 }
 
 int mg_bam_close(mg_bam *h, int64_t *n_records, int64_t *n_runs, double *times) {
   if (!h) return MG_EINVAL;
   Bam &b = h->b;
-  cudaSetDevice(mg_internal_device(b.ctx));
+  DeviceGuard g(mg_internal_device(b.ctx));
   MgBamWriter w;
   int rc = MG_OK;
   if (!w.open(b.bam.c_str(), b.bai.empty() ? nullptr : b.bai.c_str(), b.header, b.n_ref, b.level, b.threads)) rc = bam_fail(b, MG_EVALUE, w.err);
@@ -737,7 +685,7 @@ int mg_bam_close(mg_bam *h, int64_t *n_records, int64_t *n_runs, double *times) 
     if (b.run_n) {
       rc = sort_run(b);
       b.t_dev += now_ms() - t;
-      if (!rc && stream_out(b, static_cast<uint8_t *>(b.d_out), b.run_rec, [&](const uint8_t *p, int64_t n) { return w.records(p, n); }))
+      if (!rc && stream_out(b, b.d_out.as<const uint8_t>(), b.run_rec, [&](const uint8_t *p, int64_t n) { return w.records(p, n); }))
         rc = bam_fail(b, MG_EVALUE, "cannot write " + b.bam + ": " + w.err);
       b.n_runs = 1;
     }
@@ -755,8 +703,7 @@ int mg_bam_close(mg_bam *h, int64_t *n_records, int64_t *n_runs, double *times) 
   if (n_records) *n_records = n;
   if (n_runs) *n_runs = b.n_runs;
   if (times) { times[0] = b.t_dev; times[1] = b.t_d2h; times[2] = b.t_out; }
-  bam_free(b);
-  delete h;
+  bam_delete(h);
   return rc;
 }
 

@@ -165,31 +165,14 @@ __global__ void __launch_bounds__(256) k_roundtrip_check(ChkParams P) {
 struct Checker {
   mg_ctx *ctx;
   std::vector<ChkCopy> copies;
-  std::vector<void *> owned;                       // device blocks (ASCII views) to free
-  std::map<int64_t, const uint8_t *> ref_view;     // region id -> ASCII reference
-  void *d_copies = nullptr; bool dirty = true;
-  void *d_in[2] = {nullptr, nullptr}, *d_nl[2] = {nullptr, nullptr}, *d_cnt = nullptr, *d_tmp = nullptr, *d_code = nullptr, *d_bad = nullptr;
-  size_t c_in[2] = {0, 0}, c_nl[2] = {0, 0}, c_cnt = 0, c_tmp = 0, c_code = 0;
+  std::vector<DevBuf> owned;                       // ASCII views (moving a DevBuf leaves its device block in place)
+  std::map<int64_t, const uint8_t *> ref_view;     // region id -> ASCII reference, inside `owned`
+  DevBuf d_copies; bool dirty = true;
+  MgFastqChunk fq;
+  DevBuf d_code, d_bad;
 };
 
-cudaError_t grow(void **p, size_t &cap, size_t bytes) {
-  if (bytes <= cap) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr; cap = 0;
-  const cudaError_t e = cudaMalloc(p, bytes + bytes / 8 + 256);
-  if (e == cudaSuccess) cap = bytes + bytes / 8 + 256;
-  return e;
-}
-
 }  // namespace
-
-// accessors implemented in mg_api.cu (the context's internals stay there)
-int mg_internal_copy_view(mg_ctx *ctx, int64_t copy_id, int64_t *region_id, const MgNode **nodes, int *n_nodes, const uint32_t **hap, uint32_t *hap_len,
-                          const MgExc **exc, int *n_exc, int64_t *start1);
-int mg_internal_region_view(mg_ctx *ctx, int64_t region_id, const uint32_t **ref, int64_t *len, const MgExc **exc, int *n_exc);
-cudaStream_t mg_internal_stream(mg_ctx *ctx);
-int mg_internal_device(mg_ctx *ctx);
-int mg_internal_fail(mg_ctx *ctx, int code, const char *msg);
 
 extern "C" {
 
@@ -205,29 +188,31 @@ int mg_check_open(mg_ctx *ctx, mg_checker **out) {
 
 void mg_check_close(mg_checker *k) {
   if (!k) return;
-  cudaSetDevice(mg_internal_device(k->c.ctx));
+  DeviceGuard g(mg_internal_device(k->c.ctx));
   cudaStreamSynchronize(mg_internal_stream(k->c.ctx));
-  for (void *p : k->c.owned) cudaFree(p);
-  for (void *p : {k->c.d_copies, k->c.d_in[0], k->c.d_in[1], k->c.d_nl[0], k->c.d_nl[1], k->c.d_cnt, k->c.d_tmp, k->c.d_code, k->c.d_bad}) if (p) cudaFree(p);
   delete k;
 }
 
-static int expand(mg_ctx *ctx, const uint32_t *packed, int64_t len, const MgExc *exc, int n_exc, uint8_t **out, std::vector<void *> &owned) {
+static int expand(mg_ctx *ctx, const uint32_t *packed, int64_t len, const MgExc *exc, int n_exc, uint8_t **out, std::vector<DevBuf> &owned) {
   cudaStream_t st = mg_internal_stream(ctx);
-  if (cudaMalloc((void **)out, (size_t)std::max<int64_t>(len, 1)) != cudaSuccess) return mg_internal_fail(ctx, MG_ECUDA, "out of device memory for the checker's text views");
-  owned.push_back(*out);
+  DevBuf v;
+  v.cap = (size_t)std::max<int64_t>(len, 1);      // exact: the views of a genome are large
+  if (cudaMalloc(&v.p, v.cap) != cudaSuccess) return mg_internal_fail(ctx, MG_ECUDA, "out of device memory for the checker's text views");
+  *out = v.as<uint8_t>();
+  owned.push_back(std::move(v));
   if (len > 0) {
     const int64_t words = (len + 15) / 16;
     k_expand_ascii<<<(unsigned)((words + 255) / 256), 256, 0, st>>>(packed, len, *out);
     if (n_exc) k_patch_exc<<<(unsigned)(((len + 255) / 256 + 255) / 256), 256, 0, st>>>(exc, n_exc, len, *out);
   }
-  return cudaGetLastError() == cudaSuccess ? MG_OK : mg_internal_fail(ctx, MG_ECUDA, "checker: expansion kernels failed");
+  MG_CK(ctx, cudaGetLastError());
+  return MG_OK;
 }
 
 int mg_check_add_copy(mg_checker *k, int64_t copy_id, const char *chrom, int32_t cpy) {
   if (!k || !chrom || strlen(chrom) >= sizeof(((ChkCopy *)0)->chrom)) return MG_EINVAL;
   mg_ctx *ctx = k->c.ctx;
-  cudaSetDevice(mg_internal_device(ctx));
+  DeviceGuard g(mg_internal_device(ctx));
   int64_t rid, start1, rlen; const MgNode *nodes; int n_nodes, n_exc, rn_exc; const uint32_t *hap, *ref; uint32_t hap_len; const MgExc *exc, *rexc;
   int rc = mg_internal_copy_view(ctx, copy_id, &rid, &nodes, &n_nodes, &hap, &hap_len, &exc, &n_exc, &start1);
   if (rc) return rc;
@@ -258,65 +243,46 @@ int mg_check_fastq(mg_checker *k, const uint8_t *in1, int64_t len1, const uint8_
   if (!k || !in1 || len1 < 0 || (in2 && len2 < 0)) return MG_EINVAL;
   Checker &c = k->c;
   mg_ctx *ctx = c.ctx;
-  cudaSetDevice(mg_internal_device(ctx));
+  DeviceGuard g(mg_internal_device(ctx));
   cudaStream_t st = mg_internal_stream(ctx);
-#define CK(call) do { if ((call) != cudaSuccess) return mg_internal_fail(ctx, MG_ECUDA, #call); } while (0)
   if (c.dirty) {
-    if (c.d_copies) cudaFree(c.d_copies);
-    c.d_copies = nullptr;
-    CK(cudaMalloc(&c.d_copies, sizeof(ChkCopy) * std::max<size_t>(1, c.copies.size())));
-    CK(cudaMemcpyAsync(c.d_copies, c.copies.data(), sizeof(ChkCopy) * c.copies.size(), cudaMemcpyHostToDevice, st));
+    MG_CK(ctx, c.d_copies.need(sizeof(ChkCopy) * std::max<size_t>(1, c.copies.size())));
+    MG_CK(ctx, cudaMemcpyAsync(c.d_copies.p, c.copies.data(), sizeof(ChkCopy) * c.copies.size(), cudaMemcpyHostToDevice, st));
     c.dirty = false;
   }
   const int nf = in2 ? 2 : 1;
   const uint8_t *in[2] = {in1, in2}; const int64_t len[2] = {len1, len2};
-  int64_t n_lines[2] = {0, 0};
-  ChkParams P; memset(&P, 0, sizeof P);
-  for (int f = 0; f < nf; f++) {
-    CK(grow(&c.d_in[f], c.c_in[f], (size_t)len[f] + 16));
-    if (len[f]) CK(cudaMemcpyAsync(c.d_in[f], in[f], (size_t)len[f], cudaMemcpyHostToDevice, st));
-    const int64_t chunks = mg_nl_chunks(len[f]);
-    CK(grow(&c.d_cnt, c.c_cnt, 8 * (size_t)(2 * chunks + 4)));
-    CK(grow(&c.d_tmp, c.c_tmp, 8 * (size_t)mg_scan_tmp_elems(std::max<int64_t>(chunks, 1))));
-    int64_t *cnt = static_cast<int64_t *>(c.d_cnt), *off = cnt + chunks + 1;
-    mg_launch_nl_count(static_cast<uint8_t *>(c.d_in[f]), len[f], cnt, st);
-    mg_launch_scan_i64(cnt, off, chunks, static_cast<int64_t *>(c.d_tmp), st);
-    CK(cudaMemcpyAsync(&n_lines[f], off + chunks, 8, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    CK(grow(&c.d_nl[f], c.c_nl[f], 8 * (size_t)(n_lines[f] + 1)));
-    mg_launch_nl_write(static_cast<uint8_t *>(c.d_in[f]), len[f], off, static_cast<int64_t *>(c.d_nl[f]), st);
-    P.fq[f] = static_cast<uint8_t *>(c.d_in[f]); P.nl[f] = static_cast<int64_t *>(c.d_nl[f]);
-  }
-  int64_t n_rec = n_lines[0] / 4;
-  if (nf == 2) n_rec = std::min(n_rec, n_lines[1] / 4);
+  MG_CK(ctx, mg_fastq_load(c.fq, in, len, nf, st));
+  const int64_t n_rec = c.fq.n_tpl;
   if (n_records) *n_records = n_rec;
   if (n_bad) *n_bad = 0;
   if (consumed1) *consumed1 = 0;
   if (consumed2) *consumed2 = 0;
   if (n_rec == 0) return MG_OK;
   int64_t last[2] = {0, 0};
-  for (int f = 0; f < nf; f++) CK(cudaMemcpyAsync(&last[f], P.nl[f] + (4 * n_rec - 1), 8, cudaMemcpyDeviceToHost, st));
+  MG_CK(ctx, mg_fastq_ends(c.fq, n_rec, last, st));
+  ChkParams P; memset(&P, 0, sizeof P);
+  for (int f = 0; f < nf; f++) { P.fq[f] = c.fq.in[f].as<uint8_t>(); P.nl[f] = c.fq.nl[f].as<int64_t>(); }
   P.n_rec = n_rec; P.n_files = nf;
-  P.copies = static_cast<const ChkCopy *>(c.d_copies); P.n_copies = (int)c.copies.size();
-  CK(grow(&c.d_code, c.c_code, (size_t)(n_rec * nf)));
-  if (!c.d_bad) CK(cudaMalloc(&c.d_bad, 8));
-  CK(cudaMemsetAsync(c.d_bad, 0, 8, st));
-  P.code = static_cast<uint8_t *>(c.d_code); P.n_bad = static_cast<unsigned long long *>(c.d_bad);
+  P.copies = c.d_copies.as<const ChkCopy>(); P.n_copies = (int)c.copies.size();
+  MG_CK(ctx, c.d_code.need((size_t)(n_rec * nf)));
+  MG_CK(ctx, c.d_bad.need(8));
+  MG_CK(ctx, cudaMemsetAsync(c.d_bad.p, 0, 8, st));
+  P.code = c.d_code.as<uint8_t>(); P.n_bad = c.d_bad.as<unsigned long long>();
   k_roundtrip_check<<<(unsigned)((n_rec * nf + 255) / 256), 256, 0, st>>>(P);
-  CK(cudaGetLastError());
+  MG_CK(ctx, cudaGetLastError());
   unsigned long long bad = 0;
-  CK(cudaMemcpyAsync(&bad, c.d_bad, 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
+  MG_CK(ctx, cudaMemcpyAsync(&bad, c.d_bad.p, 8, cudaMemcpyDeviceToHost, st));
+  MG_CK(ctx, cudaStreamSynchronize(st));
   if (consumed1) *consumed1 = last[0] + 1;
   if (consumed2 && nf > 1) *consumed2 = last[1] + 1;
   if (n_bad) *n_bad = (int64_t)bad;
   if (bad && bad_index && bad_code && bad_cap > 0) {
     std::vector<uint8_t> codes((size_t)(n_rec * nf));
-    CK(cudaMemcpy(codes.data(), c.d_code, codes.size(), cudaMemcpyDeviceToHost));
+    MG_CK(ctx, cudaMemcpy(codes.data(), c.d_code.p, codes.size(), cudaMemcpyDeviceToHost));
     int w = 0;
     for (size_t i = 0; i < codes.size() && w < bad_cap; i++) if (codes[i]) { bad_index[w] = (int64_t)i; bad_code[w] = codes[i]; w++; }
   }
-#undef CK
   return MG_OK;
 }
 

@@ -1,8 +1,101 @@
-// Internal interface between the C-ABI host code (mg_api.cu) and the kernels (mg_kernels.cu).
+// Internal interface between the C-ABI host code (mg_api.cu, mg_check.cu, mg_bam.cu, mg_readmodel.cu) and the
+// kernels (mg_kernels.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <utility>
 #include "mg_core.cuh"
+
+struct mg_ctx;
+
+// accessors implemented in mg_api.cu (the context's internals stay there)
+cudaStream_t mg_internal_stream(mg_ctx *ctx);
+int mg_internal_device(mg_ctx *ctx);
+int mg_internal_fail(mg_ctx *ctx, int code, const char *msg);
+int mg_internal_cuda_fail(mg_ctx *ctx, cudaError_t e, const char *call, const char *file, int line);   // -> MG_ECUDA
+int mg_internal_copy_view(mg_ctx *ctx, int64_t copy_id, int64_t *region_id, const MgNode **nodes, int *n_nodes, const uint32_t **hap, uint32_t *hap_len,
+                          const MgExc **exc, int *n_exc, int64_t *start1);
+int mg_internal_region_view(mg_ctx *ctx, int64_t region_id, const uint32_t **ref, int64_t *len, const MgExc **exc, int *n_exc);
+
+// returns MG_ECUDA from the enclosing function when `call` fails; the context's error names the call, the CUDA
+// error and file:line
+#define MG_CK(ctx, call) do { const cudaError_t e_ = (call); if (e_ != cudaSuccess) return mg_internal_cuda_fail((ctx), e_, #call, __FILE__, __LINE__); } while (0)
+
+struct DeviceGuard {   // makes `dev` current for a scope, then restores the caller's device
+  int prev = -1;
+  explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
+  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+  DeviceGuard(const DeviceGuard &) = delete;
+  DeviceGuard &operator=(const DeviceGuard &) = delete;
+};
+
+struct DevBuf {  // grow-only device buffer; move-only, freed with its owner
+  void *p = nullptr;
+  size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf &) = delete;
+  DevBuf &operator=(const DevBuf &) = delete;
+  DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~DevBuf() { if (p) cudaFree(p); }
+  // at least `bytes`; the contents are not kept
+  cudaError_t need(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    if (p) { cudaFree(p); p = nullptr; cap = 0; }
+    size_t want = bytes + bytes / 8 + 256;
+    cudaError_t e = cudaMalloc(&p, want);
+    if (e == cudaSuccess) cap = want;
+    return e;
+  }
+  // at least `bytes`, keeping the first `keep`; grows by a quarter, since a buffer that grows this way (a
+  // god-aligner run) is copied on every growth.  The old block is freed once `st` has drained.
+  cudaError_t need_keep(size_t bytes, size_t keep, cudaStream_t st) {
+    if (bytes <= cap) return cudaSuccess;
+    void *q = nullptr;
+    const size_t want = bytes + bytes / 4 + 256;
+    cudaError_t e = cudaMalloc(&q, want);
+    if (e != cudaSuccess) return e;
+    if (keep) e = cudaMemcpyAsync(q, p, keep, cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (p) cudaFree(p);
+    p = q; cap = want;
+    return e;
+  }
+  template <class T> T *as() const { return reinterpret_cast<T *>(p); }
+};
+
+struct HostBuf {  // grow-only page-locked staging buffer; move-only
+  void *p = nullptr;
+  size_t cap = 0;
+  HostBuf() = default;
+  HostBuf(const HostBuf &) = delete;
+  HostBuf &operator=(const HostBuf &) = delete;
+  HostBuf(HostBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  HostBuf &operator=(HostBuf &&o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+  ~HostBuf() { if (p) cudaFreeHost(p); }
+  cudaError_t need(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    if (p) { cudaFreeHost(p); p = nullptr; cap = 0; }
+    size_t want = bytes + bytes / 4 + 4096;
+    cudaError_t e = cudaHostAlloc(&p, want, cudaHostAllocPortable);
+    if (e == cudaSuccess) cap = want;
+    return e;
+  }
+  template <class T> T *as() const { return reinterpret_cast<T *>(p); }
+};
+
+// The FASTQ ingest of corrupt-reads, check-reads and god-aligner: one or two FASTQ buffers on the device with
+// their newline index.  The caller handles (some of) the n_tpl complete templates and carries the rest of each
+// file into its next chunk.
+struct MgFastqChunk {
+  DevBuf in[2], nl[2], cnt, tmp;     // tmp: the newline scan's; a caller may reuse it for its own scans
+  int nf = 0;
+  int64_t n_tpl = 0;                 // complete templates present in every file
+};
+// per file: H2D, k_nl_count, scan, k_nl_write (5 launches); one sync per file to size the index
+cudaError_t mg_fastq_load(MgFastqChunk &q, const uint8_t *const in[2], const int64_t len[2], int nf, cudaStream_t st);
+// enqueues the D2H of the last byte offset of the first k templates of each file into last[] (the caller syncs)
+cudaError_t mg_fastq_ends(const MgFastqChunk &q, int64_t k, int64_t last[2], cudaStream_t st);
 
 #define MG_PLAN_TILE 256     // candidates per CTA tile of k_unit_plan
 #define MG_CTA 128           // threads per CTA of k_unit_emit (4 independent warps, 32 kept templates each)

@@ -20,10 +20,7 @@
 
 #include "../../include/mitty_b200.h"
 #include "mg_bgzf.h"
-
-cudaStream_t mg_internal_stream(mg_ctx *ctx);
-int mg_internal_device(mg_ctx *ctx);
-int mg_internal_fail(mg_ctx *ctx, int code, const char *msg);
+#include "mg_internal.h"
 
 namespace {
 
@@ -111,15 +108,6 @@ double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::
 void *pinned_alloc(size_t n) { void *p = nullptr; return cudaHostAlloc(&p, n, cudaHostAllocDefault) == cudaSuccess ? p : nullptr; }
 void pinned_release(void *p) { cudaFreeHost(p); }
 
-cudaError_t grow(void **p, size_t &cap, size_t bytes) {
-  if (bytes <= cap) return cudaSuccess;
-  if (*p) cudaFree(*p);
-  *p = nullptr; cap = 0;
-  const cudaError_t e = cudaMalloc(p, bytes + bytes / 8 + 256);
-  if (e == cudaSuccess) cap = bytes + bytes / 8 + 256;
-  return e;
-}
-
 }  // namespace
 
 extern "C" int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, int32_t max_tlen, int32_t min_mq, int64_t every, int32_t threads,
@@ -131,7 +119,7 @@ extern "C" int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, i
   const double t_start = now_ms();
   *bad_where = -1; *bad_code = 0;
   const int dev = mg_internal_device(ctx);
-  cudaSetDevice(dev);
+  DeviceGuard g(dev);
   int smem_max = 0, n_sm = 0;
   cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
@@ -146,87 +134,78 @@ extern "C" int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, i
   MgBamReader rd;
   if (!rd.open(path, threads, chunk_bytes, pinned_alloc, pinned_release)) return mg_internal_fail(ctx, MG_EVALUE, rd.err.c_str());
   const size_t n_bq = (size_t)2 * max_bp * RM_NQ, n_acc = n_bq + (size_t)max_bp + 1 + (size_t)max_tlen + RM_NCNT + 1;
-  void *d_acc = nullptr, *d_data[2] = {nullptr, nullptr}, *d_off[2] = {nullptr, nullptr};
-  size_t c_data[2] = {0, 0}, c_off[2] = {0, 0};
+  DevBuf d_acc, d_data[2], d_off[2];
+  HostBuf h_bad;                                     // per slot: the chunk's first_bad, read back
   cudaStream_t cs = nullptr, ks = nullptr;
   cudaEvent_t ev[2][5] = {};                         // per slot: H2D start / end, kernel start / end, first_bad read back
   bool pending[2] = {false, false}, device_bad = false;
-  unsigned long long *h_bad = static_cast<unsigned long long *>(pinned_alloc(2 * sizeof(unsigned long long)));
   double h2d_ms = 0, kernel_ms = 0;
   int64_t chunks = 0;
-  std::string msg;
-  int rc = MG_OK;
-  auto ck = [&](cudaError_t e, const char *what) {
-    if (e != cudaSuccess && rc == MG_OK) { rc = MG_ECUDA; msg = std::string("mg_readmodel_bam: ") + what + ": " + cudaGetErrorString(e); }
-    return rc == MG_OK;
-  };
+  unsigned long long first_bad = ~0ull, cnt[RM_NCNT] = {0};
   // waits for the chunk in flight in `s`, adds its copy and kernel times and notes a malformed record found so far
-  auto settle = [&](int s) {
-    if (!pending[s]) return;
+  auto settle = [&](int s) -> int {
+    if (!pending[s]) return MG_OK;
     pending[s] = false;
-    if (!ck(cudaEventSynchronize(ev[s][4]), "kernel")) return;
-    if (h_bad[s] != ~0ull) device_bad = true;
+    MG_CK(ctx, cudaEventSynchronize(ev[s][4]));
+    if (h_bad.as<unsigned long long>()[s] != ~0ull) device_bad = true;
     float a = 0, b = 0;
     cudaEventElapsedTime(&a, ev[s][0], ev[s][1]); cudaEventElapsedTime(&b, ev[s][2], ev[s][3]);
     h2d_ms += a; kernel_ms += b;
+    return MG_OK;
   };
-  ck(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking), "stream");
-  ck(cudaStreamCreateWithFlags(&ks, cudaStreamNonBlocking), "stream");
-  if (!h_bad) ck(cudaErrorMemoryAllocation, "out of page-locked memory");
-  for (int s = 0; s < 2; s++) for (int j = 0; j < 5; j++) ck(cudaEventCreate(&ev[s][j]), "event");
-  ck(cudaMalloc(&d_acc, 8 * n_acc), "out of device memory");
-  unsigned long long *acc = static_cast<unsigned long long *>(d_acc);
-  if (rc == MG_OK) {
-    ck(cudaMemsetAsync(d_acc, 0, 8 * (n_acc - 1), ks), "memset");
-    ck(cudaMemsetAsync(acc + n_acc - 1, 0xFF, 8, ks), "memset");
-  }
-  RmParams P;
-  memset(&P, 0, sizeof P);
-  P.every = (uint32_t)every; P.min_mq = min_mq; P.max_bp = max_bp; P.max_tlen = max_tlen; P.stripe = stripe;
-  P.bq = acc; P.len_hist = acc + n_bq; P.tlen = P.len_hist + max_bp + 1; P.cnt = P.tlen + max_tlen; P.first_bad = P.cnt + RM_NCNT;
-  MgBamChunk c;
-  for (int64_t k = 0; rc == MG_OK; k++) {
-    const int s = (int)(k & 1);
-    settle(s);                                         // the slot's buffers are free again
-    if (rc != MG_OK || device_bad || !rd.next(s, c)) break;   // a malformed record ends the input: it is reported, nothing later is
-    if (!ck(grow(&d_data[s], c_data[s], (size_t)c.bytes), "out of device memory") || !ck(grow(&d_off[s], c_off[s], 4 * (size_t)c.n), "out of device memory")) break;
-    ck(cudaEventRecord(ev[s][0], cs), "event");
-    ck(cudaMemcpyAsync(d_data[s], c.data, (size_t)c.bytes, cudaMemcpyHostToDevice, cs), "copy");
-    ck(cudaMemcpyAsync(d_off[s], c.off, 4 * (size_t)c.n, cudaMemcpyHostToDevice, cs), "copy");
-    ck(cudaEventRecord(ev[s][1], cs), "event");
-    ck(cudaStreamWaitEvent(ks, ev[s][1], 0), "event");
-    P.data = static_cast<uint8_t *>(d_data[s]); P.off = static_cast<uint32_t *>(d_off[s]); P.n = c.n; P.first = (uint64_t)c.first;
-    const dim3 grid((unsigned)std::min<int64_t>(n_sm, (c.n + 31) / 32), (unsigned)n_stripes);
-    ck(cudaEventRecord(ev[s][2], ks), "event");
-    k_readmodel<<<grid, RM_THREADS, smem, ks>>>(P);
-    ck(cudaGetLastError(), "launch");
-    ck(cudaEventRecord(ev[s][3], ks), "event");
-    ck(cudaMemcpyAsync(&h_bad[s], P.first_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ks), "copy");
-    ck(cudaEventRecord(ev[s][4], ks), "event");
-    pending[s] = true;
-    chunks++;
-  }
-  settle(0); settle(1);
-  unsigned long long first_bad = ~0ull, cnt[RM_NCNT] = {0};
-  if (rc == MG_OK) {
-    std::vector<unsigned long long> h(n_acc);
-    if (ck(cudaMemcpyAsync(h.data(), d_acc, 8 * n_acc, cudaMemcpyDeviceToHost, ks), "copy") && ck(cudaStreamSynchronize(ks), "copy")) {
-      memcpy(bq_mat, h.data(), 8 * n_bq);
-      memcpy(len_hist, h.data() + n_bq, 8 * ((size_t)max_bp + 1));
-      memcpy(tlen, h.data() + n_bq + max_bp + 1, 8 * (size_t)max_tlen);
-      memcpy(cnt, h.data() + n_bq + max_bp + 1 + max_tlen, sizeof cnt);
-      first_bad = h[n_acc - 1];
+  // every chunk through the kernel; returns at the first CUDA failure, the streams and events are released below
+  auto run = [&]() -> int {
+    MG_CK(ctx, cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+    MG_CK(ctx, cudaStreamCreateWithFlags(&ks, cudaStreamNonBlocking));
+    MG_CK(ctx, h_bad.need(2 * sizeof(unsigned long long)));
+    for (int s = 0; s < 2; s++) for (int j = 0; j < 5; j++) MG_CK(ctx, cudaEventCreate(&ev[s][j]));
+    MG_CK(ctx, d_acc.need(8 * n_acc));
+    unsigned long long *acc = d_acc.as<unsigned long long>();
+    MG_CK(ctx, cudaMemsetAsync(acc, 0, 8 * (n_acc - 1), ks));
+    MG_CK(ctx, cudaMemsetAsync(acc + n_acc - 1, 0xFF, 8, ks));
+    RmParams P;
+    memset(&P, 0, sizeof P);
+    P.every = (uint32_t)every; P.min_mq = min_mq; P.max_bp = max_bp; P.max_tlen = max_tlen; P.stripe = stripe;
+    P.bq = acc; P.len_hist = acc + n_bq; P.tlen = P.len_hist + max_bp + 1; P.cnt = P.tlen + max_tlen; P.first_bad = P.cnt + RM_NCNT;
+    MgBamChunk c;
+    for (int64_t k = 0;; k++) {
+      const int s = (int)(k & 1);
+      const int rc = settle(s);                        // the slot's buffers are free again
+      if (rc) return rc;
+      if (device_bad || !rd.next(s, c)) break;         // a malformed record ends the input: it is reported, nothing later is
+      MG_CK(ctx, d_data[s].need((size_t)c.bytes));
+      MG_CK(ctx, d_off[s].need(4 * (size_t)c.n));
+      MG_CK(ctx, cudaEventRecord(ev[s][0], cs));
+      MG_CK(ctx, cudaMemcpyAsync(d_data[s].p, c.data, (size_t)c.bytes, cudaMemcpyHostToDevice, cs));
+      MG_CK(ctx, cudaMemcpyAsync(d_off[s].p, c.off, 4 * (size_t)c.n, cudaMemcpyHostToDevice, cs));
+      MG_CK(ctx, cudaEventRecord(ev[s][1], cs));
+      MG_CK(ctx, cudaStreamWaitEvent(ks, ev[s][1], 0));
+      P.data = d_data[s].as<uint8_t>(); P.off = d_off[s].as<uint32_t>(); P.n = c.n; P.first = (uint64_t)c.first;
+      const dim3 grid((unsigned)std::min<int64_t>(n_sm, (c.n + 31) / 32), (unsigned)n_stripes);
+      MG_CK(ctx, cudaEventRecord(ev[s][2], ks));
+      k_readmodel<<<grid, RM_THREADS, smem, ks>>>(P);
+      MG_CK(ctx, cudaGetLastError());
+      MG_CK(ctx, cudaEventRecord(ev[s][3], ks));
+      MG_CK(ctx, cudaMemcpyAsync(h_bad.as<unsigned long long>() + s, P.first_bad, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ks));
+      MG_CK(ctx, cudaEventRecord(ev[s][4], ks));
+      pending[s] = true;
+      chunks++;
     }
-  }
+    for (int s = 0; s < 2; s++) { const int rc = settle(s); if (rc) return rc; }
+    std::vector<unsigned long long> h(n_acc);
+    MG_CK(ctx, cudaMemcpyAsync(h.data(), acc, 8 * n_acc, cudaMemcpyDeviceToHost, ks));
+    MG_CK(ctx, cudaStreamSynchronize(ks));
+    memcpy(bq_mat, h.data(), 8 * n_bq);
+    memcpy(len_hist, h.data() + n_bq, 8 * ((size_t)max_bp + 1));
+    memcpy(tlen, h.data() + n_bq + max_bp + 1, 8 * (size_t)max_tlen);
+    memcpy(cnt, h.data() + n_bq + max_bp + 1 + max_tlen, sizeof cnt);
+    first_bad = h[n_acc - 1];
+    return MG_OK;
+  };
+  const int rc = run();
   if (ks) cudaStreamSynchronize(ks);
   if (cs) cudaStreamSynchronize(cs);
-  for (int s = 0; s < 2; s++) {
-    if (d_data[s]) cudaFree(d_data[s]);
-    if (d_off[s]) cudaFree(d_off[s]);
-    for (int j = 0; j < 5; j++) if (ev[s][j]) cudaEventDestroy(ev[s][j]);
-  }
-  if (d_acc) cudaFree(d_acc);
-  if (h_bad) pinned_release(h_bad);
+  for (int s = 0; s < 2; s++) for (int j = 0; j < 5; j++) if (ev[s][j]) cudaEventDestroy(ev[s][j]);
   if (cs) cudaStreamDestroy(cs);
   if (ks) cudaStreamDestroy(ks);
 
@@ -236,7 +215,7 @@ extern "C" int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, i
   memcpy(counts, out, sizeof out);
   times[0] = rd.read_ms; times[1] = rd.inflate_ms; times[2] = rd.walk_ms; times[3] = h2d_ms; times[4] = kernel_ms; times[5] = now_ms() - t_start;
   if (thread_ms) for (size_t t = 0; t < rd.thread_ms.size(); t++) thread_ms[t] = rd.thread_ms[t];
-  if (rc != MG_OK) return mg_internal_fail(ctx, rc, msg.c_str());
+  if (rc != MG_OK) return rc;
   if (first_bad != ~0ull) { *bad_where = (int64_t)(first_bad >> 8); *bad_code = (int32_t)(first_bad & 0xFF); }
   else if (rd.code) { *bad_where = rd.where; *bad_code = rd.code; }
   else if (!rd.err.empty()) return mg_internal_fail(ctx, MG_EVALUE, rd.err.c_str());

@@ -19,6 +19,17 @@ def _ptr(a):
   return None if a is None else C.c_void_p(a.ctypes.data)
 
 
+def _u8(buf):
+  return buf if buf is None or isinstance(buf, np.ndarray) else np.frombuffer(buf, dtype=np.uint8)
+
+
+def _fastq_args(fq1, fq2):
+  """FASTQ buffers 1 and 2 (bytes or uint8 arrays; fq2 may be None) as the C ABI's (pointer, length) pairs; an
+  empty buffer 1 is passed as a non-null address, which the library does not read."""
+  a1, a2 = _u8(fq1), _u8(fq2)
+  return _ptr(a1 if a1.size else np.zeros(1, np.uint8)), a1.size, _ptr(a2), 0 if a2 is None else a2.size
+
+
 class CopyHandle(object):
   __slots__ = ('id', 'p_min', 'p_max', 'n_nodes', 'region')
 
@@ -313,8 +324,7 @@ class Engine(object):
     partial=True (chunked streaming): only the complete templates present in both buffers are
     processed and the consumed input byte counts are returned as a 4th / 5th value; first_template =
     templates processed by earlier chunks.  out: optional (pinned) output buffer pair."""
-    a1 = np.frombuffer(fq1, dtype=np.uint8) if not isinstance(fq1, np.ndarray) else fq1
-    a2 = None if fq2 is None else (np.frombuffer(fq2, dtype=np.uint8) if not isinstance(fq2, np.ndarray) else fq2)
+    a1, a2 = _u8(fq1), _u8(fq2)
     if not partial:
       if a1.size and a1[-1] != 10:
         a1 = np.concatenate([a1, np.array([10], dtype=np.uint8)])
@@ -333,9 +343,7 @@ class Engine(object):
       bq, call, base, off = draws
       bq = np.ascontiguousarray(bq, dtype=np.float64); call = np.ascontiguousarray(call, dtype=np.float64)
       base = np.ascontiguousarray(base, dtype=np.uint8); off = np.ascontiguousarray(off, dtype=np.int64)
-    self._check(self._L.mg_corrupt_fastq(self._h, _ptr(a1) if a1.size else _ptr(np.zeros(1, np.uint8)), a1.size,
-                                         _ptr(a2) if a2 is not None else None, a2.size if a2 is not None else 0,
-                                         int(mode), int(seed) & 0xFFFFFFFF, _ptr(bq), _ptr(call), _ptr(base), _ptr(off),
+    self._check(self._L.mg_corrupt_fastq(self._h, *_fastq_args(a1, a2), int(mode), int(seed) & 0xFFFFFFFF, _ptr(bq), _ptr(call), _ptr(base), _ptr(off),
                                          _ptr(o1), _ptr(o2) if a2 is not None else None, cap, C.byref(l1), C.byref(l2), C.byref(nt),
                                          int(first_template), C.byref(c1), C.byref(c2)))
     res = (o1[:l1.value], (o2[:l2.value] if a2 is not None else None), nt.value)
@@ -373,13 +381,10 @@ class Checker(object):
 
   def check(self, fq1, fq2=None, max_report=64):
     """-> (templates checked, bad reads, [(file, record, code)], consumed bytes of fq1, of fq2)."""
-    a1 = np.frombuffer(fq1, dtype=np.uint8) if not isinstance(fq1, np.ndarray) else fq1
-    a2 = None if fq2 is None else (np.frombuffer(fq2, dtype=np.uint8) if not isinstance(fq2, np.ndarray) else fq2)
     n, bad, c1, c2 = C.c_int64(0), C.c_int64(0), C.c_int64(0), C.c_int64(0)
     idx, code = np.zeros(max(1, max_report), dtype=np.int64), np.zeros(max(1, max_report), dtype=np.int32)
-    self.engine._check(self._L.mg_check_fastq(self._h, _ptr(a1) if a1.size else _ptr(np.zeros(1, np.uint8)), a1.size,
-                                              _ptr(a2) if a2 is not None else None, a2.size if a2 is not None else 0,
-                                              C.byref(n), C.byref(bad), _ptr(idx), _ptr(code), int(max_report), C.byref(c1), C.byref(c2)))
+    self.engine._check(self._L.mg_check_fastq(self._h, *_fastq_args(fq1, fq2), C.byref(n), C.byref(bad), _ptr(idx), _ptr(code), int(max_report),
+                                              C.byref(c1), C.byref(c2)))
     k = min(bad.value, max_report)
     rep = [(int(i // max(1, n.value)), int(i % max(1, n.value)), int(c)) for i, c in zip(idx[:k], code[:k])]
     return n.value, bad.value, rep, c1.value, c2.value
@@ -414,8 +419,7 @@ class BamWriter(object):
     """-> (templates encoded, consumed bytes of fq1, of fq2).  A read the BAM cannot hold raises ValueError
     with (file, record in this chunk, reason) as ``args[1:]``."""
     n, c1, c2, bi, bc = C.c_int64(0), C.c_int64(0), C.c_int64(0), C.c_int64(-1), C.c_int32(0)
-    rc = self._L.mg_bam_add(self._h, _ptr(fq1) if fq1.size else _ptr(np.zeros(1, np.uint8)), fq1.size, _ptr(fq2) if fq2 is not None else None,
-                            fq2.size if fq2 is not None else 0, C.byref(n), C.byref(c1), C.byref(c2), C.byref(bi), C.byref(bc))
+    rc = self._L.mg_bam_add(self._h, *_fastq_args(fq1, fq2), C.byref(n), C.byref(c1), C.byref(c2), C.byref(bi), C.byref(bc))
     if rc == _lib.MG_EVALUE and bi.value >= 0:
       nf = 2 if fq2 is not None else 1
       raise ValueError('not writable as a BAM record', bi.value % nf, bi.value // nf, BAM_CODES.get(bc.value, str(bc.value)))

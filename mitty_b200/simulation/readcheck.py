@@ -4,13 +4,13 @@ Mitty's ``god-aligner`` writes each read into a BAM at the POS / CIGAR its qname
 (mitty/benchmarking/god_aligner.py:141-183 over ``parse_qname``, readgenerate.py:259-291).  This
 command proves that those qnames are true for a FASTQ pair of PERFECT reads: every read is re-derived
 on the GPU from (chrom, copy, strand, POS, CIGAR) + FASTA + VCF + BED (``k_roundtrip_check``) and
-compared with the bases in the file.  The files are streamed in chunks like corrupt-reads' inputs."""
+compared with the bases in the file.  The files are read in chunks (``lib.fastqio``)."""
 import logging
 import time
 
 import mitty_b200.lib.vcfio as vio
 from mitty_b200.engine import CHECK_CODES, Checker, Engine
-from mitty_b200.simulation.readcorrupt import _Stream
+from mitty_b200.lib.fastqio import FastqStream, for_each_chunk, qname_of
 
 logger = logging.getLogger(__name__)
 
@@ -32,38 +32,21 @@ def check_fastq(fasta_fname, vcf_fname, sample_name, bed_fname, fastq1, fastq2=N
       for cpy, vl in enumerate(r['v']):
         vl, _ = _without_end_crossing_deletions(vl, region, drop_end_deletions)
         chk.add_copy(engine.build_copy(rid, vl), region[0], cpy)
-    paired = fastq2 is not None
-    ins = [_Stream(fastq1, engine.pinned(chunk_bytes))] + ([_Stream(fastq2, engine.pinned(chunk_bytes))] if paired else [])
+    ins = [FastqStream(f, engine.pinned(chunk_bytes)) for f in (fastq1, fastq2) if f is not None]
     templates = bad = 0
     examples = []
-    while True:
-      for st in ins:
-        st.refill()
-      a1 = ins[0].buf[:ins[0].fill]
-      a2 = ins[1].buf[:ins[1].fill] if paired else None
-      if a1.size == 0 or (paired and a2.size == 0):
-        break
+
+    def step(a1, a2):
+      nonlocal templates, bad
       n, nb, rep, c1, c2 = chk.check(a1, a2, max_report=max(0, max_report - len(examples)) or 1)
-      if n == 0:
-        if all(st.eof for st in ins):
-          break
-        raise ValueError('a FASTQ record is larger than the chunk size ({} bytes)'.format(chunk_bytes))
       for f, rec, code in rep:
         if len(examples) < max_report:
-          buf = a1 if f == 0 else a2
-          # the record's qname: the (4 * rec)-th line of this chunk
-          pos = 0
-          for _ in range(4 * rec):
-            pos = int(buf[pos:].tobytes().index(b'\n')) + pos + 1
-          end = int(buf[pos:].tobytes().index(b'\n')) + pos
-          examples.append((f + 1, templates + rec, CHECK_CODES.get(code, str(code)), buf[pos:end].tobytes().decode(errors='replace')))
+          examples.append((f + 1, templates + rec, CHECK_CODES.get(code, str(code)), qname_of(a1 if f == 0 else a2, rec)))
       templates += n; bad += nb
-      ins[0].consume(c1)
-      if paired:
-        ins[1].consume(c2)
-    for st in ins:
-      st.close()
-    return {'templates': templates, 'reads': templates * (2 if paired else 1), 'bad': bad, 'examples': examples, 'seconds': time.time() - t0}
+      return n, c1, c2
+
+    for_each_chunk(ins, step)
+    return {'templates': templates, 'reads': templates * len(ins), 'bad': bad, 'examples': examples, 'seconds': time.time() - t0}
   finally:
     if chk is not None:
       chk.close()

@@ -23,26 +23,11 @@ import time
 import numpy as np
 
 from mitty_b200.engine import MODE_DET, MODE_PHILOX, SEED_MAX, Engine
+from mitty_b200.lib.fastqio import FastqStream, for_each_chunk
 
 logger = logging.getLogger(__name__)
 
-
-def open_fastq(fname):
-  """One open() per input: the inputs may be FIFOs or /dev/fd/N process substitutions
-  (examples/reads/run.sh:13-16 of the reference feeds corrupt-reads from FIFOs), where a second
-  open() blocks for ever or loses the bytes already read.  Nothing is read here: see sniff_gzip."""
-  import io
-  return io.open(fname, 'rb', buffering=1 << 20)      # BufferedReader: peek() does not consume
-
-
-def sniff_gzip(fp):
-  """gzip is recognised from the first bytes of the one open stream -- at the first READ, not at
-  open time: a writer that opens its two FIFOs one after the other only starts to write once BOTH
-  have a reader, so blocking on the first input's bytes before opening the second would deadlock."""
-  import gzip
-  if fp.peek(2)[:2] == b'\x1f\x8b':
-    return gzip.GzipFile(fileobj=fp, mode='rb')
-  return fp
+_Stream = FastqStream      # corrupt-reads' input stream under the name its FIFO / /dev/fd tests use
 
 
 def seq_lengths(buf):
@@ -52,46 +37,14 @@ def seq_lengths(buf):
   return (nl[1:4 * n_rec:4] - nl[0:4 * n_rec:4] - 1).astype(np.int64)
 
 
-class _Stream(object):
-  """A FASTQ file read in chunks into one (pinned) buffer; the unconsumed tail is carried over."""
-
-  def __init__(self, fname, buf):
-    self.fp = open_fastq(fname)
-    self.sniffed = False
-    self.buf, self.fill, self.eof = buf, 0, False
-
-  def close(self):
-    self.fp.close()
-
-  def refill(self):
-    if not self.sniffed:
-      self.fp, self.sniffed = sniff_gzip(self.fp), True
-    mv = memoryview(self.buf)
-    while self.fill < self.buf.size and not self.eof:
-      n = self.fp.readinto(mv[self.fill:])
-      if not n:
-        self.eof = True
-        if self.fill and self.buf[self.fill - 1] != 10 and self.fill < self.buf.size:
-          self.buf[self.fill] = 10; self.fill += 1           # last line without a newline
-      else:
-        self.fill += n
-
-  def consume(self, n):
-    rest = self.fill - n
-    if rest:
-      self.buf[:rest] = self.buf[n:self.fill].copy()
-    self.fill = rest
-
-
 def multi_process(read_module, read_model, fastq1_in, fastq1_out, fastq2_in=None, fastq2_out=None, processes=2, seed=7,
                   mode='philox', device=0, chunk_bytes=256 << 20):
   """Same signature as the reference (readcorrupt.py:18) plus keyword-only extras.  ``processes``
   is accepted for command-line compatibility (one GPU does all the work).  Note the reference
   passes the RAW model dict here (cli.py:155-157), and so does the CLI of this package.
 
-  The files are streamed in chunks through pinned buffers: the device indexes the records of each
-  chunk, corrupts the complete templates and reports how many input bytes they occupied; the rest
-  is carried into the next chunk.  The output does not depend on the chunk size.
+  The files are read in chunks (``lib.fastqio``); the device corrupts the complete templates of each.
+  The output does not depend on the chunk size.
 
   Page-locked host memory: one input buffer of ``chunk_bytes`` and two output buffers of twice that per file,
   i.e. 10 x chunk_bytes for a pair (2.5 GB at the default 256 MB; ``chunk_bytes`` scales it down)."""
@@ -102,9 +55,9 @@ def multi_process(read_module, read_model, fastq1_in, fastq1_out, fastq2_in=None
     rlen = read_model['mean_rlen'] if 'mean_rlen' in read_model else read_model['rlen']
     engine.load_model(read_model, rlen=rlen)
     paired = fastq2_in is not None
-    ins = [_Stream(fastq1_in, engine.pinned(chunk_bytes))] + ([_Stream(fastq2_in, engine.pinned(chunk_bytes))] if paired else [])
+    ins = [FastqStream(f, engine.pinned(chunk_bytes)) for f in (fastq1_in, fastq2_in) if f is not None]
     # two output buffer sets: the files of chunk k are written (one thread per file) while chunk k+1
-    # is read (one thread per file) and corrupted
+    # is read and corrupted
     outs = [(engine.pinned(2 * chunk_bytes + 64), engine.pinned(2 * chunk_bytes + 64) if paired else None) for _ in range(2)]
     pending = [[], []]
     from concurrent.futures import ThreadPoolExecutor
@@ -115,39 +68,31 @@ def multi_process(read_module, read_model, fastq1_in, fastq1_out, fastq2_in=None
       worker_seed = np.random.RandomState(seed).randint(SEED_MAX)   # worker 0, readcorrupt.py:31,36
       rng = np.random.RandomState(worker_seed)
     fps = [open(fastq1_out, 'wb')] + ([open(fastq2_out, 'wb')] if paired and fastq2_out is not None else [])
-    try:
-      while True:
-        for fu in [pool.submit(st.refill) for st in ins]:
-          fu.result()
-        a1 = ins[0].buf[:ins[0].fill]
-        a2 = ins[1].buf[:ins[1].fill] if paired else None
-        if a1.size == 0 or (paired and a2.size == 0):
-          break
-        draws = None
-        if rng is not None:
-          l1 = seq_lengths(a1)
-          if paired:
-            l2 = seq_lengths(a2)
-            n = min(l1.size, l2.size)
-            lens = np.empty(2 * n, dtype=np.int64); lens[0::2] = l1[:n]; lens[1::2] = l2[:n]
-          else:
-            lens = l1
-          draws = read_module.corrupt_draws(lens.tolist(), rng)
-        for fu in pending[k]:                                   # this buffer set's previous writes
-          fu.result()
-        pending[k] = []
-        o1, o2, n, c1, c2 = engine.corrupt_fastq(a1, a2, mode=MODE_DET if rng is not None else MODE_PHILOX, seed=seed, draws=draws,
-                                                 first_template=cnt, out=outs[k], partial=True)
-        if n == 0:
-          if all(st.eof for st in ins):
-            break
-          raise ValueError('a FASTQ record is larger than the chunk size ({} bytes)'.format(chunk_bytes))
-        pending[k] = [pool.submit(fp.write, memoryview(o)) for fp, o in zip(fps, (o1, o2))]
-        k ^= 1
-        ins[0].consume(c1)
+
+    def step(a1, a2):
+      nonlocal k, cnt
+      draws = None
+      if rng is not None:
+        l1 = seq_lengths(a1)
         if paired:
-          ins[1].consume(c2)
-        cnt += n
+          l2 = seq_lengths(a2)
+          n = min(l1.size, l2.size)
+          lens = np.empty(2 * n, dtype=np.int64); lens[0::2] = l1[:n]; lens[1::2] = l2[:n]
+        else:
+          lens = l1
+        draws = read_module.corrupt_draws(lens.tolist(), rng)
+      for fu in pending[k]:                                   # this buffer set's previous writes
+        fu.result()
+      pending[k] = []
+      o1, o2, n, c1, c2 = engine.corrupt_fastq(a1, a2, mode=MODE_DET if rng is not None else MODE_PHILOX, seed=seed, draws=draws,
+                                               first_template=cnt, out=outs[k], partial=True)
+      pending[k] = [pool.submit(fp.write, memoryview(o)) for fp, o in zip(fps, (o1, o2))]
+      k ^= 1
+      cnt += n
+      return n, c1, c2
+
+    try:
+      for_each_chunk(ins, step)
     finally:
       for fu in pending[0] + pending[1]:
         fu.result()

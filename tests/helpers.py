@@ -219,3 +219,17 @@ def roundtrip_fastq(f1, f2, index_for):
       if e:
         errs.append((lines[k], e))
   return n, errs
+
+
+def feed_interleaved(paths, datas, piece=256 << 10):
+  """One writer for a FIFO pair, as a tool that writes mate 1 and then mate 2 of each template in one loop:
+  ``piece`` bytes of file 1, then of file 2, and so on.  A reader that waits for one file to fill its buffer
+  before it reads the other blocks this writer on the other pipe."""
+  fps = [open(p, 'wb') for p in paths]          # each open blocks until the reader has opened that FIFO
+  for off in range(0, max(len(d) for d in datas), piece):
+    for fp, d in zip(fps, datas):
+      if off < len(d):
+        fp.write(d[off:off + piece])
+        fp.flush()
+  for fp in fps:
+    fp.close()

@@ -170,3 +170,24 @@ def test_cli_gzip_and_fifo_inputs(tmp_path, edge):
   assert res.exit_code == 0, res.output
   assert open(fbam, 'rb').read() == ref and open(fbam + '.bai', 'rb').read() == open(bam + '.bai', 'rb').read()
   assert not glob.glob(str(tmp_path / '*.run*'))
+
+
+@pytest.mark.timeout(300)
+def test_fifo_pair_fed_by_one_writer(tmp_path, edge):
+  """Both files of a pair are read at once: one writer alternating between the two FIFOs does not block."""
+  data = [H.golden_fastq(n) for n in GOLDEN['corrupt']]
+  chunk = 1 << 20
+  assert min(len(d) for d in data) > 2 * chunk
+  f1, f2 = str(tmp_path / 'c1.fq'), str(tmp_path / 'c2.fq')
+  for f, d in zip((f1, f2), data):
+    open(f, 'wb').write(d)
+  bam = str(tmp_path / 'plain.bam')
+  _run(edge['fasta'], bam, f1, f2, chunk_bytes=chunk)
+  p1, p2 = str(tmp_path / 'p1'), str(tmp_path / 'p2')
+  os.mkfifo(p1); os.mkfifo(p2)
+  t = threading.Thread(target=H.feed_interleaved, args=((p1, p2), data), daemon=True)
+  t.start()
+  fbam = str(tmp_path / 'fifo.bam')
+  _run(edge['fasta'], fbam, p1, p2, chunk_bytes=chunk)
+  t.join(timeout=10)
+  assert open(fbam, 'rb').read() == open(bam, 'rb').read() and open(fbam + '.bai', 'rb').read() == open(bam + '.bai', 'rb').read()
