@@ -300,6 +300,32 @@ int mg_readmodel_bam(mg_ctx *ctx, const char *path, int32_t max_bp, int32_t max_
                      double *thread_ms, int64_t *bad_where, int32_t *bad_code);
 int mg_bam_scan(const char *path, int32_t threads, int64_t chunk_bytes, int64_t *stats, int64_t *bad_where, int32_t *bad_code);
 
+/* ---- alignment-analysis: replaces mitty/benchmarking/mq.py and derr.py -- an aligner's BAM (file or FIFO, any
+ * sort order, no index) scored against the truth in Mitty's qnames, read and inflated as mg_readmodel_bam does.
+ * Every record in file order (C = 2 * max_d + 3 columns: d_err -max_d .. max_d, then wrong_chrom = C - 2,
+ * unmapped = C - 1):
+ *   flag & 0x900 (secondary, supplementary): skipped, nothing else.  QC-fail and duplicates are analysed.
+ *   read index i = 1 iff (flag & 0xC1) == 0x81, else 0; its qname fields (the name up to its NUL, split at '|')
+ *   are 3 + 5 * i .. + 4: strand, pos, rlen, CIGAR, v_list; field 1 is the chrom.
+ *   column: unmapped if flag & 0x4 or refID == -1; else wrong_chrom if the header name of refID differs byte for
+ *   byte from the chrom field; else d = start(POS, aligned CIGAR) - start(qname pos - 1, qname CIGAR), where
+ *   start(P, C) = P - the lengths of C's leading run of S, H and I ops (P ops skipped; '>p:nI' is nI), clamped
+ *   to [-max_d, max_d] at column d + max_d.
+ *   mq[MAPQ][column] += 1                                                          u64[256][C]
+ *   vsize[clamp(v, -max_size - 1, max_size + 1) + max_size + 1][column] += 1 per v_list entry v, or
+ *   vsize[2 * max_size + 3][column] += 1 for an empty v_list                       u64[2 * max_size + 4][C]
+ * counts[14]: records, analysed, skipped, unmapped, wrong_chrom, exact (d == 0), clamped (|d| > max_d),
+ * strand_mismatch (right chrom, flag & 0x10 differs from the qname strand), no_variant_reads, variant_entries,
+ * inflated bytes, compressed bytes, EOF member present, chunks.  times[6] and thread_ms as mg_readmodel_bam.
+ * Malformed input is MG_EVALUE with bad_code / bad_where as mg_readmodel_bam (1 .. 14), plus, for an analysed
+ * record (bad_where = its ordinal), in this order: 17 refID below -1 or at or above n_ref; 15 a qname that is
+ * not Mitty's (fewer than 8 fields; strand not 0 / 1; pos, a v_list entry or the '>p:' offset not a decimal
+ * integer; CIGAR not digits + one of MIDNSHP=X per op); 16 no read for this mate (a read-2 record whose qname
+ * has fewer than 13 fields).  The first bad record in file order is reported and no chunk after the one
+ * holding it is read.  0 <= max_d, max_size <= 10000 (MG_EINVAL otherwise).                          */
+int mg_alnerr_bam(mg_ctx *ctx, const char *path, int32_t max_d, int32_t max_size, int32_t threads, int64_t chunk_bytes, uint64_t *mq,
+                  uint64_t *vsize, int64_t *counts, double *times, double *thread_ms, int64_t *bad_where, int32_t *bad_code);
+
 /* ---- profiling: device time (CUDA events on the launch stream) of the emit / corrupt kernel
  * (emit_ms over emit_launches launches, emit_bytes written) and of the planning kernel (plan_ms);
  * total_launches counts every kernel this context launched since the last reset.               */

@@ -1,5 +1,6 @@
 """Command line with the reference's ``generate-reads`` / ``corrupt-reads`` / ``qname`` commands
-(mitty/cli.py:106-157), ``god-aligner`` (mitty/cli.py:191-204) and ``create-read-model bam2illumina``: same positional arguments and options, plus ``--deterministic`` (consume
+(mitty/cli.py:106-157), ``god-aligner`` (mitty/cli.py:191-204), ``create-read-model bam2illumina`` and
+``alignment-analysis``: same positional arguments and options, plus ``--deterministic`` (consume
 the reference's numpy draws; byte-exact against ``mitty ... --threads 1``) and, for
 generate-reads, ``--corrupt`` (fuse the corruption model into the emit kernel)."""
 import logging
@@ -127,6 +128,24 @@ def god_aligner(fasta, fastq1, bam, fastq2, threads, device, level):
   import mitty_b200.benchmarking.god_aligner as ga
   res = ga.process_multi_threaded(fasta, bam, fastq1, fastq2, threads=threads, device=device, level=level)
   click.echo('{} records written to {} in {:0.2f}s'.format(res['records'], bam, res['seconds']))
+
+
+@cli.command('alignment-analysis', short_help="Score an aligner's BAM against the truth in the qnames")
+@click.argument('bam', type=click.Path(exists=True))
+@click.argument('out_prefix')
+@click.option('--max-d', type=click.IntRange(0, 10000), default=200, help='d_err beyond +/- this is counted in the outermost columns')
+@click.option('--max-size', type=click.IntRange(0, 10000), default=50, help='variant sizes beyond +/- this are counted in the del> / ins> rows')
+@click.option('--threads', type=int, default=None, help='host inflate threads (default: the cores of the box)')
+@click.option('--device', default=0, help='CUDA device')
+def alignment_analysis(bam, out_prefix, max_d, max_size, threads, device):
+  """Count the alignments of BAM (a BGZF file or FIFO, any sort order, from an aligner run on reads simulated
+  here) by MAPQ x alignment error d_err and by variant size x d_err, d_err measured against the position in each
+  read's qname, and write them as OUT_PREFIX.mq.csv and OUT_PREFIX.vsize.csv."""
+  import mitty_b200.benchmarking.alignment_analysis as aa
+  res = aa.process_bam(bam, out_prefix, max_d=max_d, max_size=max_size, threads=threads, device=device)
+  click.echo('{} of {} records analysed in {:0.2f}s: {} exact, {} beyond +/-{}, {} on the wrong chrom, {} unmapped, {} on the wrong strand; '
+             '{} skipped (secondary / supplementary)'.format(res['analysed'], res['records'], res['seconds'], res['exact'], res['clamped'], max_d,
+                                                           res['wrong_chrom'], res['unmapped'], res['strand_mismatch'], res['skipped']))
 
 
 @cli.group('create-read-model')

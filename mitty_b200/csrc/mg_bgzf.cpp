@@ -451,6 +451,15 @@ int64_t MgBamReader::header(const uint8_t *b, int64_t pos, int64_t n) {
   while (hstate_ != 3 || hskip_) {
     if (hskip_) {
       const int64_t t = std::min(hskip_, n - pos);
+      if (hname_) {                                    // the skip starts with the reference's name: keep it up to its NUL
+        const int64_t c = std::min(t, hname_);
+        if (!hnul_) {
+          const uint8_t *z = static_cast<const uint8_t *>(memchr(b + pos, 0, (size_t)c));
+          ref_names.insert(ref_names.end(), b + pos, z ? z : b + pos + c);
+          hnul_ = z != nullptr;
+        }
+        if ((hname_ -= c) == 0) ref_off.push_back((int64_t)ref_names.size());
+      }
       pos += t; hskip_ -= t;
       if (hskip_) return pos;
       continue;
@@ -461,7 +470,11 @@ int64_t MgBamReader::header(const uint8_t *b, int64_t pos, int64_t n) {
     pos += hstate_ == 0 ? 8 : 4;
     if (hstate_ == 0) { hskip_ = v; hstate_ = 1; }
     else if (hstate_ == 1) { hrefs_ = v; hstate_ = v ? 2 : 3; }
-    else { hskip_ = (int64_t)v + 4; if (--hrefs_ == 0) hstate_ = 3; }
+    else {
+      hskip_ = (int64_t)v + 4; hname_ = v; hnul_ = false;
+      if (!v) ref_off.push_back((int64_t)ref_names.size());
+      if (--hrefs_ == 0) hstate_ = 3;
+    }
   }
   return pos;
 }

@@ -125,6 +125,11 @@ class MgBamReader {
   bool eof_marker = false;                     // the last member is the 28-byte EOF member
   double read_ms = 0, inflate_ms = 0, walk_ms = 0;   // reading the file; inflating (wall time); walking the record chain
   std::vector<double> thread_ms;               // busy time of each inflate thread
+  // the header's reference names, each up to its first NUL (at most l_name bytes): name i is
+  // ref_names[ref_off[i], ref_off[i + 1]).  Collected as the header streams past, so complete once next() has
+  // returned the first chunk of records.
+  std::vector<uint8_t> ref_names;
+  std::vector<int64_t> ref_off{0};
  private:
   struct Member { const uint8_t *z; int hdr, bsize; uint32_t crc, isize; int64_t out, comp; };
   int fill(uint8_t *b, int64_t &n, int64_t cap);          // 1: next member does not fit, 0: input ended or failed
@@ -140,5 +145,6 @@ class MgBamReader {
   bool in_eof_ = false, done_ = false;
   int carry_slot_ = -1; int64_t carry_at_ = 0, carry_n_ = 0;
   int hstate_ = 0; int64_t hskip_ = 0, hrefs_ = 0;          // BAM header walk
+  int64_t hname_ = 0; bool hnul_ = false;                   // name bytes still to come of the current reference; its NUL seen
   std::vector<Member> batch_;
 };

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <functional>
 #include <utility>
 #include "mg_core.cuh"
 
@@ -96,6 +97,30 @@ struct MgFastqChunk {
 cudaError_t mg_fastq_load(MgFastqChunk &q, const uint8_t *const in[2], const int64_t len[2], int nf, cudaStream_t st);
 // enqueues the D2H of the last byte offset of the first k templates of each file into last[] (the caller syncs)
 cudaError_t mg_fastq_ends(const MgFastqChunk &q, int64_t k, int64_t last[2], cudaStream_t st);
+
+// The chunk pipeline of the BAM readers (bam2illumina, alignment-analysis; mg_readmodel.cu).  Every chunk of
+// whole records of `rd` goes to the device on a copy stream while the previous one is processed on a kernel
+// stream: two slots (chunk buffers on both sides), five events per slot (H2D start / end, kernel start / end,
+// first_bad read back).  The caller supplies only its work:
+//   begin(ks)         before the first chunk: clear its accumulators;
+//   launch(c, data, off, first_bad, ks)   one chunk: c.n records at data + off[i] (record c.first + i of the file);
+//                     a malformed record k is reported by atomicMin(first_bad, k << 8 | code);
+//   finish(ks)        after the last chunk: copy its accumulators out (ks is synchronised afterwards).
+// Each returns MG_OK or an error code.  Once a slot's read-back shows a malformed record, no further chunk is read.
+// Fills times[6] (read, inflate, walk, H2D, kernel, whole call since t_start, ms), thread_ms (may be null) and
+// *chunks; -> MG_OK, the error of a CUDA call or a callback, or MG_EVALUE with bad_where / bad_code set for
+// malformed input (the device's first bad record, else the reader's error).
+class MgBamReader;
+struct MgBamChunk;
+struct MgBamPipe {
+  std::function<int(cudaStream_t)> begin, finish;
+  std::function<int(const MgBamChunk &, const uint8_t *, const uint32_t *, unsigned long long *, cudaStream_t)> launch;
+};
+int mg_bam_pipeline(mg_ctx *ctx, MgBamReader &rd, const MgBamPipe &p, double t_start, int64_t *chunks, double *times, double *thread_ms,
+                    int64_t *bad_where, int32_t *bad_code);
+double mg_now_ms();
+void *mg_pinned_alloc(size_t n);       // the reader's chunk buffers: page-locked, for the copies to the device
+void mg_pinned_release(void *p);
 
 #define MG_PLAN_TILE 256     // candidates per CTA tile of k_unit_plan
 #define MG_CTA 128           // threads per CTA of k_unit_emit (4 independent warps, 32 kept templates each)

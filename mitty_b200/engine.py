@@ -144,6 +144,28 @@ class Engine(object):
     out.update(zip(READ_MODEL_COUNTS, (int(x) for x in cnt)))
     return out
 
+  # -- alignment-analysis -----------------------------------------------------------------------
+  def alignment_error_counts(self, path, max_d=200, max_size=50, threads=1, chunk_bytes=64 << 20):
+    """mg_alnerr_bam: an aligner's BAM (file or FIFO) scored against the truth in the qnames.  -> dict with
+    mq u64[256, 2 * max_d + 3] (rows MAPQ, columns d_err -max_d .. max_d, wrong chrom, unmapped), vsize
+    u64[2 * max_size + 4, 2 * max_d + 3] (rows variant size < -max_size, -max_size .. max_size, > max_size, no
+    variant), the counters of ALIGNMENT_COUNTS, 'times' (ms: read, inflate, walk, h2d, kernel, total) and
+    'thread_ms'.  Malformed input raises ValueError naming the record ordinal or compressed offset."""
+    threads, max_d, max_size = max(1, int(threads)), int(max_d), int(max_size)
+    mq = np.zeros((256, 2 * max_d + 3), dtype=np.uint64)
+    vs = np.zeros((2 * max_size + 4, 2 * max_d + 3), dtype=np.uint64)
+    cnt, times, tms = np.zeros(len(ALIGNMENT_COUNTS), dtype=np.int64), np.zeros(6, dtype=np.float64), np.zeros(threads, dtype=np.float64)
+    bw, bc = C.c_int64(-1), C.c_int32(0)
+    rc = self._L.mg_alnerr_bam(self._h, str(path).encode(), max_d, max_size, threads, int(chunk_bytes), _ptr(mq), _ptr(vs), _ptr(cnt), _ptr(times),
+                               _ptr(tms), C.byref(bw), C.byref(bc))
+    if rc == _lib.MG_EVALUE and bc.value:
+      raise bam_read_error(path, bc.value, bw.value)
+    self._check(rc)
+    out = {'mq': mq, 'vsize': vs, 'thread_ms': tms,
+           'times': dict(zip(('read_ms', 'inflate_ms', 'walk_ms', 'h2d_ms', 'kernel_ms', 'total_ms'), (float(x) for x in times)))}
+    out.update(zip(ALIGNMENT_COUNTS, (int(x) for x in cnt)))
+    return out
+
   # -- haplotypes --------------------------------------------------------------------------------
   def load_region(self, ref_bytes, bed_start):
     ref = np.ascontiguousarray(ref_bytes, dtype=np.uint8)
@@ -454,16 +476,20 @@ def write_sorted_bam(bam, bai, contigs, header_text, records, level=6, threads=1
   return n.value
 
 
-# mg_readmodel_bam / mg_bam_scan errors: (what, whether bad_where is a record ordinal rather than a compressed offset)
+# mg_readmodel_bam / mg_alnerr_bam / mg_bam_scan errors (15-17: mg_alnerr_bam only): (what, whether bad_where is a record ordinal rather than a compressed offset)
 BAM_READ_ERRORS = {1: ('not a gzip member', False), 2: ("a gzip member without a BGZF 'BC' extra subfield", False),
                    3: ('corrupt or truncated BGZF member', False), 4: ('CRC32 mismatch', False),
                    5: ('ISIZE differs from the inflated length', False), 6: ('not a BAM file (magic or header lengths)', False),
                    7: ('the file ends inside the BAM header', False), 8: ('block_size < 32', True),
                    9: ('the file ends inside the record', True), 10: ('read error', False),
                    11: ('read name overruns block_size', True), 12: ('CIGAR overruns block_size', True),
-                   13: ('SEQ overruns block_size', True), 14: ('QUAL overruns block_size', True)}
+                   13: ('SEQ overruns block_size', True), 14: ('QUAL overruns block_size', True),
+                   15: ("not a Mitty qname (fields, strand, pos, CIGAR or v_list)", True),
+                   16: ('no read for this mate in the qname', True), 17: ('refID out of range', True)}
 READ_MODEL_COUNTS = ('records', 'considered', 'counted', 'skip_flag', 'skip_mapq', 'skip_empty', 'skip_noqual', 'skip_long',
                      'inflated_bytes', 'compressed_bytes', 'eof_marker', 'chunks')
+ALIGNMENT_COUNTS = ('records', 'analysed', 'skipped', 'unmapped', 'wrong_chrom', 'exact', 'clamped', 'strand_mismatch', 'no_variant_reads',
+                    'variant_entries', 'inflated_bytes', 'compressed_bytes', 'eof_marker', 'chunks')
 
 
 def bam_read_error(path, code, where):
